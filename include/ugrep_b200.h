@@ -99,6 +99,19 @@ typedef struct ugx_match {
   uint32_t cap;    /* accept index: 1-based alternative number */
 } ugx_match;
 
+/* one line, in input order: what lineno()/bol()/eol() return for it, and the first match on it (the match the `ugrep -c`
+ * loop finds before it skips to the next line) */
+typedef struct ugx_line {
+  uint64_t line;   /* 1-based line number (+ base_line) */
+  uint64_t bol;    /* offset of the line's first byte (+ base_offset) */
+  uint64_t eol;    /* offset of its '\n', or the buffer end for an unterminated last line (+ base_offset) */
+  uint64_t offset; /* first match on the line (first()); = bol for UGX_LINES_INVERT records */
+  uint32_t len;    /* its size(); 0 for UGX_LINES_INVERT records */
+  uint32_t cap;    /* its accept(); 0 = the line has no match */
+} ugx_line;        /* 40 bytes */
+
+#define UGX_LINES_INVERT 1u /* ugx_find_lines*: the lines WITHOUT a match (`ugrep -v`) */
+
 /* facts about an uploaded pattern */
 typedef struct ugx_pattern_info {
   uint32_t nop;          /* opcode words */
@@ -163,7 +176,8 @@ typedef struct ugx_totals {
 
 /* scan kernels (reported in ugx_totals.kernel; DESIGN.md section 4) */
 enum { UGX_K_NONE = 0, UGX_K_STREAM_LITERAL = 1, UGX_K_STREAM_DFA = 2, UGX_K_TILE_ANY = 3, UGX_K_LINE_SCAN = 4,
-       UGX_K_RECORDS = 5, UGX_K_NEWLINES = 6, UGX_K_MATCH_LINES = 7, UGX_K_SPAN = 8, UGX_K_BATCH = 9 };
+       UGX_K_RECORDS = 5, UGX_K_NEWLINES = 6, UGX_K_MATCH_LINES = 7, UGX_K_SPAN = 8, UGX_K_BATCH = 9,
+       UGX_K_SPAN_LINES = 10 };
 
 const char *ugx_last_error(void);
 const char *ugx_kernel_name(uint32_t id);
@@ -246,6 +260,22 @@ int  ugx_find_all_device(ugx_scanner *s, const ugx_pattern *p, const void *buf, 
                          const ugx_match **dev_out, uint64_t *n_out, ugx_totals *totals);
 /* copy `count` records of the last ugx_find_all_device result, starting at record `first`, to the host */
 int  ugx_scanner_fetch(ugx_scanner *s, ugx_match *out, uint64_t first, uint64_t count);
+/*
+ * Line records (`ugrep [-n] [-b]` and `ugrep -v`, src/ugrep.cpp:10567-10586 and the output loops that read lineno(),
+ * bol(), eol()): one ugx_line per line that matches, or with flags UGX_LINES_INVERT per line that does not, in input
+ * order.  A line is buf[bol, eol); a buffer that ends in '\n' has no empty line after it.  The matching records are the
+ * lines the `ugrep -c` loop counts (ugx_count_lines), each with that loop's match.  totals->matches = records,
+ * totals->newlines is always counted.  Line records live in their own scanner arena: a ugx_find_lines* call leaves the
+ * last ugx_find_all_device result valid, and the reverse.  Any other flags bit: UGX_E_INVALID.
+ */
+int  ugx_find_lines_device(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                           uint64_t base_offset, uint64_t base_line, uint32_t flags,
+                           const ugx_line **dev_out, uint64_t *n_out, ugx_totals *totals);
+int  ugx_find_lines(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                    uint64_t base_offset, uint64_t base_line, uint32_t flags,
+                    ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
+/* copy `count` line records of the last ugx_find_lines* result, starting at record `first`, to the host */
+int  ugx_scanner_fetch_lines(ugx_scanner *s, ugx_line *out, uint64_t first, uint64_t count);
 int  ugx_count_newlines(ugx_scanner *s, const void *buf, uint64_t nbytes, ugx_totals *totals);
 
 /*
@@ -297,6 +327,10 @@ int  ugx_sharded_set_option(ugx_sharded *s, const char *name, int value);
  * and line numbers global; shards[ndev] (optional) receives what every device did */
 int  ugx_sharded_scan(ugx_sharded *s, const void *host_buf, uint64_t nbytes, int mode, ugx_match *out, uint64_t cap,
                       uint64_t *n_out, ugx_totals *totals, ugx_shard *shards);
+/* line records of all shards (ugx_find_lines) to out[cap] in input order, line numbers and offsets global;
+ * shards[r].record_base = line records before shard r */
+int  ugx_sharded_find_lines(ugx_sharded *s, const void *host_buf, uint64_t nbytes, uint32_t flags, ugx_line *out,
+                            uint64_t cap, uint64_t *n_out, ugx_totals *totals, ugx_shard *shards);
 const char *ugx_sharded_last_error(void);
 
 #ifdef __cplusplus

@@ -21,13 +21,17 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("UGX_LIB") or os.path.join(HERE, "libugrep_b200.so")  # UGX_LIB: A/B builds (tools/variants.py)
 
 MATCH_DTYPE = np.dtype([("line", "<u8"), ("offset", "<u8"), ("len", "<u4"), ("cap", "<u4")])
+# ugx_line: one record per line (find_lines): line number, the line's [bol, eol), its first match (offset, len, cap)
+LINE_DTYPE = np.dtype([("line", "<u8"), ("bol", "<u8"), ("eol", "<u8"), ("offset", "<u8"), ("len", "<u4"), ("cap", "<u4")])
+LINES_INVERT = 1
 
 ADVANCE_NAMES = ["none", "pin1_one", "pin1_pma", "pin1_pmh", "pin_one", "pin_pma", "pin_pmh", "min1", "min2", "min3",
                  "min4", "pma", "char", "char_pma", "char_pmh", "string", "string_pma", "string_pmh"]
 
 EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_version", "ugx_pattern_create", "ugx_pattern_load", "ugx_pattern_info_get",
            "ugx_pattern_destroy", "ugx_scanner_create", "ugx_scanner_destroy", "ugx_count_lines", "ugx_count_matches",
-           "ugx_viability_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines"]
+           "ugx_viability_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
+           "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines"]
 
 
 class UgxError(RuntimeError):
@@ -91,6 +95,11 @@ def lib():
                                           C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         L.ugx_scanner_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.ugx_scanner_fetch.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]
+        L.ugx_find_lines.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32,
+                                     C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_find_lines_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64,
+                                            C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_scanner_fetch_lines.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]
         _lib = L
     return _lib
 
@@ -292,6 +301,31 @@ class Scanner:
             _check(lib().ugx_scanner_fetch(self._h, out.ctypes.data, 0, cnt.value))
         return out, self._totals(t)
 
+    def find_lines_device(self, pattern: Pattern, data, invert: bool = False, base_offset: int = 0,
+                          base_line: int = 0) -> Totals:
+        """Like find_lines but the records stay on the device (fetch_lines() copies a range to the host); the match
+        records of find_all_device stay valid alongside."""
+        ptr, n, keep = _buffer(data)
+        t = _Totals()
+        dev = C.c_void_p()
+        cnt = C.c_uint64()
+        _check(lib().ugx_find_lines_device(self._h, pattern._h, C.c_void_p(ptr), n, base_offset, base_line,
+                                           LINES_INVERT if invert else 0, C.byref(dev), C.byref(cnt), C.byref(t)))
+        self.last_lines = (dev.value, cnt.value)
+        return self._totals(t)
+
+    def fetch_lines(self, first: int, count: int) -> np.ndarray:
+        out = np.zeros(count, dtype=LINE_DTYPE)
+        if count:
+            _check(lib().ugx_scanner_fetch_lines(self._h, out.ctypes.data, first, count))
+        return out
+
+    def find_lines(self, pattern: Pattern, data, invert: bool = False, base_offset: int = 0, base_line: int = 0):
+        """The lines the `ugrep -c` loop counts, each with its first match, in input order as a structured array
+        (line, bol, eol, offset, len, cap) + totals; with invert the lines without a match (`ugrep -v`)."""
+        t = self.find_lines_device(pattern, data, invert, base_offset, base_line)
+        return self.fetch_lines(0, self.last_lines[1]), t
+
     def close(self):
         if self._h:
             lib().ugx_scanner_destroy(self._h)
@@ -359,6 +393,8 @@ class Sharded:
                                          C.POINTER(C.c_void_p)]
         L.ugx_sharded_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
                                        C.POINTER(C.c_uint64), C.POINTER(_Totals), C.c_void_p]
+        L.ugx_sharded_find_lines.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64,
+                                             C.POINTER(C.c_uint64), C.POINTER(_Totals), C.c_void_p]
         L.ugx_sharded_destroy.argtypes = [C.c_void_p]
         L.ugx_sharded_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.ugx_sharded_last_error.restype = C.c_char_p
@@ -394,6 +430,30 @@ class Sharded:
         info = [{f: getattr(sh, f) for f, _ in _Shard._fields_ if not f.startswith("reserved")} for sh in shards]
         tot = Totals(t.matches, t.newlines, t.flags, t.kernel_ms, t.launches, lib().ugx_kernel_name(t.kernel).decode())
         return tot, (out[:cnt.value] if out is not None else None), info
+
+    def find_lines(self, data, invert: bool = False, cap: int | None = None):
+        """-> (line records of all shards in input order, totals, per-shard info); shard record_base = line records
+        before the shard"""
+        ptr, n, keep = _buffer(data)
+        if hasattr(keep, "is_cuda"):
+            raise TypeError("ugx_sharded_find_lines takes host memory")
+        t = _Totals()
+        shards = (_Shard * len(self.devices))()
+        cnt = C.c_uint64()
+        if cap is None:
+            cap = n // 2 + 16 if invert else max(1024, n // 16)
+        out = np.zeros(cap, dtype=LINE_DTYPE)
+        args = (self._h, C.c_void_p(ptr), n, LINES_INVERT if invert else 0)
+        rc = lib().ugx_sharded_find_lines(*args, out.ctypes.data, cap, C.byref(cnt), C.byref(t), shards)
+        if rc == 5:  # UGX_E_OVERFLOW: *n_out holds the count
+            cap = cnt.value
+            out = np.zeros(max(cap, 1), dtype=LINE_DTYPE)
+            rc = lib().ugx_sharded_find_lines(*args, out.ctypes.data, cap, C.byref(cnt), C.byref(t), shards)
+        if rc != 0:
+            raise UgxError(rc, lib().ugx_sharded_last_error().decode("utf-8", "replace"))
+        info = [{f: getattr(sh, f) for f, _ in _Shard._fields_ if not f.startswith("reserved")} for sh in shards]
+        tot = Totals(t.matches, t.newlines, t.flags, t.kernel_ms, t.launches, lib().ugx_kernel_name(t.kernel).decode())
+        return out[:cnt.value], tot, info
 
     def close(self):
         if self._h:

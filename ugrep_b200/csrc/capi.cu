@@ -142,6 +142,12 @@ struct ugx_scanner {
   uint64_t batch_cap = 0;
   bool no_span = false;           // counting matches / records take the line-at-a-time kernels (A/B timing, tests)
   bool no_cover = false;          // the streaming count evaluates the candidate predicate even where it is proven implied
+  // line records (ugx_find_lines*): an arena of their own, so that they and the match records stay valid side by side
+  ugx_line* lines = nullptr;
+  uint64_t lines_cap = 0;
+  uint64_t lines_n = 0;
+  uint64_t* lines_regions = nullptr; // [5 * regions + 8] span route: SpanLinesArgs region values and the last line
+  uint64_t lines_regions_cap = 0;
 };
 
 extern "C" {
@@ -536,6 +542,8 @@ void ugx_scanner_destroy(ugx_scanner* s)
   cudaFree(s->partials);
   cudaFree(s->ticket);
   cudaFree(s->records);
+  cudaFree(s->lines);
+  cudaFree(s->lines_regions);
   cudaFree(s->stage);
   if (s->ev0)
     cudaEventDestroy(s->ev0);
@@ -740,28 +748,24 @@ bool is_pinned_host_pointer(const void* buf)
   return at.type == cudaMemoryTypeHost;
 }
 
-// `ugrep -c -o` / `ugrep -o -n -b` through the span kernels (span_scan.cu).  *valid = false: the spans could not vouch
-// for their result on this buffer (a match longer than a window across a region start in a line without newlines, an
-// attempt that failed at the very end of the buffer, a match of 64 KiB or more) — the caller then takes the
-// line-at-a-time kernels.
-int scan_spans(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, bool want_records, uint64_t base_offset,
-               uint64_t base_line, ugx_totals* tt, bool* valid)
+// the count pass of the span kernels (last line, span_scan_kernel, span_final_kernel) up to the host's read of
+// s->h_totals[0..2]; with want_sel the selected match starts are left in s->span_sel
+int span_count_pass(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, bool want_sel, uint64_t base_offset,
+                    uint64_t base_line, ugx::SpanArgs& a, ugx_totals* tt)
 {
-  *valid = false;
   const uint64_t nreg = ugx::stream_regions(n);
   int rc = ensure(s->span_regions, s->span_regions_cap, 5 * nreg + 8);
-  if (rc == UGX_OK && want_records)
+  if (rc == UGX_OK && want_sel)
     rc = ensure(s->span_sel, s->span_sel_cap, (n + 15) / 16 + 64);
   if (rc != UGX_OK)
     return rc;
-  ugx::SpanArgs a;
   memset(&a, 0, sizeof(a));
   a.reg_matches = s->span_regions;
   a.reg_newlines = s->span_regions + nreg;
   a.reg_emain = s->span_regions + 2 * nreg;
   a.reg_elast = s->span_regions + 3 * nreg;
   a.reg_v = s->span_regions + 4 * nreg;
-  a.sel_bits = want_records ? s->span_sel : nullptr;
+  a.sel_bits = want_sel ? s->span_sel : nullptr;
   a.base_offset = base_offset;
   a.base_line = base_line;
   a.no_cover = s->no_cover ? 1u : 0u;
@@ -774,6 +778,21 @@ int scan_spans(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64
   CU(cudaMemcpyAsync(s->h_totals, s->totals, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
   CU(cudaStreamSynchronize(s->stream));
   tt->launches += 3;
+  return UGX_OK;
+}
+
+// `ugrep -c -o` / `ugrep -o -n -b` through the span kernels (span_scan.cu).  *valid = false: the spans could not vouch
+// for their result on this buffer (a match longer than a window across a region start in a line without newlines, an
+// attempt that failed at the very end of the buffer, a match of 64 KiB or more) — the caller then takes the
+// line-at-a-time kernels.
+int scan_spans(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, bool want_records, uint64_t base_offset,
+               uint64_t base_line, ugx_totals* tt, bool* valid)
+{
+  *valid = false;
+  ugx::SpanArgs a;
+  int rc = span_count_pass(s, p, dbuf, n, want_records, base_offset, base_line, a, tt);
+  if (rc != UGX_OK)
+    return rc;
   if (s->h_totals[2] != 0)
     return UGX_OK; // not valid: nothing of this attempt is used
   const uint64_t nrec = s->h_totals[0];
@@ -1087,9 +1106,209 @@ int scan_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t 
   return UGX_OK;
 }
 
+// line records through the span kernels: the selected match starts of span_scan_kernel, then span_lines_kernel's count
+// pass, one CTA for the bases and carries, and the emit pass.  *valid = false as for scan_spans.
+int span_lines(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, uint32_t flags, uint64_t base_offset,
+               uint64_t base_line, ugx_totals* tt, bool* valid)
+{
+  *valid = false;
+  ugx::SpanArgs sa;
+  int rc = span_count_pass(s, p, dbuf, n, true, base_offset, base_line, sa, tt);
+  if (rc != UGX_OK)
+    return rc;
+  if (s->h_totals[2] != 0)
+    return UGX_OK;
+  const uint64_t nreg = ugx::stream_regions(n);
+  rc = ensure(s->lines_regions, s->lines_regions_cap, 5 * nreg + 8);
+  if (rc != UGX_OK)
+    return rc;
+  ugx::SpanLinesArgs a;
+  memset(&a, 0, sizeof(a));
+  a.reg_nl = s->lines_regions;
+  a.reg_m = s->lines_regions + nreg;
+  a.reg_bol = s->lines_regions + 2 * nreg;
+  a.reg_fb = s->lines_regions + 3 * nreg;
+  a.reg_fa = s->lines_regions + 4 * nreg;
+  a.tail = s->lines_regions + 5 * nreg;
+  a.sel_bits = s->span_sel;
+  a.limit = sa.tail;
+  a.base_offset = base_offset;
+  a.base_line = base_line;
+  a.invert = flags & UGX_LINES_INVERT;
+  CU(ugx::launch_span_lines(p->dev, dbuf, n, a, false, s->sm_count, s->stream));
+  CU(ugx::launch_span_lines_final(p->dev, dbuf, n, a, s->totals, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  tt->launches += 2;
+  const uint64_t nrec = s->h_totals[0];
+  rc = ensure(s->lines, s->lines_cap, nrec);
+  if (rc != UGX_OK)
+    return rc;
+  if (nrec > 0)
+  {
+    a.out = s->lines;
+    a.out_cap = nrec;
+    CU(ugx::launch_span_lines(p->dev, dbuf, n, a, true, s->sm_count, s->stream));
+    tt->launches += 1;
+  }
+  s->lines_n = nrec;
+  tt->matches = nrec;
+  tt->newlines = s->h_totals[1];
+  tt->flags |= UGX_TOT_NEWLINES;
+  tt->kernel = UGX_K_SPAN_LINES;
+  *valid = true;
+  return UGX_OK;
+}
+
+int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint64_t base_offset,
+                      uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals)
+{
+  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
+    return fail(UGX_E_INVALID, "null argument");
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return fail(UGX_E_INVALID, "ugx_find_lines: unknown flags");
+  if (s->device != p->device)
+    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+  ugx_totals tt;
+  memset(&tt, 0, sizeof(tt));
+  tt.flags = UGX_TOT_NEWLINES;
+  if (n_out)
+    *n_out = 0;
+  if (dev_out)
+    *dev_out = nullptr;
+  if (n == 0)
+  {
+    s->lines_n = 0;
+    if (totals)
+      *totals = tt;
+    return UGX_OK;
+  }
+  CU(cudaSetDevice(s->device));
+  const uint8_t* dbuf = nullptr;
+  uint64_t h2d = 0;
+  int rc = resolve(s, buf, n, &dbuf, &h2d);
+  if (rc != UGX_OK)
+    return rc;
+  CU(cudaEventRecord(s->ev0, s->stream));
+  bool done = false;
+  if (!p->never && !s->force_generic && !s->no_span && ugx::span_scan_eligible(p->dev))
+  {
+    rc = span_lines(s, p, dbuf, n, flags, base_offset, base_line, &tt, &done);
+    if (rc != UGX_OK)
+      return rc;
+    if (!done)
+    {
+      tt.launches = 0; // the line-at-a-time kernels take over
+      tt.flags |= UGX_TOT_SPAN_HANDOVER;
+    }
+  }
+  if (!done)
+  {
+    // the line-at-a-time kernels: a count pass into strip_counts, the tile prefix, an emit pass.  A pattern whose
+    // prefilter admits no candidate searches no line (all lines are records of the inverted form).
+    const uint64_t tile_bytes = ugx::scan_tile_bytes(p->dev);
+    const uint64_t ntiles = (n + tile_bytes - 1) / tile_bytes;
+    const uint64_t nstrips = (n + ugx::SCAN_STRIP - 1) / ugx::SCAN_STRIP;
+    uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
+    rc = ensure(s->tile_matches, cap1, ntiles);
+    if (rc == UGX_OK)
+      rc = ensure(s->tile_newlines, cap2, ntiles);
+    s->tiles_cap = cap1 < cap2 ? cap1 : cap2;
+    if (rc == UGX_OK)
+      rc = ensure(s->strip_counts, s->strips_cap, nstrips);
+    if (rc != UGX_OK)
+      return rc;
+    ugx::ScanArgs a;
+    a.buf = dbuf;
+    a.n = n;
+    a.ntiles = ntiles;
+    a.tile_matches = s->tile_matches;
+    a.tile_newlines = s->tile_newlines;
+    a.strip_counts = s->strip_counts;
+    a.out = nullptr;
+    a.out_cap = 0;
+    a.base_offset = base_offset;
+    a.base_line = base_line;
+    const uint32_t lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
+    CU(ugx::launch_scan_line_records(p->dev, a, nullptr, lflags, false, s->sm_count, s->stream));
+    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
+    CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    tt.launches += 2;
+    const uint64_t nrec = s->h_totals[0];
+    rc = ensure(s->lines, s->lines_cap, nrec);
+    if (rc != UGX_OK)
+      return rc;
+    if (nrec > 0)
+    {
+      a.out_cap = nrec;
+      CU(ugx::launch_scan_line_records(p->dev, a, s->lines, lflags, true, s->sm_count, s->stream));
+      tt.launches += 1;
+    }
+    s->lines_n = nrec;
+    tt.matches = nrec;
+    tt.newlines = s->h_totals[1];
+    tt.kernel = UGX_K_LINE_SCAN;
+  }
+  CU(cudaEventRecord(s->ev1, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  float ms = 0;
+  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+  tt.kernel_ms = ms;
+  if (n_out)
+    *n_out = s->lines_n;
+  if (dev_out)
+    *dev_out = s->lines;
+  if (totals)
+    *totals = tt;
+  return UGX_OK;
+}
+
 } // namespace
 
 extern "C" {
+
+int ugx_find_lines_device(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
+                          uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals)
+{
+  return find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, dev_out, n_out, totals);
+}
+
+int ugx_find_lines(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
+                   uint64_t base_line, uint32_t flags, ugx_line* out, uint64_t cap, uint64_t* n_out, ugx_totals* totals)
+{
+  const ugx_line* dev = nullptr;
+  uint64_t n = 0;
+  int rc = find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, &dev, &n, totals);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  if (n > cap)
+    return fail(UGX_E_OVERFLOW, "line record buffer too small");
+  if (n > 0)
+  {
+    if (out == nullptr)
+      return fail(UGX_E_INVALID, "null record buffer");
+    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+  }
+  return UGX_OK;
+}
+
+int ugx_scanner_fetch_lines(ugx_scanner* s, ugx_line* out, uint64_t first, uint64_t count)
+{
+  if (s == nullptr || (out == nullptr && count != 0))
+    return fail(UGX_E_INVALID, "null argument");
+  if (first > s->lines_n || count > s->lines_n - first)
+    return fail(UGX_E_INVALID, "record range outside the last line-record result");
+  if (count == 0)
+    return UGX_OK;
+  CU(cudaSetDevice(s->device));
+  CU(cudaMemcpyAsync(out, s->lines + first, count * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  return UGX_OK;
+}
 
 int ugx_count_lines(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, ugx_totals* totals)
 {
@@ -1142,6 +1361,7 @@ const char* ugx_kernel_name(uint32_t id)
     case UGX_K_MATCH_LINES: return "match_lines_kernel";
     case UGX_K_SPAN: return "span_scan_kernel";
     case UGX_K_BATCH: return "scan_batch_kernel";
+    case UGX_K_SPAN_LINES: return "span_lines_kernel";
     default: return "none";
   }
 }

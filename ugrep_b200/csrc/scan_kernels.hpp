@@ -38,6 +38,11 @@ struct ScanArgs {
 int scan_threads(const DevPattern& P);
 uint32_t scan_tile_bytes(const DevPattern& P);
 cudaError_t launch_scan_lines(const DevPattern& P, const ScanArgs& a, int mode, bool emit, int sm_count, cudaStream_t st);
+// line records (`ugrep -c` loop per line, ugx_find_lines): the count pass writes a.strip_counts and the tile sums, the
+// emit pass (after launch_tile_prefix) writes out[]; lflags = UGX_LINES_INVERT | SCAN_LINES_NEVER
+constexpr uint32_t SCAN_LINES_NEVER = 2u;
+cudaError_t launch_scan_line_records(const DevPattern& P, const ScanArgs& a, ugx_line* out, uint32_t lflags, bool emit,
+                                     int sm_count, cudaStream_t st);
 // `ugrep -c` for patterns without look-back: one position-parallel kernel, totals[0] = matching lines, [1] = newlines
 bool count_lines_any_eligible(const DevPattern& P);
 cudaError_t launch_count_lines_any(const DevPattern& P, const uint8_t* buf, uint64_t n, unsigned long long* totals,
@@ -117,6 +122,31 @@ cudaError_t launch_span_scan(const DevPattern& P, const uint8_t* buf, uint64_t n
                              cudaStream_t st);
 cudaError_t launch_span_final(const DevPattern& P, const uint8_t* buf, uint64_t n, const SpanArgs& a, bool emit,
                               unsigned long long* totals, cudaStream_t st);
+
+// ---- line records from the span kernels' selected match starts (span_scan.cu, ugx_find_lines) ----
+// A line belongs to the region that holds its '\n'; a line that began in an earlier region gets its start and its first
+// match from carries over the regions before (span_lines_final_kernel).  The region values, [regions] each:
+struct SpanLinesArgs {
+  uint64_t* reg_nl;        // count pass: newlines in the region;            after the final kernel: newlines before it
+  uint64_t* reg_m;         //   owned lines after the first with a selected start;           records before the region
+  uint64_t* reg_bol;       //   last newline + 1 (0 = none);                 start of the line that runs into the region
+  uint64_t* reg_fb;        //   first selected start before the first newline (~0 = none)   (unused afterwards)
+  uint64_t* reg_fa;        //   first selected start after the last newline;  first selected start since reg_bol, before the region
+  uint64_t* tail;          // [8] the line after the last region's last newline: {line, bol, eol, offset, len | cap << 32
+                           //     (~0 = longest_at still to run), record index, present}
+  const uint16_t* sel_bits;// span_scan_kernel's selected match starts
+  const uint64_t* limit;   // device: where the spans stop (SpanArgs::tail)
+  ugx_line* out;           // emit pass: records in input order
+  uint64_t out_cap;
+  uint64_t base_offset, base_line;
+  uint32_t invert;         // UGX_LINES_INVERT: the records are the lines without a selected start
+  uint32_t stage_table;    // set by the launcher
+};
+cudaError_t launch_span_lines(const DevPattern& P, const uint8_t* buf, uint64_t n, SpanLinesArgs a, bool emit, int sm_count,
+                              cudaStream_t st);
+// one CTA: record / line bases and carries of the regions, the last line; totals[0] = records, [1] = newlines
+cudaError_t launch_span_lines_final(const DevPattern& P, const uint8_t* buf, uint64_t n, const SpanLinesArgs& a,
+                                    unsigned long long* totals, cudaStream_t st);
 
 // reflex::nlcount (newline_count.cu)
 cudaError_t launch_count_newlines(const uint8_t* buf, uint64_t n, unsigned long long* total, int sm_count, cudaStream_t st);

@@ -135,8 +135,14 @@ int ugx_sharded_set_option(ugx_sharded* s, const char* name, int value)
   return UGX_OK;
 }
 
-int ugx_sharded_scan(ugx_sharded* s, const void* host_buf, uint64_t n, int mode, ugx_match* out, uint64_t cap,
-                     uint64_t* n_out, ugx_totals* totals, ugx_shard* shards)
+} // extern "C"
+
+namespace {
+
+// ugx_sharded_scan, and with `lines` ugx_sharded_find_lines (mode UGX_MODE_RECORDS, out is a ugx_line array): line
+// records go through the same two phases as match records, with ugx_find_lines_device in place of ugx_find_all_device
+int sharded_run(ugx_sharded* s, const void* host_buf, uint64_t n, int mode, bool lines, uint32_t lflags, void* out,
+                uint64_t cap, uint64_t* n_out, ugx_totals* totals, ugx_shard* shards)
 {
   if (s == nullptr || (host_buf == nullptr && n != 0) || mode < UGX_MODE_LINES || mode > UGX_MODE_RECORDS)
     return sfail(UGX_E_INVALID, "ugx_sharded_scan: bad argument");
@@ -220,9 +226,18 @@ int ugx_sharded_scan(ugx_sharded* s, const void* host_buf, uint64_t n, int mode,
       const uint64_t len = cuts[r + 1] - cuts[r];
       if (len == 0)
         return;
-      const ugx_match* dev = nullptr;
       ugx_totals t2;
-      rcs[r] = ugx_find_all_device(s->scanners[r], s->patterns[r], s->dbuf[r], len, cuts[r], line_base[r], &dev, &nrec[r], &t2);
+      if (lines)
+      {
+        const ugx_line* dev = nullptr;
+        rcs[r] = ugx_find_lines_device(s->scanners[r], s->patterns[r], s->dbuf[r], len, cuts[r], line_base[r], lflags, &dev,
+                                       &nrec[r], &t2);
+      }
+      else
+      {
+        const ugx_match* dev = nullptr;
+        rcs[r] = ugx_find_all_device(s->scanners[r], s->patterns[r], s->dbuf[r], len, cuts[r], line_base[r], &dev, &nrec[r], &t2);
+      }
       if (rcs[r] != UGX_OK)
         errs[r] = ugx_last_error();
       else
@@ -252,7 +267,8 @@ int ugx_sharded_scan(ugx_sharded* s, const void* host_buf, uint64_t n, int mode,
       // records come back in shard order = input order; offsets and line numbers already carry their bases
       each([&](int r) {
         if (nrec[r] != 0)
-          rcs[r] = ugx_scanner_fetch(s->scanners[r], out + rec_base[r], 0, nrec[r]);
+          rcs[r] = lines ? ugx_scanner_fetch_lines(s->scanners[r], static_cast<ugx_line*>(out) + rec_base[r], 0, nrec[r])
+                         : ugx_scanner_fetch(s->scanners[r], static_cast<ugx_match*>(out) + rec_base[r], 0, nrec[r]);
         if (rcs[r] != UGX_OK)
           errs[r] = ugx_last_error();
       });
@@ -296,6 +312,24 @@ int ugx_sharded_scan(ugx_sharded* s, const void* host_buf, uint64_t n, int mode,
       shards[r].kernel_ms = tt[r].kernel_ms;
     }
   return UGX_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int ugx_sharded_scan(ugx_sharded* s, const void* host_buf, uint64_t n, int mode, ugx_match* out, uint64_t cap,
+                     uint64_t* n_out, ugx_totals* totals, ugx_shard* shards)
+{
+  return sharded_run(s, host_buf, n, mode, false, 0, out, cap, n_out, totals, shards);
+}
+
+int ugx_sharded_find_lines(ugx_sharded* s, const void* host_buf, uint64_t n, uint32_t flags, ugx_line* out, uint64_t cap,
+                           uint64_t* n_out, ugx_totals* totals, ugx_shard* shards)
+{
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return sfail(UGX_E_INVALID, "ugx_sharded_find_lines: unknown flags");
+  return sharded_run(s, host_buf, n, UGX_MODE_RECORDS, true, flags, out, cap, n_out, totals, shards);
 }
 
 } // extern "C"

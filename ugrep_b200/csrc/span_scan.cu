@@ -890,6 +890,352 @@ span_final_kernel(const __grid_constant__ DevPattern P, const uint8_t* __restric
   }
 }
 
+// ---- line records (ugx_find_lines) from the selected match starts ----
+//
+// A line is on the `ugrep -c` loop's list when it holds a selected start: the chain is fresh after every newline (no
+// match crosses one), so the first selected start at or after a line's start is the match the loop's find() returns
+// from there, and the loop then skips to the next line.  A line belongs to the region that holds its '\n'.  The count
+// pass knows, per region, every owned line but the first; the first one began at or before the region start, and
+// whether it matches also depends on the regions before: span_lines_final_kernel carries "last newline before the
+// region" (max) and "first selected start since then" (a minimum that restarts at every region with a newline) over
+// all regions, so a line over thousands of regions comes out of one prefix.
+
+namespace {
+constexpr uint64_t SL_NONE = ~0ull;
+}
+
+// count pass (EMIT = false): per region the SpanLinesArgs count values; emit pass: the records of the owned lines in
+// their final slots (bases and carries from span_lines_final_kernel), and the last line's record from thread 0
+template <bool EMIT, int THREADS>
+__global__ void __launch_bounds__(THREADS, 4)
+span_lines_kernel(const __grid_constant__ DevPattern P, const uint8_t* __restrict__ buf, uint64_t n, SpanLinesArgs a)
+{
+  constexpr uint32_t NWARPS = THREADS / 32;
+  extern __shared__ __align__(16) uint8_t smem[];
+  __shared__ __align__(8) uint64_t s_bar;
+  Tables T;
+  if (EMIT)
+  {
+    // longest_at at the first selected start of every matching line
+    uint8_t* s_cls = smem;
+    uint8_t* s_pred = s_cls + 256;
+    uint8_t* s_tap = s_pred + UGX_HASH;
+    uint16_t* s_next = reinterpret_cast<uint16_t*>(s_tap + UGX_BTAP);
+    stage_tables_bulk(&s_bar, s_cls, P.cls, s_pred, P.pred, s_tap, P.tap, s_next, P.next,
+                      a.stage_table ? ((P.table_bytes + 15) / 16) * 16 : 0);
+    __syncthreads();
+    T.cls = s_cls;
+    T.pred = s_pred;
+    T.tap = s_tap;
+    T.next = a.stage_table ? s_next : P.next;
+  }
+  const Text t{buf, n};
+  const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const bool inv = a.invert != 0;
+  const uint64_t limit = __ldcg(a.limit);
+  const uint64_t nregions = (limit + SC_REGION - 1) / SC_REGION;
+  const uint64_t total_warps = static_cast<uint64_t>(gridDim.x) * NWARPS;
+  if (EMIT && blockIdx.x == 0 && threadIdx.x == 0 && a.tail[6] != 0)
+  {
+    const Stepper step(T, P.ncls, a.stage_table != 0);
+    ugx_line rec;
+    rec.line = a.tail[0];
+    rec.bol = a.tail[1] + a.base_offset;
+    rec.eol = a.tail[2] + a.base_offset;
+    rec.offset = a.tail[3] + a.base_offset;
+    uint64_t lc = a.tail[4];
+    if (lc == SL_NONE)
+    {
+      const uint32_t d = longest_at(t, P, step, a.tail[3]);
+      lc = (static_cast<uint64_t>(d >> 16) << 32) | (d & 0xffffu);
+    }
+    rec.len = static_cast<uint32_t>(lc);
+    rec.cap = static_cast<uint32_t>(lc >> 32);
+    if (a.tail[5] < a.out_cap)
+      a.out[a.tail[5]] = rec;
+  }
+  for (uint64_t r = static_cast<uint64_t>(blockIdx.x) * NWARPS + wid; r < nregions; r += total_warps)
+  {
+    const uint64_t rb = r * SC_REGION;
+    // warp-uniform state at the current span: first selected start since the last newline, start of the current line
+    uint64_t first = EMIT ? a.reg_fa[r] : SL_NONE;
+    uint64_t bol = EMIT ? a.reg_bol[r] : 0;
+    uint64_t idx0 = EMIT ? a.reg_m[r] : 0;
+    uint64_t line0 = EMIT ? a.reg_nl[r] + 1 + a.base_line : 0;
+    uint64_t nl_run = 0, fb = SL_NONE;
+    uint32_t m_run = 0; // lane-private: matching owned lines but the region's first
+    for (int s = 0; s < SP_SPANS; ++s)
+    {
+      const uint64_t sbase = rb + static_cast<uint64_t>(s) * SP_SPAN;
+      if (sbase >= limit)
+        break;
+      const uint64_t base = sbase + lane * 16;
+      uint32_t nl = 0, sel = 0;
+      if (base < limit)
+      {
+        const uint4 v = load_chunk_guarded(buf, n, base);
+        nl = newline_mask_exact4(v.x, v.y, v.z, v.w);
+        sel = a.sel_bits[(sbase >> 4) + lane];
+        if (base + 16 > limit)
+        {
+          nl &= (1u << (limit - base)) - 1u;
+          sel &= (1u << (limit - base)) - 1u;
+        }
+      }
+      // per lane: the first selected start after its last newline (of the whole chunk without one), the start of the
+      // line after its last newline, its newlines; then inclusive scans over the lanes (the first one restarts at every
+      // lane with a newline)
+      const uint32_t hb = nl != 0 ? 31u - __clz(nl) : 0u;
+      const uint32_t after = nl != 0 ? sel & ~((2u << hb) - 1u) : sel;
+      uint64_t v = after != 0 ? base + __ffs(after) - 1 : SL_NONE;
+      uint64_t lp = nl != 0 ? base + hb + 1 : 0;
+      uint32_t f = nl != 0 ? 1u : 0u, cnt = __popc(nl);
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1)
+      {
+        const uint64_t yv = __shfl_up_sync(0xffffffffu, v, d), yl = __shfl_up_sync(0xffffffffu, lp, d);
+        const uint32_t yf = __shfl_up_sync(0xffffffffu, f, d), yc = __shfl_up_sync(0xffffffffu, cnt, d);
+        if (lane >= static_cast<uint32_t>(d))
+        {
+          if (f == 0)
+            v = yv < v ? yv : v;
+          f |= yf;
+          lp = yl > lp ? yl : lp;
+          cnt += yc;
+        }
+      }
+      uint64_t ev = __shfl_up_sync(0xffffffffu, v, 1), el = __shfl_up_sync(0xffffffffu, lp, 1);
+      uint32_t ef = __shfl_up_sync(0xffffffffu, f, 1), ec = __shfl_up_sync(0xffffffffu, cnt, 1);
+      if (lane == 0)
+      {
+        ev = SL_NONE;
+        el = 0;
+        ef = 0;
+        ec = 0;
+      }
+      const uint64_t c_in = ef != 0 ? ev : (first < ev ? first : ev); // positions grow: the minimum is the earliest
+      const uint64_t b_in = el > bol ? el : bol;
+      // the lines that end in my chunk, in order: first match = the carry, else the first selected start on the line
+      uint64_t fb_lane = SL_NONE;
+      uint32_t my_recs = 0;
+      uint64_t my_idx = 0;
+      for (int pass = 0; pass < (EMIT ? 2 : 1); ++pass)
+      {
+        if (EMIT && pass == 1)
+        {
+          const uint32_t ex = warp_excl_scan(my_recs, lane);
+          my_idx = idx0 + ex;
+          idx0 += __shfl_sync(0xffffffffu, ex + my_recs, 31);
+        }
+        uint64_t c = c_in, lb = b_in;
+        uint32_t from = 0, j = 0, mm = nl;
+        while (mm != 0)
+        {
+          const uint32_t k = __ffs(mm) - 1;
+          mm &= mm - 1;
+          const uint32_t seg = sel & ((1u << k) - 1u) & ~((1u << from) - 1u);
+          const uint64_t fm = c != SL_NONE ? c : (seg != 0 ? base + __ffs(seg) - 1 : SL_NONE);
+          if (!EMIT)
+          {
+            if (nl_run == 0 && ec == 0 && j == 0)
+              fb_lane = fm; // the region's first owned line: the final kernel adds what came before
+            else
+              m_run += fm != SL_NONE ? 1u : 0u;
+          }
+          else if ((fm != SL_NONE) != inv)
+          {
+            if (pass == 0)
+              ++my_recs;
+            else
+            {
+              ugx_line rec;
+              rec.line = line0 + ec + j;
+              rec.bol = lb + a.base_offset;
+              rec.eol = base + k + a.base_offset;
+              if (inv)
+              {
+                rec.offset = rec.bol;
+                rec.len = 0;
+                rec.cap = 0;
+              }
+              else
+              {
+                const Stepper step(T, P.ncls, a.stage_table != 0);
+                const uint32_t d = longest_at(t, P, step, fm);
+                rec.offset = fm + a.base_offset;
+                rec.len = d & 0xffffu;
+                rec.cap = d >> 16;
+              }
+              if (my_idx < a.out_cap)
+                a.out[my_idx] = rec;
+              ++my_idx;
+            }
+          }
+          c = SL_NONE;
+          from = k + 1;
+          lb = base + k + 1;
+          ++j;
+        }
+      }
+      if (!EMIT && nl_run == 0)
+      {
+        const uint32_t any = __ballot_sync(0xffffffffu, nl != 0);
+        if (any != 0)
+          fb = __shfl_sync(0xffffffffu, fb_lane, __ffs(any) - 1);
+      }
+      const uint64_t v31 = __shfl_sync(0xffffffffu, v, 31), l31 = __shfl_sync(0xffffffffu, lp, 31);
+      const uint32_t f31 = __shfl_sync(0xffffffffu, f, 31), c31 = __shfl_sync(0xffffffffu, cnt, 31);
+      first = f31 != 0 ? v31 : (first < v31 ? first : v31);
+      bol = l31 > bol ? l31 : bol;
+      nl_run += c31;
+      line0 += c31;
+    }
+    if (!EMIT)
+    {
+      const uint32_t m_tot = __reduce_add_sync(0xffffffffu, m_run);
+      if (lane == 0)
+      {
+        a.reg_nl[r] = nl_run;
+        a.reg_m[r] = m_tot;
+        a.reg_bol[r] = bol;
+        a.reg_fb[r] = fb;
+        a.reg_fa[r] = first;
+      }
+    }
+  }
+}
+
+// one CTA over the regions in tiles of blockDim.x: the carries (last newline, first selected start since it) into every
+// region, its number of records (the first owned line matches when it has a selected start before the region's first
+// newline or the carry has one), record and line bases; then the buffer's last line: the line after the last newline
+// when the spans own the end of the buffer, or the set-aside last line (one find_in_line from its start)
+__global__ void __launch_bounds__(1024)
+span_lines_final_kernel(const __grid_constant__ DevPattern P, const uint8_t* __restrict__ buf, uint64_t n, SpanLinesArgs a,
+                        unsigned long long* __restrict__ totals)
+{
+  __shared__ uint64_t s_v[32], s_l[32];
+  __shared__ uint32_t s_f[32];
+  __shared__ uint32_t s_wx[33], s_wy[33];
+  __shared__ uint64_t s_carry[2];
+  const uint64_t limit = a.limit[0];
+  const uint64_t nreg = (limit + SC_REGION - 1) / SC_REGION;
+  const uint32_t tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, B = blockDim.x;
+  uint64_t c_nl = 0, c_rec = 0, c_bol = 0, c_first = SL_NONE; // over the regions before the tile
+  for (uint64_t base = 0; base < nreg; base += B)
+  {
+    const uint64_t i = base + tid;
+    const bool in = i < nreg;
+    const uint64_t nl = in ? a.reg_nl[i] : 0, m = in ? a.reg_m[i] : 0, fb = in ? a.reg_fb[i] : SL_NONE;
+    uint64_t v = in ? a.reg_fa[i] : SL_NONE, l = in ? a.reg_bol[i] : 0;
+    uint32_t f = nl != 0 ? 1u : 0u;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1)
+    {
+      const uint64_t yv = __shfl_up_sync(0xffffffffu, v, d), yl = __shfl_up_sync(0xffffffffu, l, d);
+      const uint32_t yf = __shfl_up_sync(0xffffffffu, f, d);
+      if (lane >= static_cast<uint32_t>(d))
+      {
+        if (f == 0)
+          v = yv < v ? yv : v;
+        f |= yf;
+        l = yl > l ? yl : l;
+      }
+    }
+    if (lane == 31)
+    {
+      s_v[wid] = v;
+      s_l[wid] = l;
+      s_f[wid] = f;
+    }
+    __syncthreads();
+    uint64_t pv = c_first, pl = c_bol; // everything before my warp
+    for (uint32_t w = 0; w < wid; ++w)
+    {
+      pv = s_f[w] != 0 ? s_v[w] : (s_v[w] < pv ? s_v[w] : pv);
+      pl = s_l[w] > pl ? s_l[w] : pl;
+    }
+    uint64_t ev = __shfl_up_sync(0xffffffffu, v, 1), el = __shfl_up_sync(0xffffffffu, l, 1);
+    uint32_t ef = __shfl_up_sync(0xffffffffu, f, 1);
+    if (lane == 0)
+    {
+      ev = SL_NONE;
+      el = 0;
+      ef = 0;
+    }
+    const uint64_t first_in = ef != 0 ? ev : (pv < ev ? pv : ev);
+    const uint64_t bol_in = el > pl ? el : pl;
+    const uint32_t matched = nl == 0 ? 0u : static_cast<uint32_t>(m) + ((fb != SL_NONE || first_in != SL_NONE) ? 1u : 0u);
+    const uint32_t recs = a.invert != 0 ? static_cast<uint32_t>(nl) - matched : matched;
+    uint32_t tx, ty;
+    const uint32_t ex = block_excl_scan(recs, s_wx, &tx);
+    const uint32_t ey = block_excl_scan(static_cast<uint32_t>(nl), s_wy, &ty);
+    if (in)
+    {
+      a.reg_nl[i] = c_nl + ey;
+      a.reg_m[i] = c_rec + ex;
+      a.reg_bol[i] = bol_in;
+      a.reg_fa[i] = first_in;
+    }
+    if (tid == B - 1)
+    {
+      s_carry[0] = f != 0 ? v : (pv < v ? pv : v);
+      s_carry[1] = l > pl ? l : pl;
+    }
+    __syncthreads();
+    c_first = s_carry[0];
+    c_bol = s_carry[1];
+    c_nl += ty;
+    c_rec += tx;
+    __syncthreads();
+  }
+  if (tid == 0)
+  {
+    uint64_t present = 0, tbol = 0, teol = 0, off = SL_NONE, lc = 0, tail_nl = 0;
+    if (limit < n)
+    {
+      // the set-aside last line: the `ugrep -c` loop's first find() from its start
+      Tables T;
+      T.cls = P.cls;
+      T.next = P.next;
+      T.pred = P.pred;
+      T.tap = P.tap;
+      const Text t{buf, n};
+      const CandMap cm{nullptr, 0, 0};
+      Cursor m;
+      set_current(t, m, limit);
+      const uint32_t cap = find_in_line<false>(t, P, T, cm, m, n - 1);
+      tail_nl = buf[n - 1] == '\n' ? 1 : 0;
+      present = 1;
+      tbol = limit;
+      teol = tail_nl != 0 ? n - 1 : n;
+      if (cap != 0)
+      {
+        off = m.txt;
+        lc = (static_cast<uint64_t>(cap) << 32) | m.len;
+      }
+    }
+    else if (n > 0 && buf[n - 1] != '\n')
+    {
+      // an unterminated line the spans own: carried like a region's first line (longest_at runs in the emit pass)
+      present = 1;
+      tbol = c_bol;
+      teol = n;
+      off = c_first;
+      lc = SL_NONE;
+    }
+    const bool rec = present != 0 && (off != SL_NONE) != (a.invert != 0);
+    a.tail[0] = c_nl + 1 + a.base_line;
+    a.tail[1] = tbol;
+    a.tail[2] = teol;
+    a.tail[3] = a.invert != 0 ? tbol : off;
+    a.tail[4] = a.invert != 0 ? 0 : lc;
+    a.tail[5] = c_rec;
+    a.tail[6] = rec ? 1 : 0;
+    totals[0] = c_rec + (rec ? 1 : 0);
+    totals[1] = c_nl + tail_nl;
+  }
+}
+
 // ---- host side ----
 
 bool span_scan_eligible(const DevPattern& P)
@@ -979,6 +1325,41 @@ cudaError_t launch_span_final(const DevPattern& P, const uint8_t* buf, uint64_t 
     span_final_kernel<true><<<1, 32, 0, st>>>(P, buf, n, a, totals); // the last line's records: one thread
   else
     span_final_kernel<false><<<1, 1024, 0, st>>>(P, buf, n, a, totals);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_span_lines(const DevPattern& P, const uint8_t* buf, uint64_t n, SpanLinesArgs a, bool emit, int sm_count,
+                              cudaStream_t st)
+{
+  constexpr int THREADS = 256;
+  // the emit pass runs longest_at once per matching line: the transition table is staged when it fits
+  const bool stage = emit && 256 + UGX_HASH + UGX_BTAP + ((P.table_bytes + 15) / 16) * 16 <= static_cast<uint32_t>(UGX_MAX_DYN_SMEM);
+  const size_t smem = emit ? 256 + UGX_HASH + UGX_BTAP + (stage ? ((P.table_bytes + 15) / 16) * 16 : 0) : 0;
+  a.stage_table = stage ? 1u : 0u;
+  auto kern = emit ? span_lines_kernel<true, THREADS> : span_lines_kernel<false, THREADS>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, UGX_MAX_DYN_SMEM);
+  if (e != cudaSuccess)
+    return e;
+  int per_sm = 1;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, THREADS, smem);
+  if (e != cudaSuccess)
+    return e;
+  if (per_sm < 1)
+    per_sm = 1;
+  uint64_t g = static_cast<uint64_t>(sm_count) * per_sm;
+  const uint64_t need = ((n + SC_REGION - 1) / SC_REGION + THREADS / 32 - 1) / (THREADS / 32);
+  if (g > need)
+    g = need;
+  if (g == 0)
+    g = 1;
+  kern<<<static_cast<int>(g), THREADS, smem, st>>>(P, buf, n, a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_span_lines_final(const DevPattern& P, const uint8_t* buf, uint64_t n, const SpanLinesArgs& a,
+                                    unsigned long long* totals, cudaStream_t st)
+{
+  span_lines_final_kernel<<<1, 1024, 0, st>>>(P, buf, n, a, totals);
   return cudaGetLastError();
 }
 
