@@ -288,6 +288,24 @@ int  ugx_count_newlines(ugx_scanner *s, const void *buf, uint64_t nbytes, ugx_to
 int  ugx_count_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
                      const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, int mode,
                      uint64_t *counts, ugx_totals *totals);
+/*
+ * Records of many files in one launch sequence (`ugrep -rn`, `ugrep -r -o -n -b`, `ugrep -rv` over a source tree).  The
+ * file layout is that of ugx_count_batch.  File i's records are exactly what ugx_find_all / ugx_find_lines (same flags)
+ * return for that file ALONE with base_offset = base_line = 0: offsets are relative to the file's start and line
+ * numbers start at 1 in every file.  The records are grouped by file in file order; first[nfiles + 1] (host) receives
+ * the ranges, file i owning records [first[i], first[i + 1]).  They stay in the scanner's match arena
+ * (ugx_find_all_batch) or line arena (ugx_find_lines_batch), so ugx_scanner_fetch / ugx_scanner_fetch_lines page
+ * through them, and the other arena's last result stays valid.  totals->matches = records, totals->newlines = the
+ * files' '\n' bytes, totals->kernel = UGX_K_BATCH.  out == NULL with cap == 0: the records stay on the device, UGX_OK.
+ * Otherwise n > cap returns UGX_E_OVERFLOW with *n_out and first[] filled, and the records remain fetchable.
+ * nfiles == 0: UGX_OK, first[0] = 0.  A bad file table or any flags bit other than UGX_LINES_INVERT: UGX_E_INVALID.
+ */
+int  ugx_find_all_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                        const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, uint64_t *first,
+                        ugx_match *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
+int  ugx_find_lines_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                          const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, uint32_t flags,
+                          uint64_t *first, ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 
 /* what ugrep asks about a file before it prints from it (Grep::init_is_binary, src/ugrep.cpp:3998-4017):
  * is_utf8 = reflex::isutf8 (lib/simd.cpp:169-421: valid UTF-8 structure, no NUL), has_nul = memchr(buf, 0, n) != NULL;

@@ -31,7 +31,8 @@ ADVANCE_NAMES = ["none", "pin1_one", "pin1_pma", "pin1_pmh", "pin_one", "pin_pma
 EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_version", "ugx_pattern_create", "ugx_pattern_load", "ugx_pattern_info_get",
            "ugx_pattern_destroy", "ugx_scanner_create", "ugx_scanner_destroy", "ugx_count_lines", "ugx_count_matches",
            "ugx_viability_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
-           "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines"]
+           "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines",
+           "ugx_find_all_batch", "ugx_find_lines_batch"]
 
 
 class UgxError(RuntimeError):
@@ -100,6 +101,12 @@ def lib():
         L.ugx_find_lines_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64,
                                             C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         L.ugx_scanner_fetch_lines.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]
+        L.ugx_find_all_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                         C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64),
+                                         C.POINTER(_Totals)]
+        L.ugx_find_lines_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                           C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
+                                           C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         _lib = L
     return _lib
 
@@ -122,6 +129,34 @@ def _buffer(data):
     else:
         a = np.ascontiguousarray(data, dtype=np.uint8)
     return a.ctypes.data, a.size, a
+
+
+def _pack_files(files):
+    """(buffer, begins, lens) of the batch entry points: the files (bytes-like) back to back on 16-byte boundaries in
+    one host buffer, as a batching feeder would pack them; the padding between files is 'X'."""
+    begins = np.zeros(len(files), dtype=np.uint64)
+    lens = np.array([len(f) for f in files], dtype=np.uint64)
+    at = 0
+    for i, f in enumerate(files):
+        begins[i] = at
+        at = (at + len(f) + 15) & ~15
+    pack = np.full(max(at, 16), 0x58, dtype=np.uint8)
+    for i, f in enumerate(files):
+        pack[int(begins[i]):int(begins[i]) + len(f)] = np.frombuffer(bytes(f), dtype=np.uint8)
+    return pack, begins, lens
+
+
+def _batch_input(files):
+    """(pointer, nbytes, keepalive, begins, lens) of a batch: a list of bytes-like packed by _pack_files, or an already
+    packed (buffer, begins, lens) with the buffer as _buffer takes it"""
+    if isinstance(files, tuple):
+        data, begins, lens = files
+        begins = np.ascontiguousarray(begins, dtype=np.uint64)
+        lens = np.ascontiguousarray(lens, dtype=np.uint64)
+    else:
+        data, begins, lens = _pack_files(files)
+    ptr, n, keep = _buffer(data)
+    return C.c_void_p(ptr), n, keep, begins, lens
 
 
 PREFILTER_BYTES = 12 * 4 + 256 + 256 + 2048 + 4096 + 4096 + 32 + 32 + 256
@@ -243,25 +278,48 @@ class Scanner:
         _check(lib().ugx_count_newlines(self._h, C.c_void_p(ptr), n, C.byref(t)))
         return self._totals(t)
 
-    def count_batch(self, pattern: Pattern, files: list, mode: str = "lines"):
+    def count_batch(self, pattern: Pattern, files, mode: str = "lines"):
         """`ugrep -c` / `ugrep -c -o` of many files in ONE launch: (per-file counts, totals).  The files (bytes-like)
-        are packed back to back on 16-byte boundaries into one host buffer, as a batching feeder would."""
-        begins = np.zeros(len(files), dtype=np.uint64)
-        lens = np.array([len(f) for f in files], dtype=np.uint64)
-        at = 0
-        for i, f in enumerate(files):
-            begins[i] = at
-            at = (at + len(f) + 15) & ~15
-        pack = np.full(max(at, 16), 0x58, dtype=np.uint8)
-        for i, f in enumerate(files):
-            pack[int(begins[i]):int(begins[i]) + len(f)] = np.frombuffer(bytes(f), dtype=np.uint8)
-        counts = np.zeros(max(1, len(files)), dtype=np.uint64)
+        are packed back to back on 16-byte boundaries into one host buffer, as a batching feeder would; or `files` is
+        an already packed (buffer, begins, lens) with a host or device buffer."""
+        ptr, n, keep, begins, lens = _batch_input(files)
+        counts = np.zeros(max(1, len(lens)), dtype=np.uint64)
         t = _Totals()
         lib().ugx_count_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                           C.c_uint64, C.c_int, C.c_void_p, C.POINTER(_Totals)]
-        _check(lib().ugx_count_batch(self._h, pattern._h, pack.ctypes.data, pack.size, begins.ctypes.data, lens.ctypes.data,
-                                     len(files), 0 if mode == "lines" else 1, counts.ctypes.data, C.byref(t)))
-        return counts[:len(files)], self._totals(t)
+        _check(lib().ugx_count_batch(self._h, pattern._h, ptr, n, begins.ctypes.data, lens.ctypes.data,
+                                     len(lens), 0 if mode == "lines" else 1, counts.ctypes.data, C.byref(t)))
+        return counts[:len(lens)], self._totals(t)
+
+    def batch_records_device(self, pattern: Pattern, files, lines: bool, invert: bool = False):
+        """ugx_find_lines_batch (lines) or ugx_find_all_batch with the records left on the device: (first, totals);
+        fetch_lines() / fetch() page through them.  `files` is a list of bytes-like, packed as for count_batch, or an
+        already packed (buffer, begins, lens) with a host or device buffer and begins on 16-byte boundaries."""
+        ptr, n, keep, begins, lens = _batch_input(files)
+        first = np.zeros(len(lens) + 1, dtype=np.uint64)
+        cnt = C.c_uint64()
+        t = _Totals()
+        args = (self._h, pattern._h, ptr, n, begins.ctypes.data, lens.ctypes.data, len(lens))
+        if lines:
+            _check(lib().ugx_find_lines_batch(*args, LINES_INVERT if invert else 0, first.ctypes.data, None, 0,
+                                              C.byref(cnt), C.byref(t)))
+        else:
+            _check(lib().ugx_find_all_batch(*args, first.ctypes.data, None, 0, C.byref(cnt), C.byref(t)))
+        return first, self._totals(t)
+
+    def find_all_batch(self, pattern: Pattern, files):
+        """`ugrep -o -n -b` of many files in one launch sequence: (match records, first, totals).  File i's records are
+        rec[first[i]:first[i + 1]], exactly find_all(file i) with offsets and line numbers relative to the file.
+        `files` as for batch_records_device."""
+        first, t = self.batch_records_device(pattern, files, False)
+        return self.fetch(0, t.matches), first, t
+
+    def find_lines_batch(self, pattern: Pattern, files, invert: bool = False):
+        """`ugrep -n` / `ugrep -v -n` of many files in one launch sequence: (line records, first, totals).  File i's
+        records are rec[first[i]:first[i + 1]], exactly find_lines(file i, invert).  `files` as for
+        batch_records_device."""
+        first, t = self.batch_records_device(pattern, files, True, invert)
+        return self.fetch_lines(0, t.matches), first, t
 
     def check_text(self, data) -> dict:
         """reflex::isutf8 / NUL test over the buffer (ugrep's binary-file detection)"""

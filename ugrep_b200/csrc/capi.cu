@@ -1437,6 +1437,202 @@ int ugx_scanner_fetch(ugx_scanner* s, ugx_match* out, uint64_t first, uint64_t c
   return UGX_OK;
 }
 
+} // extern "C"
+
+namespace {
+
+// ---- many files in one launch (ugx_count_batch, ugx_find_all_batch, ugx_find_lines_batch) ----
+// The files lie in one buffer, file f at buf[begins[f], begins[f] + lens[f]); tile g of a launch is tile ti[g] of file
+// tf[g], so the tiles are ordered by file and then by offset.
+struct Batch {
+  std::vector<uint32_t> tf, ti;
+  const uint8_t* dbuf = nullptr;
+  ugx::BatchArgs a;
+};
+
+// the checks of the file table every batch entry point makes, and the tile table; `who` names the entry point
+int batch_tiles(const char* who, uint64_t nbytes, const uint64_t* begins, const uint64_t* lens, uint64_t nfiles, Batch& b)
+{
+  for (uint64_t f = 0; f < nfiles; ++f)
+  {
+    if ((begins[f] & 15) != 0 || begins[f] > nbytes || lens[f] > nbytes - begins[f])
+      return fail(UGX_E_INVALID, std::string(who) + ": file " + std::to_string(f) + " is not a 16-byte aligned range of the buffer");
+    if (nfiles > 0xffffffffull || lens[f] / ugx::SCAN_TILE > 0xfffffffeull)
+      return fail(UGX_E_INVALID, std::string(who) + ": too many files / a file too large for one batch");
+    const uint64_t nt = (lens[f] + ugx::SCAN_TILE - 1) / ugx::SCAN_TILE;
+    for (uint64_t j = 0; j < nt; ++j)
+    {
+      b.tf.push_back(static_cast<uint32_t>(f));
+      b.ti.push_back(static_cast<uint32_t>(j));
+    }
+  }
+  return UGX_OK;
+}
+
+// the buffer made visible to the device, the file and tile tables uploaded and the per-file counters zeroed, all on the
+// scanner's stream: b.a is ready for a launch
+int batch_upload(ugx_scanner* s, const void* buf, uint64_t nbytes, const uint64_t* begins, const uint64_t* lens,
+                 uint64_t nfiles, Batch& b)
+{
+  CU(cudaSetDevice(s->device));
+  uint64_t h2d = 0;
+  int rc = resolve(s, buf, nbytes, &b.dbuf, &h2d);
+  if (rc != UGX_OK)
+    return rc;
+  // one scratch block: begins | lens | counts | tile_file | tile_index
+  const uint64_t words = 3 * nfiles + (b.tf.size() + 1) / 2 * 2;
+  rc = ensure(s->batch, s->batch_cap, words + 4);
+  if (rc != UGX_OK)
+    return rc;
+  uint64_t* d_begins = s->batch;
+  uint64_t* d_lens = d_begins + nfiles;
+  unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(d_lens + nfiles);
+  uint32_t* d_tf = reinterpret_cast<uint32_t*>(d_counts + nfiles);
+  uint32_t* d_ti = d_tf + b.tf.size();
+  CU(cudaMemcpyAsync(d_begins, begins, nfiles * 8, cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemcpyAsync(d_lens, lens, nfiles * 8, cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemsetAsync(d_counts, 0, nfiles * 8, s->stream));
+  CU(cudaMemcpyAsync(d_tf, b.tf.data(), b.tf.size() * 4, cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemcpyAsync(d_ti, b.ti.data(), b.ti.size() * 4, cudaMemcpyHostToDevice, s->stream));
+  b.a.begins = d_begins;
+  b.a.lens = d_lens;
+  b.a.tile_file = d_tf;
+  b.a.tile_index = d_ti;
+  b.a.ntiles = b.tf.size();
+  b.a.counts = d_counts;
+  b.a.stage_table = 0;
+  return UGX_OK;
+}
+
+// match records (lines == false) or line records of a batch: the count pass, the tile prefix, then the per-file counts
+// and the totals to the host in the one synchronise that sizes the arena, and the emit pass into the scanner's match or
+// line arena.  first[nfiles + 1] receives every file's record range, *n_out the number of records.
+int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
+                  const uint64_t* lens, uint64_t nfiles, bool lines, uint32_t flags, uint64_t* first, uint64_t* n_out,
+                  ugx_totals* totals)
+{
+  const char* who = lines ? "ugx_find_lines_batch" : "ugx_find_all_batch";
+  if (s == nullptr || p == nullptr || (buf == nullptr && nbytes != 0) ||
+      (nfiles != 0 && (begins == nullptr || lens == nullptr || first == nullptr)))
+    return fail(UGX_E_INVALID, std::string(who) + ": bad argument");
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
+  if (s->device != p->device)
+    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+  ugx_totals tt;
+  memset(&tt, 0, sizeof(tt));
+  tt.flags = UGX_TOT_NEWLINES;
+  if (totals)
+    *totals = tt;
+  *n_out = 0;
+  if (first != nullptr)
+    first[0] = 0;
+  if (nfiles == 0)
+  {
+    (lines ? s->lines_n : s->records_n) = 0;
+    return UGX_OK;
+  }
+  try
+  {
+    Batch b;
+    int rc = batch_tiles(who, nbytes, begins, lens, nfiles, b);
+    if (rc != UGX_OK)
+      return rc;
+    // the arena is rewritten below: its last result is gone from here on
+    (lines ? s->lines_n : s->records_n) = 0;
+    memset(first, 0, (nfiles + 1) * sizeof(uint64_t));
+    if (b.tf.empty())
+      return UGX_OK; // only empty files: no lines, no records
+    rc = batch_upload(s, buf, nbytes, begins, lens, nfiles, b);
+    if (rc != UGX_OK)
+      return rc;
+    const uint64_t ntiles = b.tf.size();
+    uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
+    rc = ensure(s->tile_matches, cap1, ntiles);
+    if (rc == UGX_OK)
+      rc = ensure(s->tile_newlines, cap2, ntiles);
+    s->tiles_cap = cap1 < cap2 ? cap1 : cap2;
+    if (rc == UGX_OK)
+      rc = ensure(s->strip_counts, s->strips_cap, ntiles * ugx::SCAN_THREADS);
+    if (rc != UGX_OK)
+      return rc;
+    ugx::BatchRecordArgs r;
+    r.tile_matches = s->tile_matches;
+    r.tile_newlines = s->tile_newlines;
+    r.strip_counts = s->strip_counts;
+    r.out = nullptr;
+    r.lout = nullptr;
+    r.out_cap = 0;
+    // a prefilter that admits no candidate (config 3) searches no line: no match records, and the inverted line
+    // records are every line
+    r.lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
+    CU(cudaEventRecord(s->ev0, s->stream));
+    CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, false, s->sm_count, s->stream));
+    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
+    CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(first + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    tt.launches = 2;
+    const uint64_t nrec = s->h_totals[0];
+    for (uint64_t f = 0; f < nfiles; ++f)
+      first[f + 1] += first[f];
+    if (first[nfiles] != nrec)
+      return fail(UGX_E_CUDA, std::string(who) + ": per-file record counts disagree with the total");
+    if (lines)
+      rc = ensure(s->lines, s->lines_cap, nrec);
+    else
+      rc = ensure(s->records, s->records_cap, nrec);
+    if (rc != UGX_OK)
+      return rc;
+    if (nrec > 0)
+    {
+      r.out = lines ? nullptr : s->records;
+      r.lout = lines ? s->lines : nullptr;
+      r.out_cap = nrec;
+      CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, true, s->sm_count, s->stream));
+      tt.launches += 1;
+    }
+    CU(cudaEventRecord(s->ev1, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    (lines ? s->lines_n : s->records_n) = nrec;
+    *n_out = nrec;
+    tt.matches = nrec;
+    tt.newlines = s->h_totals[1];
+    tt.kernel_ms = ms;
+    tt.kernel = UGX_K_BATCH;
+    if (totals)
+      *totals = tt;
+    return UGX_OK;
+  }
+  catch (const std::bad_alloc&)
+  {
+    return fail(UGX_E_NOMEM, "out of host memory");
+  }
+}
+
+// the host side of ugx_find_{all,lines}_batch: out == NULL with cap == 0 leaves the records on the device
+int batch_copy_out(ugx_scanner* s, const void* dev, size_t rec_bytes, void* out, uint64_t cap, uint64_t n)
+{
+  if (out == nullptr && cap == 0)
+    return UGX_OK;
+  if (n > cap)
+    return fail(UGX_E_OVERFLOW, "record buffer too small");
+  if (n > 0)
+  {
+    if (out == nullptr)
+      return fail(UGX_E_INVALID, "null record buffer");
+    CU(cudaMemcpyAsync(out, dev, n * rec_bytes, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+  }
+  return UGX_OK;
+}
+
+} // namespace
+
+extern "C" {
+
 int ugx_count_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                     const uint64_t* lens, uint64_t nfiles, int mode, uint64_t* counts, ugx_totals* totals)
 {
@@ -1453,57 +1649,20 @@ int ugx_count_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint6
     return UGX_OK;
   try
   {
-    // the tile table: tile g of the launch is tile tile_index[g] of file tile_file[g]
-    std::vector<uint32_t> tf, ti;
-    for (uint64_t f = 0; f < nfiles; ++f)
-    {
-      if ((begins[f] & 15) != 0 || begins[f] > nbytes || lens[f] > nbytes - begins[f])
-        return fail(UGX_E_INVALID, "ugx_count_batch: file " + std::to_string(f) + " is not a 16-byte aligned range of the buffer");
-      if (nfiles > 0xffffffffull || lens[f] / ugx::SCAN_TILE > 0xfffffffeull)
-        return fail(UGX_E_INVALID, "ugx_count_batch: too many files / a file too large for one batch");
-      const uint64_t nt = (lens[f] + ugx::SCAN_TILE - 1) / ugx::SCAN_TILE;
-      for (uint64_t j = 0; j < nt; ++j)
-      {
-        tf.push_back(static_cast<uint32_t>(f));
-        ti.push_back(static_cast<uint32_t>(j));
-      }
-    }
+    Batch b;
+    int rc = batch_tiles("ugx_count_batch", nbytes, begins, lens, nfiles, b);
+    if (rc != UGX_OK)
+      return rc;
     memset(counts, 0, nfiles * sizeof(uint64_t));
-    if (tf.empty() || p->never)
+    if (b.tf.empty() || p->never)
       return UGX_OK; // only empty files, or a prefilter that admits no candidate (config 3): nothing matches
-    CU(cudaSetDevice(s->device));
-    const uint8_t* dbuf = nullptr;
-    uint64_t h2d = 0;
-    int rc = resolve(s, buf, nbytes, &dbuf, &h2d);
+    rc = batch_upload(s, buf, nbytes, begins, lens, nfiles, b);
     if (rc != UGX_OK)
       return rc;
-    // one scratch block: begins | lens | counts | tile_file | tile_index
-    const uint64_t words = 3 * nfiles + (tf.size() + 1) / 2 * 2;
-    rc = ensure(s->batch, s->batch_cap, words + 4);
-    if (rc != UGX_OK)
-      return rc;
-    uint64_t* d_begins = s->batch;
-    uint64_t* d_lens = d_begins + nfiles;
-    unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(d_lens + nfiles);
-    uint32_t* d_tf = reinterpret_cast<uint32_t*>(d_counts + nfiles);
-    uint32_t* d_ti = d_tf + tf.size();
-    CU(cudaMemcpyAsync(d_begins, begins, nfiles * 8, cudaMemcpyHostToDevice, s->stream));
-    CU(cudaMemcpyAsync(d_lens, lens, nfiles * 8, cudaMemcpyHostToDevice, s->stream));
-    CU(cudaMemsetAsync(d_counts, 0, nfiles * 8, s->stream));
-    CU(cudaMemcpyAsync(d_tf, tf.data(), tf.size() * 4, cudaMemcpyHostToDevice, s->stream));
-    CU(cudaMemcpyAsync(d_ti, ti.data(), ti.size() * 4, cudaMemcpyHostToDevice, s->stream));
-    ugx::BatchArgs a;
-    a.begins = d_begins;
-    a.lens = d_lens;
-    a.tile_file = d_tf;
-    a.tile_index = d_ti;
-    a.ntiles = tf.size();
-    a.counts = d_counts;
-    a.stage_table = 0;
     CU(cudaEventRecord(s->ev0, s->stream));
-    CU(ugx::launch_scan_batch(p->dev, dbuf, a, mode, s->sm_count, s->stream));
+    CU(ugx::launch_scan_batch(p->dev, b.dbuf, b.a, mode, s->sm_count, s->stream));
     CU(cudaEventRecord(s->ev1, s->stream));
-    CU(cudaMemcpyAsync(counts, d_counts, nfiles * 8, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(counts, b.a.counts, nfiles * 8, cudaMemcpyDeviceToHost, s->stream));
     CU(cudaStreamSynchronize(s->stream));
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
@@ -1520,6 +1679,36 @@ int ugx_count_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint6
   {
     return fail(UGX_E_NOMEM, "out of host memory");
   }
+}
+
+int ugx_find_all_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
+                       const uint64_t* lens, uint64_t nfiles, uint64_t* first, ugx_match* out, uint64_t cap,
+                       uint64_t* n_out, ugx_totals* totals)
+{
+  uint64_t n = 0;
+  if (n_out)
+    *n_out = 0;
+  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, false, 0, first, &n, totals);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  return batch_copy_out(s, s->records, sizeof(ugx_match), out, cap, n);
+}
+
+int ugx_find_lines_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
+                         const uint64_t* lens, uint64_t nfiles, uint32_t flags, uint64_t* first, ugx_line* out,
+                         uint64_t cap, uint64_t* n_out, ugx_totals* totals)
+{
+  uint64_t n = 0;
+  if (n_out)
+    *n_out = 0;
+  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, &n, totals);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  return batch_copy_out(s, s->lines, sizeof(ugx_line), out, cap, n);
 }
 
 int ugx_check_text(ugx_scanner* s, const void* buf, uint64_t nbytes, ugx_text_info* out)

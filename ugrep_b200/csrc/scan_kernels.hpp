@@ -162,6 +162,19 @@ struct BatchArgs {
   uint32_t stage_table;          // set by the launcher
 };
 cudaError_t launch_scan_batch(const DevPattern& P, const uint8_t* buf, BatchArgs a, int mode, int sm_count, cudaStream_t st);
+// records of a batch (batch_records.cu, ugx_find_all_batch / ugx_find_lines_batch): a count pass, launch_tile_prefix over
+// the batch tiles, an emit pass.  a.counts receives the records of every file (count pass).
+struct BatchRecordArgs {
+  uint64_t* tile_matches;   // [ntiles] count pass: records of the tile; after launch_tile_prefix: records before it
+  uint64_t* tile_newlines;  // [ntiles] likewise, newlines
+  uint32_t* strip_counts;   // [ntiles * SCAN_THREADS] records owned by every 64-byte strip of every tile
+  ugx_match* out;           // emit pass: match records (lines == false)
+  ugx_line* lout;           // emit pass: line records (lines == true)
+  uint64_t out_cap;         // emit pass: the total number of records
+  uint32_t lflags;          // UGX_LINES_INVERT | SCAN_LINES_NEVER
+};
+cudaError_t launch_scan_batch_records(const DevPattern& P, const uint8_t* buf, BatchArgs a, const BatchRecordArgs& r,
+                                      bool lines, bool emit, int sm_count, cudaStream_t st);
 
 // reflex::isutf8 / NUL test (utf8_check.cu): flags bit 0 = not UTF-8 by the reference's rule, bit 1 = has a NUL
 cudaError_t launch_utf8_check(const uint8_t* buf, uint64_t n, unsigned int* flags, int sm_count, cudaStream_t st);
