@@ -274,8 +274,27 @@ int  ugx_find_lines_device(ugx_scanner *s, const ugx_pattern *p, const void *buf
 int  ugx_find_lines(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
                     uint64_t base_offset, uint64_t base_line, uint32_t flags,
                     ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
-/* copy `count` line records of the last ugx_find_lines* result, starting at record `first`, to the host */
+/* copy `count` line records of the last ugx_find_lines* / ugx_find_context* result, starting at record `first`, to
+ * the host */
 int  ugx_scanner_fetch_lines(ugx_scanner *s, ugx_line *out, uint64_t first, uint64_t count);
+/*
+ * Context lines (`ugrep -n -A NUM -B NUM -C NUM`, with UGX_LINES_INVERT `ugrep -v -n -C NUM`).  The selected lines are
+ * the records ugx_find_lines returns with the same flags.  A line is printed when some selected line s has
+ * s - before <= line <= s + after; windows stop at the buffer's first and last line (GNU grep's context rule, which
+ * ugrep follows).  One ugx_line per printed line, in input order, none twice; every record is exactly the record
+ * ugx_find_lines gives that line in its own polarity (a matching line carries its first match, a line without one has
+ * offset = bol, len = 0, cap = 0).  So a line is selected iff (cap != 0) != invert, every other record is a context
+ * line (`-` instead of `:`), and a group separator (`--`) goes wherever consecutive records' line numbers are not
+ * consecutive.  before = after = 0 gives ugx_find_lines' result.  *n_out = printed lines, totals->matches = selected
+ * lines; totals->kernel names the route that selected them.  The records live in the line arena
+ * (ugx_scanner_fetch_lines); arguments, errors and paging are those of ugx_find_lines.
+ */
+int  ugx_find_context_device(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                             uint64_t base_offset, uint64_t base_line, uint32_t flags, uint32_t before, uint32_t after,
+                             const ugx_line **dev_out, uint64_t *n_out, ugx_totals *totals);
+int  ugx_find_context(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                      uint64_t base_offset, uint64_t base_line, uint32_t flags, uint32_t before, uint32_t after,
+                      ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 int  ugx_count_newlines(ugx_scanner *s, const void *buf, uint64_t nbytes, ugx_totals *totals);
 
 /*
@@ -306,6 +325,13 @@ int  ugx_find_all_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, u
 int  ugx_find_lines_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
                           const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, uint32_t flags,
                           uint64_t *first, ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
+/* context lines of many files (`ugrep -rn -C NUM PATTERN tree/`): file i's records are exactly what ugx_find_context
+ * returns for that file alone with base_offset = base_line = 0, and context never crosses a file boundary; first[]
+ * gives every file's range of printed lines.  Otherwise as ugx_find_lines_batch. */
+int  ugx_find_context_batch(ugx_scanner *s, const ugx_pattern *p, const void *buf, uint64_t nbytes,
+                            const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, uint32_t flags,
+                            uint32_t before, uint32_t after, uint64_t *first,
+                            ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 
 /* what ugrep asks about a file before it prints from it (Grep::init_is_binary, src/ugrep.cpp:3998-4017):
  * is_utf8 = reflex::isutf8 (lib/simd.cpp:169-421: valid UTF-8 structure, no NUL), has_nul = memchr(buf, 0, n) != NULL;

@@ -32,7 +32,8 @@ EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_ve
            "ugx_pattern_destroy", "ugx_scanner_create", "ugx_scanner_destroy", "ugx_count_lines", "ugx_count_matches",
            "ugx_viability_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
            "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines",
-           "ugx_find_all_batch", "ugx_find_lines_batch"]
+           "ugx_find_all_batch", "ugx_find_lines_batch", "ugx_find_context", "ugx_find_context_device",
+           "ugx_find_context_batch"]
 
 
 class UgxError(RuntimeError):
@@ -107,6 +108,15 @@ def lib():
         L.ugx_find_lines_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                            C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
                                            C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_find_context.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64,
+                                       C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64,
+                                       C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_find_context_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64,
+                                              C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p),
+                                              C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_find_context_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                             C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
+                                             C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         _lib = L
     return _lib
 
@@ -383,6 +393,41 @@ class Scanner:
         (line, bol, eol, offset, len, cap) + totals; with invert the lines without a match (`ugrep -v`)."""
         t = self.find_lines_device(pattern, data, invert, base_offset, base_line)
         return self.fetch_lines(0, self.last_lines[1]), t
+
+    def find_context_device(self, pattern: Pattern, data, before: int = 0, after: int = 0, invert: bool = False,
+                            base_offset: int = 0, base_line: int = 0) -> Totals:
+        """Like find_context but the records stay on the device: self.last_lines = (device pointer, printed lines),
+        and fetch_lines() copies a range to the host.  totals.matches counts the selected lines."""
+        ptr, n, keep = _buffer(data)
+        t = _Totals()
+        dev = C.c_void_p()
+        cnt = C.c_uint64()
+        _check(lib().ugx_find_context_device(self._h, pattern._h, C.c_void_p(ptr), n, base_offset, base_line,
+                                             LINES_INVERT if invert else 0, before, after, C.byref(dev), C.byref(cnt),
+                                             C.byref(t)))
+        self.last_lines = (dev.value, cnt.value)
+        return self._totals(t)
+
+    def find_context(self, pattern: Pattern, data, before: int = 0, after: int = 0, invert: bool = False,
+                     base_offset: int = 0, base_line: int = 0):
+        """`ugrep -n -B before -A after` (with invert `ugrep -v -n ...`): one record per printed line, in input order,
+        each exactly as find_lines gives that line in its own polarity, + totals.  A record is a selected line iff
+        (cap != 0) != invert, otherwise a context line; a gap in the line numbers is a group separator."""
+        t = self.find_context_device(pattern, data, before, after, invert, base_offset, base_line)
+        return self.fetch_lines(0, self.last_lines[1]), t
+
+    def find_context_batch(self, pattern: Pattern, files, before: int = 0, after: int = 0, invert: bool = False):
+        """`ugrep -rn -B before -A after` of many files in one launch sequence: (line records, first, totals).  File
+        i's records are rec[first[i]:first[i + 1]], exactly find_context(file i); context never crosses files.
+        `files` as for batch_records_device."""
+        ptr, n, keep, begins, lens = _batch_input(files)
+        first = np.zeros(len(lens) + 1, dtype=np.uint64)
+        cnt = C.c_uint64()
+        t = _Totals()
+        _check(lib().ugx_find_context_batch(self._h, pattern._h, ptr, n, begins.ctypes.data, lens.ctypes.data,
+                                            len(lens), LINES_INVERT if invert else 0, before, after, first.ctypes.data,
+                                            None, 0, C.byref(cnt), C.byref(t)))
+        return self.fetch_lines(0, cnt.value), first, self._totals(t)
 
     def close(self):
         if self._h:

@@ -148,6 +148,11 @@ struct ugx_scanner {
   uint64_t lines_n = 0;
   uint64_t* lines_regions = nullptr; // [5 * regions + 8] span route: SpanLinesArgs region values and the last line
   uint64_t lines_regions_cap = 0;
+  // context lines (ugx_find_context*): the selected records, swapped out of the line arena, and the count pass scratch
+  ugx_line* ctx_sel = nullptr;
+  uint64_t ctx_sel_cap = 0;
+  uint64_t* ctx_pos = nullptr;   // [nsel] | [2 * blocks] | a batch: fsel, ftile, fout [nfiles + 1] each
+  uint64_t ctx_pos_cap = 0;
 };
 
 extern "C" {
@@ -544,6 +549,8 @@ void ugx_scanner_destroy(ugx_scanner* s)
   cudaFree(s->records);
   cudaFree(s->lines);
   cudaFree(s->lines_regions);
+  cudaFree(s->ctx_sel);
+  cudaFree(s->ctx_pos);
   cudaFree(s->stage);
   if (s->ev0)
     cudaEventDestroy(s->ev0);
@@ -1160,13 +1167,80 @@ int span_lines(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64
   return UGX_OK;
 }
 
-int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint64_t base_offset,
-                      uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals)
+// `-A` / `-B` / `-C`: the context stage over the selected line records in the line arena (context_lines.cu).  The
+// caller fills a's buffer and file fields; the selected records are swapped out of the arena into s->ctx_sel, the
+// count pass and the prefix over its block sums size the arena in one synchronise, and the emit pass writes every
+// printed line to its final slot.  A batch (a.fsel != nullptr on entry: the host's selected-record ranges) gets every
+// file's printed-line range in first_out[nfiles + 1], valid after the caller's next synchronise.
+struct Context {
+  uint32_t before, after;
+};
+
+int context_stage(ugx_scanner* s, const ugx_pattern* p, ugx::ContextArgs& a, const uint64_t* fsel_host,
+                  const std::vector<uint64_t>& ftile_host, uint64_t* first_out, ugx_totals* tt)
 {
+  const uint64_t nsel = s->lines_n;
+  std::swap(s->lines, s->ctx_sel);
+  std::swap(s->lines_cap, s->ctx_sel_cap);
+  s->lines_n = 0;
+  const bool batch = fsel_host != nullptr;
+  const uint64_t nf = batch ? a.nfiles + 1 : 0;
+  if (nsel == 0)
+  {
+    if (batch)
+      memset(first_out, 0, nf * sizeof(uint64_t));
+    return UGX_OK;
+  }
+  const uint64_t nblk = ugx::context_blocks(nsel);
+  int rc = ensure(s->ctx_pos, s->ctx_pos_cap, nsel + 2 * nblk + 3 * nf);
+  if (rc != UGX_OK)
+    return rc;
+  a.sel = s->ctx_sel;
+  a.nsel = nsel;
+  a.pos = s->ctx_pos;
+  a.blk = s->ctx_pos + nsel;
+  if (batch)
+  {
+    uint64_t* d_fsel = a.blk + 2 * nblk;
+    CU(cudaMemcpyAsync(d_fsel, fsel_host, nf * sizeof(uint64_t), cudaMemcpyHostToDevice, s->stream));
+    CU(cudaMemcpyAsync(d_fsel + nf, ftile_host.data(), nf * sizeof(uint64_t), cudaMemcpyHostToDevice, s->stream));
+    a.fsel = d_fsel;
+    a.ftile = d_fsel + nf;
+    a.fout = d_fsel + 2 * nf;
+  }
+  CU(ugx::launch_context_count(a, s->stream));
+  CU(ugx::launch_tile_prefix(a.blk, a.blk + nblk, nblk, s->totals, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals, s->totals, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  tt->launches += 2;
+  const uint64_t nout = s->h_totals[0];
+  rc = ensure(s->lines, s->lines_cap, nout);
+  if (rc != UGX_OK)
+    return rc;
+  a.out = s->lines;
+  a.nout = nout;
+  CU(ugx::launch_context_emit(a, s->sm_count, s->stream));
+  tt->launches += 1;
+  if (a.invert)
+  {
+    CU(ugx::launch_context_match(p->dev, a, s->sm_count, s->stream));
+    tt->launches += 1;
+  }
+  if (batch)
+    CU(cudaMemcpyAsync(first_out, a.fout, nf * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+  s->lines_n = nout;
+  return UGX_OK;
+}
+
+int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint64_t base_offset,
+                      uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals,
+                      const Context* ctx = nullptr)
+{
+  const char* who = ctx ? "ugx_find_context" : "ugx_find_lines";
   if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
     return fail(UGX_E_INVALID, "null argument");
   if ((flags & ~UGX_LINES_INVERT) != 0)
-    return fail(UGX_E_INVALID, "ugx_find_lines: unknown flags");
+    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
   if (s->device != p->device)
     return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
   ugx_totals tt;
@@ -1250,6 +1324,23 @@ int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uin
     tt.newlines = s->h_totals[1];
     tt.kernel = UGX_K_LINE_SCAN;
   }
+  if (ctx != nullptr)
+  {
+    ugx::ContextArgs a;
+    memset(&a, 0, sizeof(a));
+    a.buf = dbuf;
+    a.n = n;
+    a.nl_total = tt.newlines;
+    a.base_offset = base_offset;
+    a.base_line = base_line;
+    a.nfiles = 1;
+    a.before = ctx->before;
+    a.after = ctx->after;
+    a.invert = flags & UGX_LINES_INVERT;
+    rc = context_stage(s, p, a, nullptr, {}, nullptr, &tt);
+    if (rc != UGX_OK)
+      return rc;
+  }
   CU(cudaEventRecord(s->ev1, s->stream));
   CU(cudaStreamSynchronize(s->stream));
   float ms = 0;
@@ -1261,6 +1352,30 @@ int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uin
     *dev_out = s->lines;
   if (totals)
     *totals = tt;
+  return UGX_OK;
+}
+
+// ugx_find_lines / ugx_find_context: the records copied to out[cap]
+int find_lines_to_host(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
+                       uint64_t base_line, uint32_t flags, ugx_line* out, uint64_t cap, uint64_t* n_out,
+                       ugx_totals* totals, const Context* ctx)
+{
+  const ugx_line* dev = nullptr;
+  uint64_t n = 0;
+  int rc = find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, &dev, &n, totals, ctx);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  if (n > cap)
+    return fail(UGX_E_OVERFLOW, "line record buffer too small");
+  if (n > 0)
+  {
+    if (out == nullptr)
+      return fail(UGX_E_INVALID, "null record buffer");
+    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+  }
   return UGX_OK;
 }
 
@@ -1277,23 +1392,23 @@ int ugx_find_lines_device(ugx_scanner* s, const ugx_pattern* p, const void* buf,
 int ugx_find_lines(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
                    uint64_t base_line, uint32_t flags, ugx_line* out, uint64_t cap, uint64_t* n_out, ugx_totals* totals)
 {
-  const ugx_line* dev = nullptr;
-  uint64_t n = 0;
-  int rc = find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, &dev, &n, totals);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  if (n > cap)
-    return fail(UGX_E_OVERFLOW, "line record buffer too small");
-  if (n > 0)
-  {
-    if (out == nullptr)
-      return fail(UGX_E_INVALID, "null record buffer");
-    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-  }
-  return UGX_OK;
+  return find_lines_to_host(s, p, buf, nbytes, base_offset, base_line, flags, out, cap, n_out, totals, nullptr);
+}
+
+int ugx_find_context_device(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
+                            uint64_t base_line, uint32_t flags, uint32_t before, uint32_t after, const ugx_line** dev_out,
+                            uint64_t* n_out, ugx_totals* totals)
+{
+  const Context ctx{before, after};
+  return find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, dev_out, n_out, totals, &ctx);
+}
+
+int ugx_find_context(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, uint64_t base_offset,
+                     uint64_t base_line, uint32_t flags, uint32_t before, uint32_t after, ugx_line* out, uint64_t cap,
+                     uint64_t* n_out, ugx_totals* totals)
+{
+  const Context ctx{before, after};
+  return find_lines_to_host(s, p, buf, nbytes, base_offset, base_line, flags, out, cap, n_out, totals, &ctx);
 }
 
 int ugx_scanner_fetch_lines(ugx_scanner* s, ugx_line* out, uint64_t first, uint64_t count)
@@ -1509,9 +1624,9 @@ int batch_upload(ugx_scanner* s, const void* buf, uint64_t nbytes, const uint64_
 // line arena.  first[nfiles + 1] receives every file's record range, *n_out the number of records.
 int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                   const uint64_t* lens, uint64_t nfiles, bool lines, uint32_t flags, uint64_t* first, uint64_t* n_out,
-                  ugx_totals* totals)
+                  ugx_totals* totals, const Context* ctx = nullptr)
 {
-  const char* who = lines ? "ugx_find_lines_batch" : "ugx_find_all_batch";
+  const char* who = ctx ? "ugx_find_context_batch" : lines ? "ugx_find_lines_batch" : "ugx_find_all_batch";
   if (s == nullptr || p == nullptr || (buf == nullptr && nbytes != 0) ||
       (nfiles != 0 && (begins == nullptr || lens == nullptr || first == nullptr)))
     return fail(UGX_E_INVALID, std::string(who) + ": bad argument");
@@ -1546,6 +1661,14 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
     rc = batch_upload(s, buf, nbytes, begins, lens, nfiles, b);
     if (rc != UGX_OK)
       return rc;
+    // with context, first[] receives the printed lines' ranges and the selected records' ranges go to sfirst
+    std::vector<uint64_t> ctx_first;
+    uint64_t* sfirst = first;
+    if (ctx != nullptr)
+    {
+      ctx_first.assign(nfiles + 1, 0);
+      sfirst = ctx_first.data();
+    }
     const uint64_t ntiles = b.tf.size();
     uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
     rc = ensure(s->tile_matches, cap1, ntiles);
@@ -1570,13 +1693,14 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
     CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, false, s->sm_count, s->stream));
     CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
     CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaMemcpyAsync(first + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(sfirst + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
     CU(cudaStreamSynchronize(s->stream));
     tt.launches = 2;
     const uint64_t nrec = s->h_totals[0];
+    const uint64_t nl_total = s->h_totals[1];
     for (uint64_t f = 0; f < nfiles; ++f)
-      first[f + 1] += first[f];
-    if (first[nfiles] != nrec)
+      sfirst[f + 1] += sfirst[f];
+    if (sfirst[nfiles] != nrec)
       return fail(UGX_E_CUDA, std::string(who) + ": per-file record counts disagree with the total");
     if (lines)
       rc = ensure(s->lines, s->lines_cap, nrec);
@@ -1592,14 +1716,36 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
       CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, true, s->sm_count, s->stream));
       tt.launches += 1;
     }
+    (lines ? s->lines_n : s->records_n) = nrec;
+    if (ctx != nullptr)
+    {
+      // every file's first batch tile: the tiles are ordered by file
+      std::vector<uint64_t> ftile(nfiles + 1, 0);
+      for (uint64_t f = 0; f < nfiles; ++f)
+        ftile[f + 1] = ftile[f] + (lens[f] + ugx::SCAN_TILE - 1) / ugx::SCAN_TILE;
+      ugx::ContextArgs c;
+      memset(&c, 0, sizeof(c));
+      c.buf = b.dbuf;
+      c.nl_total = nl_total;
+      c.nfiles = nfiles;
+      c.begins = b.a.begins;
+      c.lens = b.a.lens;
+      c.tile_nl = s->tile_newlines;
+      c.ntiles = ntiles;
+      c.before = ctx->before;
+      c.after = ctx->after;
+      c.invert = flags & UGX_LINES_INVERT;
+      rc = context_stage(s, p, c, sfirst, ftile, first, &tt);
+      if (rc != UGX_OK)
+        return rc;
+    }
     CU(cudaEventRecord(s->ev1, s->stream));
     CU(cudaStreamSynchronize(s->stream));
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    (lines ? s->lines_n : s->records_n) = nrec;
-    *n_out = nrec;
+    *n_out = lines ? s->lines_n : s->records_n;
     tt.matches = nrec;
-    tt.newlines = s->h_totals[1];
+    tt.newlines = nl_total;
     tt.kernel_ms = ms;
     tt.kernel = UGX_K_BATCH;
     if (totals)
@@ -1704,6 +1850,22 @@ int ugx_find_lines_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, 
   if (n_out)
     *n_out = 0;
   const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, &n, totals);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  return batch_copy_out(s, s->lines, sizeof(ugx_line), out, cap, n);
+}
+
+int ugx_find_context_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
+                           const uint64_t* lens, uint64_t nfiles, uint32_t flags, uint32_t before, uint32_t after,
+                           uint64_t* first, ugx_line* out, uint64_t cap, uint64_t* n_out, ugx_totals* totals)
+{
+  uint64_t n = 0;
+  if (n_out)
+    *n_out = 0;
+  const Context ctx{before, after};
+  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, &n, totals, &ctx);
   if (rc != UGX_OK)
     return rc;
   if (n_out)

@@ -176,6 +176,41 @@ struct BatchRecordArgs {
 cudaError_t launch_scan_batch_records(const DevPattern& P, const uint8_t* buf, BatchArgs a, const BatchRecordArgs& r,
                                       bool lines, bool emit, int sm_count, cudaStream_t st);
 
+// ---- context lines (context_lines.cu, ugx_find_context / ugx_find_context_batch: `-A` / `-B` / `-C`) ----
+// The selected line records of ugx_find_lines[_batch] in, one record per printed line out: a count pass (printed lines
+// every selected record owns), launch_tile_prefix over the count pass's block sums, an emit pass, and under
+// UGX_LINES_INVERT a pass that gives every context line its first match.
+constexpr uint32_t CTX_PER_BLOCK = 4096; // selected records per block of the count pass
+struct ContextArgs {
+  const ugx_line* sel;      // [nsel] selected records, grouped by file, in input order
+  uint64_t nsel;
+  const uint8_t* buf;       // the buffer (one buffer) or the batch buffer
+  uint64_t n;               // one buffer: its size
+  uint64_t nl_total;        // newlines of the buffer / of all files of the batch
+  uint64_t base_offset, base_line; // one buffer; 0 for a batch
+  // a batch (fsel == nullptr: one buffer): the file table of BatchArgs, every file's selected records
+  // [fsel[f], fsel[f + 1]) and first batch tile ftile[f], and the exclusive newline prefix of the batch tiles
+  uint64_t nfiles;
+  const uint64_t* begins;
+  const uint64_t* lens;
+  const uint64_t* fsel;     // [nfiles + 1]
+  const uint64_t* ftile;    // [nfiles + 1]
+  const uint64_t* tile_nl;  // [ntiles]
+  uint64_t ntiles;
+  uint32_t before, after;
+  uint32_t invert;          // UGX_LINES_INVERT: context lines are matching lines and carry their first match
+  uint64_t* pos;            // [nsel] count pass: printed lines before record i within its block
+  uint64_t* blk;            // [2 * blocks] count pass: printed lines of every block (then zeros); after the prefix: before it
+  ugx_line* out;            // emit pass: [nout] records in input order
+  uint64_t nout;
+  uint64_t* fout;           // emit pass, a batch: [nfiles + 1] every file's first printed line, or nullptr
+};
+uint64_t context_blocks(uint64_t nsel);
+cudaError_t launch_context_count(const ContextArgs& a, cudaStream_t st);
+cudaError_t launch_context_emit(const ContextArgs& a, int sm_count, cudaStream_t st);
+// under UGX_LINES_INVERT, after the emit pass: the first match of every context line
+cudaError_t launch_context_match(const DevPattern& P, const ContextArgs& a, int sm_count, cudaStream_t st);
+
 // reflex::isutf8 / NUL test (utf8_check.cu): flags bit 0 = not UTF-8 by the reference's rule, bit 1 = has a NUL
 cudaError_t launch_utf8_check(const uint8_t* buf, uint64_t n, unsigned int* flags, int sm_count, cudaStream_t st);
 
