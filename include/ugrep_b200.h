@@ -177,7 +177,7 @@ typedef struct ugx_totals {
 /* scan kernels (reported in ugx_totals.kernel; DESIGN.md section 4) */
 enum { UGX_K_NONE = 0, UGX_K_STREAM_LITERAL = 1, UGX_K_STREAM_DFA = 2, UGX_K_TILE_ANY = 3, UGX_K_LINE_SCAN = 4,
        UGX_K_RECORDS = 5, UGX_K_NEWLINES = 6, UGX_K_MATCH_LINES = 7, UGX_K_SPAN = 8, UGX_K_BATCH = 9,
-       UGX_K_SPAN_LINES = 10 };
+       UGX_K_SPAN_LINES = 10, UGX_K_STREAM_SEARCH = 11 };
 
 const char *ugx_last_error(void);
 const char *ugx_kernel_name(uint32_t id);
@@ -223,6 +223,27 @@ int  ugx_plan_describe(const uint32_t *opc, uint32_t nop, const ugx_prefilter *p
 int  ugx_viability_describe(const uint32_t *opc, uint32_t nop, uint32_t *k, uint32_t *stride, uint32_t *t01, uint32_t *t23,
                             uint8_t *pair, uint32_t cap_pair, uint32_t *npair,
                             uint32_t *bits, uint32_t cap_words, uint32_t *words);
+/* host only: the line-resetting search automaton that `-c` runs in count_lines_search_kernel (csrc/pattern_host.hpp
+ * SearchDfa, DESIGN.md 4.3a).  A state is MATCHED or the set of anchored DFA states of the line's still undecided
+ * attempts; per byte: state = table[state + cls[byte]], success = (state == 0); the empty set is state offset `classes`.
+ * out->eligible = 1 when `-c` takes the kernel (scanner option "no_search" aside); else out->refusal says why
+ * (UGX_SEARCH_*).  cls[256] and table[cap] (u16 pre-multiplied row offsets, states * classes entries) are filled
+ * when the automaton was built (refusal UGX_SEARCH_OK or UGX_SEARCH_ROUTE) and the pointers are not NULL;
+ * UGX_E_OVERFLOW when cap is too small. */
+enum { UGX_SEARCH_OK = 0, UGX_SEARCH_META = 1, UGX_SEARCH_ACC0 = 2, UGX_SEARCH_CYCLE = 3, UGX_SEARCH_DEPTH = 4,
+       UGX_SEARCH_NEWLINE = 5, UGX_SEARCH_SIZE = 6, UGX_SEARCH_ROUTE = 7 };
+typedef struct ugx_search_info {
+  uint32_t eligible;
+  uint32_t refusal;      /* UGX_SEARCH_*: META edges, accepting start state, cyclic or too deep undecided graph,
+                            a live '\n' edge, table over 128 KiB, or not on the streaming `-c` DFA route (look-back,
+                            option W, no prefilter, a literal's `one`, a candidate test not proven implied) */
+  uint32_t depth;        /* decision depth D: an attempt has decided after at most D bytes (0 = not bounded) */
+  uint32_t states;       /* minimised, MATCHED and the empty set included */
+  uint32_t classes;
+  uint32_t table_bytes;
+} ugx_search_info;
+int  ugx_search_describe(const uint32_t *opc, uint32_t nop, const ugx_prefilter *pf, uint32_t matcher_flags,
+                         ugx_search_info *out, uint8_t *cls, uint16_t *table, uint32_t cap);
 int  ugx_pattern_info_get(const ugx_pattern *p, ugx_pattern_info *info);
 void ugx_pattern_destroy(ugx_pattern *p);
 
@@ -238,7 +259,9 @@ void ugx_scanner_destroy(ugx_scanner *s);
  *   "two_pass_records" records by a count pass + an emit pass instead of the single-pass staging form
  *   "no_pipeline"     host buffers: one copy, then the scan (default: chunked copy overlapped with the scan)
  *   "no_feeder"       pageable host buffers take one plain cudaMemcpyAsync instead of the feeder threads
- *   "no_span"         counting matches / records take the line-at-a-time kernels instead of the span kernels */
+ *   "no_span"         counting matches / records take the line-at-a-time kernels instead of the span kernels
+ *   "no_search"       `-c` keeps count_lines_stream_kernel where the search automaton (count_lines_search_kernel,
+ *                     ugx_search_describe) applies */
 int  ugx_scanner_set_option(ugx_scanner *s, const char *name, int value);
 
 /*

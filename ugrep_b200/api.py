@@ -30,7 +30,7 @@ ADVANCE_NAMES = ["none", "pin1_one", "pin1_pma", "pin1_pmh", "pin_one", "pin_pma
 
 EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_version", "ugx_pattern_create", "ugx_pattern_load", "ugx_pattern_info_get",
            "ugx_pattern_destroy", "ugx_scanner_create", "ugx_scanner_destroy", "ugx_count_lines", "ugx_count_matches",
-           "ugx_viability_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
+           "ugx_viability_describe", "ugx_search_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
            "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines",
            "ugx_find_all_batch", "ugx_find_lines_batch", "ugx_find_context", "ugx_find_context_device",
            "ugx_find_context_batch"]

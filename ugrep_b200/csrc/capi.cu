@@ -142,6 +142,7 @@ struct ugx_scanner {
   uint64_t batch_cap = 0;
   bool no_span = false;           // counting matches / records take the line-at-a-time kernels (A/B timing, tests)
   bool no_cover = false;          // the streaming count evaluates the candidate predicate even where it is proven implied
+  bool no_search = false;         // `-c` keeps count_lines_stream_kernel where the search automaton applies (A/B, tests)
   // line records (ugx_find_lines*): an arena of their own, so that they and the match records stay valid side by side
   ugx_line* lines = nullptr;
   uint64_t lines_cap = 0;
@@ -162,6 +163,17 @@ int ugx_abi_version(void) { return UGX_ABI_VERSION; }
 
 static int pattern_create_impl(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, int device,
                                ugx_pattern** out);
+
+// the search automaton of `-c` (stream_search.cu), built when the attempt semantics allow it and then kept only on the
+// streaming `-c` DFA route where DevPattern::covers makes "a line counts iff some position in it starts a match" exact
+static void plan_search(const ugx::HostDfa& dfa, const ugx_prefilter& pf, uint32_t matcher_flags, int adv, bool covers,
+                        ugx::SearchDfa& sd)
+{
+  ugx::build_search_dfa(dfa, sd);
+  if (sd.refusal == UGX_SEARCH_OK &&
+      (pf.lbk != 0 || (matcher_flags & UGX_OPT_W) != 0 || adv == UGX_ADV_NONE || pf.one != 0 || !covers))
+    sd.refusal = UGX_SEARCH_ROUTE;
+}
 
 // no C++ exception may cross the C ABI: allocation failures inside the export become status codes
 int ugx_pattern_create(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, int device,
@@ -233,6 +245,8 @@ static int pattern_create_impl(const uint32_t* opc, uint32_t nop, const ugx_pref
   d.acc0 = p->dfa.accept[0] != 0;
   ugx::plan_filter(*pf, p->adv, d.plan);
   d.covers = ugx::prefilter_covers_matches(p->dfa, *pf, p->adv, matcher_flags) ? 1u : 0u;
+  ugx::SearchDfa sd;
+  plan_search(p->dfa, *pf, matcher_flags, p->adv, d.covers != 0, sd);
   d.n_word_ranges = sizeof(k_word_ranges) / sizeof(int) / 2;
   memcpy(d.chr, pf->chr, 256);
   set256(d.cbk, pf->cbk);
@@ -305,6 +319,24 @@ static int pattern_create_impl(const uint32_t* opc, uint32_t nop, const ugx_pref
   if (rc == UGX_OK) { p->allocs.push_back(d_vids); rc = upload(d_vbits, via.bits.data(), via.bits.size() * 4); }
   if (rc == UGX_OK) { p->allocs.push_back(d_vbits); rc = upload(d_vpair, via.pair.data(), via.pair.size()); }
   if (rc == UGX_OK) p->allocs.push_back(d_vpair);
+  uint8_t* d_scls = nullptr;
+  uint16_t* d_snext = nullptr;
+  if (rc == UGX_OK && sd.refusal == UGX_SEARCH_OK)
+  {
+    sd.next.resize((sd.next.size() + 7) / 8 * 8, 0); // whole 16-byte units for the bulk copy into shared memory
+    rc = upload(d_scls, sd.cls, 256);
+    if (rc == UGX_OK) { p->allocs.push_back(d_scls); rc = upload(d_snext, sd.next.data(), sd.next.size() * 2); }
+    if (rc == UGX_OK)
+    {
+      p->allocs.push_back(d_snext);
+      d.search_ok = 1;
+      d.search_depth = sd.depth;
+      d.search_ncls = sd.ncls;
+      d.search_bytes = static_cast<uint32_t>(sd.next.size() * 2);
+      d.search_cls = d_scls;
+      d.search_next = d_snext;
+    }
+  }
   if (rc != UGX_OK)
   {
     return rc;
@@ -412,6 +444,48 @@ int ugx_viability_describe(const uint32_t* opc, uint32_t nop, uint32_t* k, uint3
       memcpy(pair, v.pair.data(), v.pair.size());
     if (!v.bits.empty() && bits != nullptr)
       memcpy(bits, v.bits.data(), v.bits.size() * 4);
+    return UGX_OK;
+  }
+  catch (const std::exception&)
+  {
+    return fail(UGX_E_NOMEM, "out of host memory");
+  }
+}
+
+int ugx_search_describe(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags,
+                        ugx_search_info* out, uint8_t* cls, uint16_t* table, uint32_t cap)
+{
+  if (opc == nullptr || nop == 0 || pf == nullptr || out == nullptr)
+    return fail(UGX_E_INVALID, "ugx_search_describe: null argument");
+  try
+  {
+    ugx::HostDfa dfa;
+    std::string err;
+    int rc = ugx::flatten_dfa(opc, nop, dfa, err);
+    if (rc == UGX_OK)
+      rc = ugx::check_scope(dfa, *pf, matcher_flags, err);
+    if (rc != UGX_OK)
+      return fail(rc, err);
+    const int adv = ugx::select_advance(*pf, matcher_flags);
+    ugx::SearchDfa sd;
+    plan_search(dfa, *pf, matcher_flags, adv, ugx::prefilter_covers_matches(dfa, *pf, adv, matcher_flags), sd);
+    memset(out, 0, sizeof(*out));
+    out->eligible = sd.refusal == UGX_SEARCH_OK ? 1u : 0u;
+    out->refusal = sd.refusal;
+    out->depth = sd.depth;
+    out->states = sd.next.empty() ? 0u : sd.nstates;
+    out->classes = sd.next.empty() ? 0u : sd.ncls;
+    out->table_bytes = sd.next.empty() ? 0u : sd.table_bytes();
+    if (sd.next.empty())
+      return UGX_OK;
+    if (cls != nullptr)
+      memcpy(cls, sd.cls, 256);
+    if (table != nullptr)
+    {
+      if (sd.next.size() > cap)
+        return fail(UGX_E_OVERFLOW, "search table larger than the caller's buffer");
+      memcpy(table, sd.next.data(), sd.next.size() * 2);
+    }
     return UGX_OK;
   }
   catch (const std::exception&)
@@ -958,6 +1032,7 @@ int scan_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t 
     sa.use_via = 0;
     sa.no_cover = s->no_cover ? 1u : 0u;
     const uint64_t nreg = ugx::stream_regions(n);
+    const bool search = p->dev.search_ok != 0 && !s->no_search;
     if (pipelined)
     {
       // host buffer: copy in chunks on the copy stream and scan chunk i while chunk i + 1 is in flight.  A launch
@@ -983,7 +1058,8 @@ int scan_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t 
         sa.region_end = upto;
         sa.finalize = upto == nreg ? 1u : 0u;
         sa.accumulate = scanned == 0 ? 0u : 1u;
-        CU(ugx::launch_count_lines_stream(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream));
+        CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream)
+                  : ugx::launch_count_lines_stream(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream));
         scanned = upto;
         ++tt.launches;
       }
@@ -994,10 +1070,13 @@ int scan_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t 
       sa.region_end = nreg;
       sa.finalize = 1;
       sa.accumulate = 0;
-      CU(ugx::launch_count_lines_stream(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream));
+      CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream)
+                : ugx::launch_count_lines_stream(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream));
       tt.launches = 1;
     }
-    tt.kernel = ugx::count_lines_literal_eligible(p->dev) ? UGX_K_STREAM_LITERAL : UGX_K_STREAM_DFA;
+    tt.kernel = ugx::count_lines_literal_eligible(p->dev) ? UGX_K_STREAM_LITERAL
+                : search                                   ? UGX_K_STREAM_SEARCH
+                                                           : UGX_K_STREAM_DFA;
   }
   else if (mode == 0 && !want_records && !s->force_generic && ugx::count_lines_any_eligible(p->dev))
   {
@@ -1469,6 +1548,7 @@ const char* ugx_kernel_name(uint32_t id)
   {
     case UGX_K_STREAM_LITERAL: return "count_lines_literal_kernel";
     case UGX_K_STREAM_DFA: return "count_lines_stream_kernel";
+    case UGX_K_STREAM_SEARCH: return "count_lines_search_kernel";
     case UGX_K_TILE_ANY: return "count_lines_any_kernel";
     case UGX_K_LINE_SCAN: return "scan_lines_kernel";
     case UGX_K_RECORDS: return "scan_records_kernel";
@@ -1528,6 +1608,11 @@ int ugx_scanner_set_option(ugx_scanner* s, const char* name, int value)
   if (strcmp(name, "no_cover") == 0)
   {
     s->no_cover = value != 0;
+    return UGX_OK;
+  }
+  if (strcmp(name, "no_search") == 0)
+  {
+    s->no_search = value != 0;
     return UGX_OK;
   }
   if (strcmp(name, "count_newlines") == 0)

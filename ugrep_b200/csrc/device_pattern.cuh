@@ -46,6 +46,10 @@ struct DevPattern {
   const uint32_t* via_ids;   // [512] t01 / t23 interleaved: one 64-bit lookup per text byte
   const uint32_t* via_bits;  // [via_words] (a multiple of 4 words)
   const uint8_t* via_pair;   // [via_pair_bytes] (a multiple of 16 bytes)
+  // line-resetting search automaton of `-c` (pattern_host.hpp SearchDfa, stream_search.cu); search_ok = 0: not built
+  uint32_t search_ok, search_depth, search_ncls, search_bytes; // search_bytes: the table, padded to 16 bytes
+  const uint8_t* search_cls;    // [256]
+  const uint16_t* search_next;  // [search_bytes / 2] pre-multiplied row offsets, MATCHED = 0
 };
 
 // the tables a kernel actually reads (shared-memory copies when staged, else the global ones)

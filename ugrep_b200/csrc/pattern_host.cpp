@@ -10,6 +10,7 @@
 // range search does (lib/matcher.cpp:467-502).
 #include "pattern_host.hpp"
 
+#include <algorithm>
 #include <cstring>
 #include <map>
 #include <queue>
@@ -339,6 +340,206 @@ int flatten_dfa(const uint32_t* opc, uint32_t nop, HostDfa& out, std::string& er
     }
   }
   return UGX_OK;
+}
+
+// ---- line-resetting search automaton (`-c`) --------------------------------------------------------------
+
+void build_search_dfa(const HostDfa& dfa, SearchDfa& out, uint32_t max_bytes)
+{
+  out = SearchDfa();
+  if (dfa.has_meta)
+  {
+    out.refusal = UGX_SEARCH_META;
+    return;
+  }
+  if (dfa.nstates == 0 || dfa.accept[0] != 0)
+  {
+    out.refusal = UGX_SEARCH_ACC0;
+    return;
+  }
+  const uint32_t ncls = dfa.ncls;
+  // one anchored transition as attempt_table (stream_count.cu) takes it: -1 the attempt fails, -2 it matches, else the
+  // attempt is still undecided in the returned state
+  auto outcome = [&](uint32_t s, uint32_t c) -> int32_t {
+    const uint32_t t = dfa.next[static_cast<size_t>(s) * ncls + c];
+    if (t >= dfa.first_acc)
+    {
+      if (t == DEAD)
+        return -1;
+      if (t < dfa.first_leaf)
+        return -2;
+      return (dfa.accept[t] & 0x7fffffffu) != 0 ? -2 : -1; // a leaf: a match unless it is a dead end
+    }
+    return static_cast<int32_t>(t);
+  };
+
+  // decision depth: the undecided states reachable from the start state must form an acyclic graph; D = its longest path
+  // (in edges) plus one, so an attempt has decided after at most D bytes
+  std::vector<uint8_t> color(dfa.nstates, 0); // 0 unseen, 1 on the DFS stack, 2 done
+  std::vector<uint32_t> longest(dfa.nstates, 0);
+  std::vector<std::pair<uint32_t, uint32_t>> stack{{0u, 0u}};
+  color[0] = 1;
+  while (!stack.empty())
+  {
+    auto& top = stack.back();
+    if (top.second < ncls)
+    {
+      const int32_t o = outcome(top.first, top.second++);
+      if (o < 0)
+        continue;
+      if (color[o] == 1)
+      {
+        out.refusal = UGX_SEARCH_CYCLE;
+        return;
+      }
+      if (color[o] == 0)
+      {
+        color[o] = 1;
+        stack.push_back({static_cast<uint32_t>(o), 0u});
+      }
+      continue;
+    }
+    const uint32_t s = top.first;
+    uint32_t lp = 0;
+    for (uint32_t c = 0; c < ncls; ++c)
+    {
+      const int32_t o = outcome(s, c);
+      if (o >= 0 && longest[o] + 1 > lp)
+        lp = longest[o] + 1;
+    }
+    longest[s] = lp;
+    color[s] = 2;
+    stack.pop_back();
+  }
+  out.depth = longest[0] + 1;
+  if (out.depth > SEARCH_MAX_DEPTH)
+  {
+    out.refusal = UGX_SEARCH_DEPTH;
+    return;
+  }
+  // '\n' must end every undecided attempt without a match (check_scope already rejects live '\n' edges), so that the
+  // reset on '\n' is what the attempts themselves do
+  const uint32_t nlc = dfa.cls[static_cast<uint8_t>('\n')];
+  for (uint32_t s = 0; s < dfa.nstates; ++s)
+    if (color[s] == 2 && outcome(s, nlc) != -1)
+    {
+      out.refusal = UGX_SEARCH_NEWLINE;
+      return;
+    }
+
+  // classes: the anchored ones, '\n' split off when it shares its class (MATCHED resets on '\n' only)
+  bool shared = false;
+  for (uint32_t b = 0; b < 256; ++b)
+    shared = shared || (b != '\n' && dfa.cls[b] == nlc);
+  const uint32_t nc = shared ? ncls + 1 : ncls;
+  if (nc > 256)
+  {
+    out.refusal = UGX_SEARCH_SIZE; // the class map holds bytes
+    return;
+  }
+  const uint32_t nl_class = shared ? ncls : nlc;
+  memcpy(out.cls, dfa.cls, 256);
+  out.cls[static_cast<uint8_t>('\n')] = static_cast<uint8_t>(nl_class);
+
+  // subset construction: state 0 = MATCHED, state 1 = the empty set
+  const uint32_t max_raw = 1u << 18;
+  std::map<std::vector<uint16_t>, uint32_t> id_of;
+  std::vector<std::vector<uint16_t>> sets{{}, {}};
+  std::vector<uint32_t> raw; // [raw states * nc]
+  id_of[{}] = 1;
+  std::vector<uint16_t> nxt;
+  for (uint32_t s = 0; s < sets.size(); ++s)
+  {
+    raw.resize(static_cast<size_t>(sets.size()) * nc, 0);
+    for (uint32_t c = 0; c < nc; ++c)
+    {
+      uint32_t to;
+      if (c == nl_class)
+        to = 1;
+      else if (s == 0)
+        to = 0;
+      else
+      {
+        const uint32_t ac = c == ncls ? nlc : c;
+        bool matched = false;
+        nxt.clear();
+        const int32_t o0 = outcome(0, ac); // the attempt that starts at this byte
+        matched = o0 == -2;
+        if (o0 >= 0)
+          nxt.push_back(static_cast<uint16_t>(o0));
+        for (uint16_t e : sets[s])
+        {
+          const int32_t o = outcome(e, ac);
+          matched = matched || o == -2;
+          if (o >= 0)
+            nxt.push_back(static_cast<uint16_t>(o));
+        }
+        if (matched)
+          to = 0;
+        else
+        {
+          std::sort(nxt.begin(), nxt.end());
+          nxt.erase(std::unique(nxt.begin(), nxt.end()), nxt.end());
+          auto it = id_of.find(nxt);
+          if (it != id_of.end())
+            to = it->second;
+          else
+          {
+            if (sets.size() >= max_raw)
+            {
+              out.refusal = UGX_SEARCH_SIZE;
+              return;
+            }
+            to = static_cast<uint32_t>(sets.size());
+            id_of.emplace(nxt, to);
+            sets.push_back(nxt);
+            raw.resize(static_cast<size_t>(sets.size()) * nc, 0);
+          }
+        }
+      }
+      raw[static_cast<size_t>(s) * nc + c] = to;
+    }
+  }
+  const uint32_t nraw = static_cast<uint32_t>(sets.size());
+
+  // Moore minimisation; MATCHED is alone in its block from the start
+  std::vector<uint32_t> block(nraw), nblock(nraw);
+  for (uint32_t s = 0; s < nraw; ++s)
+    block[s] = s == 0 ? 0u : 1u;
+  uint32_t nblocks = nraw > 1 ? 2 : 1;
+  for (;;)
+  {
+    std::map<std::vector<uint32_t>, uint32_t> sig_id;
+    std::vector<uint32_t> sig(nc + 1);
+    // numbered in state order: MATCHED and the empty set keep blocks 0 and 1
+    auto visit = [&](uint32_t s) {
+      sig[0] = block[s];
+      for (uint32_t c = 0; c < nc; ++c)
+        sig[c + 1] = block[raw[static_cast<size_t>(s) * nc + c]];
+      auto it = sig_id.find(sig);
+      if (it == sig_id.end())
+        it = sig_id.emplace(sig, static_cast<uint32_t>(sig_id.size())).first;
+      nblock[s] = it->second;
+    };
+    for (uint32_t s = 0; s < nraw; ++s)
+      visit(s);
+    const uint32_t nb = static_cast<uint32_t>(sig_id.size());
+    block.swap(nblock);
+    if (nb == nblocks)
+      break;
+    nblocks = nb;
+  }
+  out.nstates = nblocks;
+  out.ncls = nc;
+  if (static_cast<uint64_t>(nblocks) * nc > 65536u || out.table_bytes() > max_bytes)
+  {
+    out.refusal = UGX_SEARCH_SIZE;
+    return;
+  }
+  out.next.assign(static_cast<size_t>(nblocks) * nc, 0);
+  for (uint32_t s = 0; s < nraw; ++s)
+    for (uint32_t c = 0; c < nc; ++c)
+      out.next[static_cast<size_t>(block[s]) * nc + c] = static_cast<uint16_t>(block[raw[static_cast<size_t>(s) * nc + c]] * nc);
 }
 
 // ---- k-gram viability ----------------------------------------------------------------------------------

@@ -64,6 +64,27 @@ struct Viability {
 };
 void build_viability(const HostDfa& dfa, Viability& v, uint32_t max_bits = 1u << 18);
 
+// Line-resetting search automaton for `-c` (stream_search.cu, DESIGN.md §4.3a).  A state is the set of anchored states of
+// the attempts started earlier in the line that are still undecided, or MATCHED once one of them has decided "match" the
+// way attempt_table decides it.  On each byte: add the start state, step every element; '\n' resets to the empty set.
+// A line counts iff the automaton is MATCHED somewhere in it.  Minimised; `next` holds pre-multiplied row offsets
+// (state * ncls) with MATCHED at offset 0 and the empty set at offset ncls, so the device steps by one add and one
+// lookup and tests for success with `== 0`.
+constexpr uint32_t SEARCH_MAX_DEPTH = 16;
+constexpr uint32_t SEARCH_MAX_BYTES = 128 * 1024;
+
+struct SearchDfa {
+  uint32_t refusal = UGX_SEARCH_OK; // UGX_SEARCH_* (include/ugrep_b200.h)
+  uint32_t depth = 0;          // D: the state at x depends only on bytes [x - (D - 1), x) of the line (MATCHED aside)
+  uint32_t nstates = 0;        // minimised, MATCHED and the empty set included
+  uint32_t ncls = 0;           // the anchored DFA's classes, plus one for '\n' when it shares its class
+  uint8_t cls[256] = {0};
+  std::vector<uint16_t> next;  // [nstates * ncls] pre-multiplied row offsets
+  uint32_t table_bytes() const { return nstates * ncls * 2; }
+};
+// fills `out` (refusal = UGX_SEARCH_OK when the automaton applies; the route conditions are the caller's)
+void build_search_dfa(const HostDfa& dfa, SearchDfa& out, uint32_t max_bytes = SEARCH_MAX_BYTES);
+
 // Matcher::init_advance, /root/reference/lib/matcher.cpp:797-954
 int select_advance(const ugx_prefilter& pf, uint32_t matcher_flags);
 

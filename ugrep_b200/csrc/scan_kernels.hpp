@@ -79,6 +79,9 @@ uint64_t stream_regions(uint64_t n);
 int stream_grid(uint64_t n, int sm_count, int per_sm, int threads);
 cudaError_t launch_count_lines_stream(const DevPattern& P, const uint8_t* buf, uint64_t n, StreamArgs a, bool want_nl,
                                       int sm_count, cudaStream_t st);
+// the search-automaton form (stream_search.cu) for DevPattern::search_ok: the same regions, summaries and totals
+cudaError_t launch_count_lines_search(const DevPattern& P, const uint8_t* buf, uint64_t n, const StreamArgs& a, bool want_nl,
+                                      int sm_count, cudaStream_t st);
 // the literal specialisation (stream_literal.cu), taken by launch_count_lines_stream when eligible
 bool count_lines_literal_eligible(const DevPattern& P);
 cudaError_t launch_count_lines_literal(const DevPattern& P, const uint8_t* buf, uint64_t n, const StreamArgs& a, bool want_nl,
