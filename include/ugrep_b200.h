@@ -177,7 +177,7 @@ typedef struct ugx_totals {
 /* scan kernels (reported in ugx_totals.kernel; DESIGN.md section 4) */
 enum { UGX_K_NONE = 0, UGX_K_STREAM_LITERAL = 1, UGX_K_STREAM_DFA = 2, UGX_K_TILE_ANY = 3, UGX_K_LINE_SCAN = 4,
        UGX_K_RECORDS = 5, UGX_K_NEWLINES = 6, UGX_K_MATCH_LINES = 7, UGX_K_SPAN = 8, UGX_K_BATCH = 9,
-       UGX_K_SPAN_LINES = 10, UGX_K_STREAM_SEARCH = 11 };
+       UGX_K_SPAN_LINES = 10, UGX_K_STREAM_SEARCH = 11, UGX_K_BOOL_LINES = 12 };
 
 const char *ugx_last_error(void);
 const char *ugx_kernel_name(uint32_t id);
@@ -319,6 +319,64 @@ int  ugx_find_context(ugx_scanner *s, const ugx_pattern *p, const void *buf, uin
                       uint64_t base_offset, uint64_t base_line, uint32_t flags, uint32_t before, uint32_t after,
                       ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 int  ugx_count_newlines(ugx_scanner *s, const void *buf, uint64_t nbytes, ugx_totals *totals);
+
+/*
+ * Boolean line queries (`ugrep -e A --and -e B`, `A --andnot B`, `--not A`, `--bool 'A|B -C'`; the CNF sub-matchers of
+ * cnf_matching, src/ugrep.cpp:3298-3366).  A query is K compiled patterns, patterns[0..K) with 1 <= K <= 32, plus a
+ * conjunction of clauses.  Each clause is a pair of bit masks:
+ *   pos: bit j: the clause holds on a line on which patterns[j] has a match
+ *   neg: bit j: the clause holds on a line on which patterns[j] has none
+ * M(L), the term mask of a line L: bit j of M(L) is set iff L is one of the matching records that
+ * ugx_find_lines(patterns[j]) returns for the same buffer (equivalently, the `ugrep -c` loop of pattern j counts L).
+ * A line satisfies clause c iff (M(L) & pos) != 0 || (~M(L) & neg) != 0.  A line satisfies the query iff it satisfies
+ * every clause; with nclauses == 0 every line satisfies it.  The selected lines are the lines that satisfy the query;
+ * with UGX_LINES_INVERT they are the lines that do not (`ugrep -v`).  Lines are those of ugx_find_lines: a line is
+ * buf[bol, eol), a buffer that ends in '\n' has no empty line after it, an empty buffer has no lines.
+ *
+ *   ugrep                   clauses
+ *   -e A --and -e B         {pos=A}, {pos=B}
+ *   A --andnot B            {pos=A}, {neg=B}
+ *   --bool 'A|B -C'         {pos=A|B}, {neg=C}
+ *   --not A                 {neg=A}
+ *   -v                      UGX_LINES_INVERT
+ * Turning a query string into clauses (src/cnf.cpp) stays with the caller.
+ *
+ * Records: one ugx_line per selected line, in input order: line 1-based (+ base_line), bol and eol as in ugx_find_lines
+ * (+ base_offset), offset = bol, len = 0, cap = M(L) over all K patterns, including patterns no clause names.  Under
+ * UGX_LINES_INVERT cap is M(L) too and may be 0.  These are NOT ugx_find_lines records: cap is a term mask, not an
+ * accept index.
+ *
+ * Errors, all checked before any device work.  UGX_E_INVALID: a null scanner, pattern array or pattern; a null buf
+ * with nbytes > 0; a null clauses with nclauses > 0; npatterns == 0; a pattern on a different device from the scanner;
+ * a clause with pos == neg == 0 (always false); a mask bit at or above npatterns; any flags bit other than
+ * UGX_LINES_INVERT.  UGX_E_UNSUPPORTED: more than UGX_BOOL_MAX_PATTERNS patterns or more than UGX_BOOL_MAX_CLAUSES
+ * clauses.  UGX_E_OVERFLOW, cap and paging: as in ugx_find_lines (*n_out is set, the records stay fetchable with
+ * ugx_scanner_fetch_lines).
+ *
+ * Totals: matches = selected lines; newlines always counted; UGX_TOT_SPAN_HANDOVER when any term's selection handed
+ * over; launches = every kernel of the call; kernel_ms = the whole call on the device (every term's selection and the
+ * Boolean stage); kernel = UGX_K_BOOL_LINES.
+ *
+ * The records live in the line arena; the last ugx_find_all_device result stays valid.  ugx_count_lines_bool leaves
+ * the line arena with zero records.
+ */
+#define UGX_BOOL_MAX_PATTERNS 32
+#define UGX_BOOL_MAX_CLAUSES  64
+typedef struct ugx_bool_clause {
+  uint32_t pos; /* bit j: the clause holds on a line on which patterns[j] has a match */
+  uint32_t neg; /* bit j: the clause holds on a line on which patterns[j] has none   */
+} ugx_bool_clause;
+int  ugx_count_lines_bool(ugx_scanner *s, const ugx_pattern *const *patterns, uint32_t npatterns,
+                          const ugx_bool_clause *clauses, uint32_t nclauses,
+                          const void *buf, uint64_t nbytes, uint32_t flags, ugx_totals *totals);
+int  ugx_find_lines_bool_device(ugx_scanner *s, const ugx_pattern *const *patterns, uint32_t npatterns,
+                                const ugx_bool_clause *clauses, uint32_t nclauses,
+                                const void *buf, uint64_t nbytes, uint64_t base_offset, uint64_t base_line,
+                                uint32_t flags, const ugx_line **dev_out, uint64_t *n_out, ugx_totals *totals);
+int  ugx_find_lines_bool(ugx_scanner *s, const ugx_pattern *const *patterns, uint32_t npatterns,
+                         const ugx_bool_clause *clauses, uint32_t nclauses,
+                         const void *buf, uint64_t nbytes, uint64_t base_offset, uint64_t base_line,
+                         uint32_t flags, ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 
 /*
  * Many files in one launch: what the reference's per-file job queue feeds its workers (GrepMaster::submit /

@@ -33,7 +33,7 @@ EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_ve
            "ugx_viability_describe", "ugx_search_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
            "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines",
            "ugx_find_all_batch", "ugx_find_lines_batch", "ugx_find_context", "ugx_find_context_device",
-           "ugx_find_context_batch"]
+           "ugx_find_context_batch", "ugx_count_lines_bool", "ugx_find_lines_bool", "ugx_find_lines_bool_device"]
 
 
 class UgxError(RuntimeError):
@@ -45,6 +45,38 @@ class UgxError(RuntimeError):
 class _Totals(C.Structure):
     _fields_ = [("matches", C.c_uint64), ("newlines", C.c_uint64), ("flags", C.c_uint64),
                 ("kernel_ms", C.c_float), ("launches", C.c_uint32), ("kernel", C.c_uint32)]
+
+
+class BoolClause(C.Structure):
+    """ugx_bool_clause: the clause holds on a line on which a pattern of `pos` has a match or one of `neg` has none"""
+    _fields_ = [("pos", C.c_uint32), ("neg", C.c_uint32)]
+
+
+BOOL_MAX_PATTERNS = 32
+
+
+def bool_clauses(cnf):
+    """The ugx_bool_clause array of a CNF written as a list of clauses, each a list of ints: j = pattern j has a match
+    on the line, ~j = pattern j has none.  `-e A --and -e B` is [[0], [1]], `A --andnot B` is [[0], [~1]], `--bool
+    'A|B -C'` is [[0, 1], [~2]].  Malformed input (not a list of non-empty lists of ints in [-32, 31]) raises
+    ValueError; whether a pattern index exists is checked by the library against its pattern count."""
+    if not isinstance(cnf, (list, tuple)):
+        raise ValueError("a CNF is a list of clauses")
+    out = (BoolClause * len(cnf))()
+    for c, clause in enumerate(cnf):
+        if not isinstance(clause, (list, tuple)) or len(clause) == 0:
+            raise ValueError("clause %d: a clause is a non-empty list of ints" % c)
+        for t in clause:
+            if isinstance(t, bool) or not isinstance(t, (int, np.integer)):
+                raise ValueError("clause %d: %r is not an int" % (c, t))
+            t = int(t)
+            if not -BOOL_MAX_PATTERNS <= t < BOOL_MAX_PATTERNS:
+                raise ValueError("clause %d: %d names no pattern (0..31, or ~0..~31)" % (c, t))
+            if t >= 0:
+                out[c].pos |= 1 << t
+            else:
+                out[c].neg |= 1 << ~t
+    return out
 
 
 class _TextInfo(C.Structure):
@@ -117,6 +149,12 @@ def lib():
         L.ugx_find_context_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                              C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
                                              C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        bool_args = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64]
+        L.ugx_count_lines_bool.argtypes = bool_args + [C.c_uint32, C.POINTER(_Totals)]
+        L.ugx_find_lines_bool_device.argtypes = bool_args + [C.c_uint64, C.c_uint64, C.c_uint32, C.POINTER(C.c_void_p),
+                                                             C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        L.ugx_find_lines_bool.argtypes = bool_args + [C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64,
+                                                      C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         _lib = L
     return _lib
 
@@ -428,6 +466,43 @@ class Scanner:
                                             len(lens), LINES_INVERT if invert else 0, before, after, first.ctypes.data,
                                             None, 0, C.byref(cnt), C.byref(t)))
         return self.fetch_lines(0, cnt.value), first, self._totals(t)
+
+    @staticmethod
+    def _bool_query(patterns, cnf):
+        """(pattern handle array, count, clause array, count) for the ugx_*_lines_bool calls; `cnf` is a CNF as
+        bool_clauses takes it, or an already built BoolClause array"""
+        pats = (C.c_void_p * len(patterns))(*[p._h for p in patterns])
+        clauses = cnf if isinstance(cnf, C.Array) else bool_clauses(cnf)
+        return pats, len(patterns), clauses, len(clauses)
+
+    def count_lines_bool(self, patterns, cnf, data, invert: bool = False) -> Totals:
+        """The number of lines that satisfy the CNF over the patterns' matching lines (`ugrep -c -e A --and -e B`,
+        `--andnot`, `--bool`; with invert `-v`) in totals.matches.  See bool_clauses for the CNF."""
+        ptr, n, keep = _buffer(data)
+        t = _Totals()
+        _check(lib().ugx_count_lines_bool(self._h, *self._bool_query(patterns, cnf), C.c_void_p(ptr), n,
+                                          LINES_INVERT if invert else 0, C.byref(t)))
+        return self._totals(t)
+
+    def find_lines_bool_device(self, patterns, cnf, data, invert: bool = False, base_offset: int = 0,
+                               base_line: int = 0) -> Totals:
+        """Like find_lines_bool but the records stay on the device: self.last_lines = (device pointer, records), and
+        fetch_lines() copies a range to the host."""
+        ptr, n, keep = _buffer(data)
+        t = _Totals()
+        dev = C.c_void_p()
+        cnt = C.c_uint64()
+        _check(lib().ugx_find_lines_bool_device(self._h, *self._bool_query(patterns, cnf), C.c_void_p(ptr), n,
+                                                base_offset, base_line, LINES_INVERT if invert else 0, C.byref(dev),
+                                                C.byref(cnt), C.byref(t)))
+        self.last_lines = (dev.value, cnt.value)
+        return self._totals(t)
+
+    def find_lines_bool(self, patterns, cnf, data, invert: bool = False, base_offset: int = 0, base_line: int = 0):
+        """The lines that satisfy the CNF (with invert: that do not), in input order as LINE_DTYPE records + totals.
+        offset = bol, len = 0, and cap is the line's term mask: bit j set iff patterns[j] matches on the line."""
+        t = self.find_lines_bool_device(patterns, cnf, data, invert, base_offset, base_line)
+        return self.fetch_lines(0, self.last_lines[1]), t
 
     def close(self):
         if self._h:

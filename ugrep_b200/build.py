@@ -17,7 +17,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libugrep_b200.so")
-SOURCES = ["capi.cu", "scan_kernels.cu", "line_records.cu", "records_kernel.cu", "match_lines.cu", "span_scan.cu", "newline_count.cu", "utf8_check.cu", "batch_kernel.cu", "batch_records.cu", "context_lines.cu", "fast_kernels.cu", "stream_count.cu", "stream_literal.cu", "stream_search.cu", "pattern_host.cpp", "sharded.cpp", "literal_compile.cpp", "wordlist_compile.cpp"]
+SOURCES = ["capi.cu", "scan_kernels.cu", "line_records.cu", "records_kernel.cu", "match_lines.cu", "span_scan.cu", "newline_count.cu", "utf8_check.cu", "batch_kernel.cu", "batch_records.cu", "context_lines.cu", "bool_lines.cu", "fast_kernels.cu", "stream_count.cu", "stream_literal.cu", "stream_search.cu", "pattern_host.cpp", "sharded.cpp", "literal_compile.cpp", "wordlist_compile.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

@@ -154,6 +154,11 @@ struct ugx_scanner {
   uint64_t ctx_sel_cap = 0;
   uint64_t* ctx_pos = nullptr;   // [nsel] | [2 * blocks] | a batch: fsel, ftile, fout [nfiles + 1] each
   uint64_t ctx_pos_cap = 0;
+  // Boolean line queries (ugx_*_lines_bool): the term mask of every line, and the count pass's block values + line ends
+  uint32_t* bool_mask = nullptr;
+  uint64_t bool_mask_cap = 0;
+  uint64_t* bool_pos = nullptr;  // [2 * blocks] | [lines]
+  uint64_t bool_pos_cap = 0;
 };
 
 extern "C" {
@@ -625,6 +630,8 @@ void ugx_scanner_destroy(ugx_scanner* s)
   cudaFree(s->lines_regions);
   cudaFree(s->ctx_sel);
   cudaFree(s->ctx_pos);
+  cudaFree(s->bool_mask);
+  cudaFree(s->bool_pos);
   cudaFree(s->stage);
   if (s->ev0)
     cudaEventDestroy(s->ev0);
@@ -1311,48 +1318,23 @@ int context_stage(ugx_scanner* s, const ugx_pattern* p, ugx::ContextArgs& a, con
   return UGX_OK;
 }
 
-int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint64_t base_offset,
-                      uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals,
-                      const Context* ctx = nullptr)
+// the line selection of ugx_find_lines: the span route where it applies, else (or after its hand-over) the line-at-a-time
+// count pass, tile prefix and emit pass.  The records land in s->lines[0, s->lines_n); *tt receives their count, the
+// newlines, the launches, the kernel and the hand-over flag.
+int select_lines(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, uint32_t flags, uint64_t base_offset,
+                 uint64_t base_line, ugx_totals* tt)
 {
-  const char* who = ctx ? "ugx_find_context" : "ugx_find_lines";
-  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
-    return fail(UGX_E_INVALID, "null argument");
-  if ((flags & ~UGX_LINES_INVERT) != 0)
-    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
-  if (s->device != p->device)
-    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
-  tt.flags = UGX_TOT_NEWLINES;
-  if (n_out)
-    *n_out = 0;
-  if (dev_out)
-    *dev_out = nullptr;
-  if (n == 0)
-  {
-    s->lines_n = 0;
-    if (totals)
-      *totals = tt;
-    return UGX_OK;
-  }
-  CU(cudaSetDevice(s->device));
-  const uint8_t* dbuf = nullptr;
-  uint64_t h2d = 0;
-  int rc = resolve(s, buf, n, &dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
-  CU(cudaEventRecord(s->ev0, s->stream));
+  int rc;
   bool done = false;
   if (!p->never && !s->force_generic && !s->no_span && ugx::span_scan_eligible(p->dev))
   {
-    rc = span_lines(s, p, dbuf, n, flags, base_offset, base_line, &tt, &done);
+    rc = span_lines(s, p, dbuf, n, flags, base_offset, base_line, tt, &done);
     if (rc != UGX_OK)
       return rc;
     if (!done)
     {
-      tt.launches = 0; // the line-at-a-time kernels take over
-      tt.flags |= UGX_TOT_SPAN_HANDOVER;
+      tt->launches = 0; // the line-at-a-time kernels take over
+      tt->flags |= UGX_TOT_SPAN_HANDOVER;
     }
   }
   if (!done)
@@ -1387,7 +1369,7 @@ int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uin
     CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
     CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
     CU(cudaStreamSynchronize(s->stream));
-    tt.launches += 2;
+    tt->launches += 2;
     const uint64_t nrec = s->h_totals[0];
     rc = ensure(s->lines, s->lines_cap, nrec);
     if (rc != UGX_OK)
@@ -1396,13 +1378,51 @@ int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uin
     {
       a.out_cap = nrec;
       CU(ugx::launch_scan_line_records(p->dev, a, s->lines, lflags, true, s->sm_count, s->stream));
-      tt.launches += 1;
+      tt->launches += 1;
     }
     s->lines_n = nrec;
-    tt.matches = nrec;
-    tt.newlines = s->h_totals[1];
-    tt.kernel = UGX_K_LINE_SCAN;
+    tt->matches = nrec;
+    tt->newlines = s->h_totals[1];
+    tt->kernel = UGX_K_LINE_SCAN;
   }
+  return UGX_OK;
+}
+
+int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint64_t base_offset,
+                      uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals,
+                      const Context* ctx = nullptr)
+{
+  const char* who = ctx ? "ugx_find_context" : "ugx_find_lines";
+  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
+    return fail(UGX_E_INVALID, "null argument");
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
+  if (s->device != p->device)
+    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+  ugx_totals tt;
+  memset(&tt, 0, sizeof(tt));
+  tt.flags = UGX_TOT_NEWLINES;
+  if (n_out)
+    *n_out = 0;
+  if (dev_out)
+    *dev_out = nullptr;
+  if (n == 0)
+  {
+    s->lines_n = 0;
+    if (totals)
+      *totals = tt;
+    return UGX_OK;
+  }
+  CU(cudaSetDevice(s->device));
+  const uint8_t* dbuf = nullptr;
+  uint64_t h2d = 0;
+  int rc = resolve(s, buf, n, &dbuf, &h2d);
+  if (rc != UGX_OK)
+    return rc;
+  CU(cudaEventRecord(s->ev0, s->stream));
+  rc = select_lines(s, p, dbuf, n, flags, base_offset, base_line, &tt);
+  if (rc != UGX_OK)
+    return rc;
   if (ctx != nullptr)
   {
     ugx::ContextArgs a;
@@ -1458,6 +1478,154 @@ int find_lines_to_host(ugx_scanner* s, const ugx_pattern* p, const void* buf, ui
   return UGX_OK;
 }
 
+// ugx_*_lines_bool: every check before any device work
+int bool_check(const ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns, const ugx_bool_clause* clauses,
+               uint32_t nclauses, const void* buf, uint64_t n, uint32_t flags)
+{
+  if (s == nullptr || patterns == nullptr || (buf == nullptr && n != 0) || (clauses == nullptr && nclauses != 0))
+    return fail(UGX_E_INVALID, "null argument");
+  if (npatterns == 0)
+    return fail(UGX_E_INVALID, "ugx_lines_bool: no patterns");
+  if (npatterns > UGX_BOOL_MAX_PATTERNS || nclauses > UGX_BOOL_MAX_CLAUSES)
+    return fail(UGX_E_UNSUPPORTED, "ugx_lines_bool: more than 32 patterns or 64 clauses");
+  for (uint32_t j = 0; j < npatterns; ++j)
+  {
+    if (patterns[j] == nullptr)
+      return fail(UGX_E_INVALID, "null argument");
+    if (patterns[j]->device != s->device)
+      return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+  }
+  const uint32_t terms = npatterns == 32 ? ~0u : (1u << npatterns) - 1u;
+  for (uint32_t c = 0; c < nclauses; ++c)
+  {
+    if ((clauses[c].pos | clauses[c].neg) == 0)
+      return fail(UGX_E_INVALID, "ugx_lines_bool: an empty clause");
+    if (((clauses[c].pos | clauses[c].neg) & ~terms) != 0)
+      return fail(UGX_E_INVALID, "ugx_lines_bool: a clause names a pattern at or above npatterns");
+  }
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return fail(UGX_E_INVALID, "ugx_lines_bool: unknown flags");
+  return UGX_OK;
+}
+
+// Boolean line queries: every term's matching lines (select_lines, bases 0) marked into one term mask per line, then
+// the clauses (bool_lines.cu).  want_records = false stops after the count (ugx_count_lines_bool).
+int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns, const ugx_bool_clause* clauses,
+                uint32_t nclauses, const void* buf, uint64_t n, uint64_t base_offset, uint64_t base_line, uint32_t flags,
+                bool want_records, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals)
+{
+  int rc = bool_check(s, patterns, npatterns, clauses, nclauses, buf, n, flags);
+  if (rc != UGX_OK)
+    return rc;
+  ugx_totals tt;
+  memset(&tt, 0, sizeof(tt));
+  tt.flags = UGX_TOT_NEWLINES;
+  tt.kernel = UGX_K_BOOL_LINES;
+  if (n_out)
+    *n_out = 0;
+  if (dev_out)
+    *dev_out = nullptr;
+  s->lines_n = 0;
+  if (n == 0)
+  {
+    if (totals)
+      *totals = tt;
+    return UGX_OK;
+  }
+  CU(cudaSetDevice(s->device));
+  const uint8_t* dbuf = nullptr;
+  uint64_t h2d = 0;
+  rc = resolve(s, buf, n, &dbuf, &h2d);
+  if (rc != UGX_OK)
+    return rc;
+  CU(cudaEventRecord(s->ev0, s->stream));
+  uint64_t nlines = 0;
+  for (uint32_t j = 0; j < npatterns; ++j)
+  {
+    ugx_totals t;
+    memset(&t, 0, sizeof(t));
+    rc = select_lines(s, patterns[j], dbuf, n, 0, 0, 0, &t);
+    if (rc != UGX_OK)
+      return rc;
+    tt.launches += t.launches;
+    tt.flags |= t.flags & UGX_TOT_SPAN_HANDOVER;
+    if (j == 0)
+    {
+      uint8_t last = 0;
+      CU(cudaMemcpyAsync(&last, dbuf + n - 1, 1, cudaMemcpyDeviceToHost, s->stream));
+      CU(cudaStreamSynchronize(s->stream));
+      tt.newlines = t.newlines;
+      nlines = t.newlines + (last != '\n' ? 1u : 0u);
+      rc = ensure(s->bool_mask, s->bool_mask_cap, nlines);
+      if (rc != UGX_OK)
+        return rc;
+      CU(cudaMemsetAsync(s->bool_mask, 0, nlines * sizeof(uint32_t), s->stream));
+    }
+    if (s->lines_n > 0)
+    {
+      CU(ugx::launch_bool_mark(s->lines, s->lines_n, s->bool_mask, 1u << j, s->sm_count, s->stream));
+      tt.launches += 1;
+    }
+  }
+  s->lines_n = 0;
+  ugx::BoolQuery q;
+  memset(&q, 0, sizeof(q));
+  for (uint32_t c = 0; c < nclauses; ++c)
+  {
+    q.pos[c] = clauses[c].pos;
+    q.neg[c] = clauses[c].neg;
+  }
+  q.nclauses = nclauses;
+  q.invert = flags & UGX_LINES_INVERT;
+  const uint64_t nlb = ugx::bool_line_blocks(nlines), nreg = want_records ? ugx::bool_regions(n) : 0;
+  const uint64_t nblk = nlb > nreg ? nlb : nreg;
+  rc = ensure(s->bool_pos, s->bool_pos_cap, 2 * nblk + (want_records ? nlines : 0));
+  if (rc != UGX_OK)
+    return rc;
+  ugx::BoolArgs a;
+  memset(&a, 0, sizeof(a));
+  a.buf = dbuf;
+  a.n = n;
+  a.nlines = nlines;
+  a.mask = s->bool_mask;
+  a.blk = s->bool_pos;
+  a.nblocks = nblk;
+  a.want_index = want_records ? 1u : 0u;
+  a.eol = s->bool_pos + 2 * nblk;
+  a.base_offset = base_offset;
+  a.base_line = base_line;
+  CU(ugx::launch_bool_count(a, q, s->stream));
+  CU(ugx::launch_tile_prefix(a.blk, a.blk + nblk, nblk, s->totals, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals, s->totals, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  tt.launches += 2;
+  const uint64_t nsel = s->h_totals[0];
+  tt.matches = nsel;
+  if (want_records && nsel > 0)
+  {
+    rc = ensure(s->lines, s->lines_cap, nsel);
+    if (rc != UGX_OK)
+      return rc;
+    a.out = s->lines;
+    CU(ugx::launch_bool_index(a, s->stream));
+    CU(ugx::launch_bool_emit(a, q, s->stream));
+    tt.launches += 2;
+    s->lines_n = nsel;
+  }
+  CU(cudaEventRecord(s->ev1, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  float ms = 0;
+  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+  tt.kernel_ms = ms;
+  if (n_out)
+    *n_out = s->lines_n;
+  if (dev_out)
+    *dev_out = s->lines;
+  if (totals)
+    *totals = tt;
+  return UGX_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -1488,6 +1656,47 @@ int ugx_find_context(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint
 {
   const Context ctx{before, after};
   return find_lines_to_host(s, p, buf, nbytes, base_offset, base_line, flags, out, cap, n_out, totals, &ctx);
+}
+
+int ugx_count_lines_bool(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns,
+                         const ugx_bool_clause* clauses, uint32_t nclauses, const void* buf, uint64_t nbytes, uint32_t flags,
+                         ugx_totals* totals)
+{
+  return bool_common(s, patterns, npatterns, clauses, nclauses, buf, nbytes, 0, 0, flags, false, nullptr, nullptr, totals);
+}
+
+int ugx_find_lines_bool_device(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns,
+                               const ugx_bool_clause* clauses, uint32_t nclauses, const void* buf, uint64_t nbytes,
+                               uint64_t base_offset, uint64_t base_line, uint32_t flags, const ugx_line** dev_out,
+                               uint64_t* n_out, ugx_totals* totals)
+{
+  return bool_common(s, patterns, npatterns, clauses, nclauses, buf, nbytes, base_offset, base_line, flags, true, dev_out,
+                     n_out, totals);
+}
+
+int ugx_find_lines_bool(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns,
+                        const ugx_bool_clause* clauses, uint32_t nclauses, const void* buf, uint64_t nbytes,
+                        uint64_t base_offset, uint64_t base_line, uint32_t flags, ugx_line* out, uint64_t cap,
+                        uint64_t* n_out, ugx_totals* totals)
+{
+  const ugx_line* dev = nullptr;
+  uint64_t n = 0;
+  int rc = bool_common(s, patterns, npatterns, clauses, nclauses, buf, nbytes, base_offset, base_line, flags, true, &dev,
+                       &n, totals);
+  if (rc != UGX_OK)
+    return rc;
+  if (n_out)
+    *n_out = n;
+  if (n > cap)
+    return fail(UGX_E_OVERFLOW, "line record buffer too small");
+  if (n > 0)
+  {
+    if (out == nullptr)
+      return fail(UGX_E_INVALID, "null record buffer");
+    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+  }
+  return UGX_OK;
 }
 
 int ugx_scanner_fetch_lines(ugx_scanner* s, ugx_line* out, uint64_t first, uint64_t count)
@@ -1557,6 +1766,7 @@ const char* ugx_kernel_name(uint32_t id)
     case UGX_K_SPAN: return "span_scan_kernel";
     case UGX_K_BATCH: return "scan_batch_kernel";
     case UGX_K_SPAN_LINES: return "span_lines_kernel";
+    case UGX_K_BOOL_LINES: return "bool_count_kernel";
     default: return "none";
   }
 }

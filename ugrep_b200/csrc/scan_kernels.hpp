@@ -214,6 +214,39 @@ cudaError_t launch_context_emit(const ContextArgs& a, int sm_count, cudaStream_t
 // under UGX_LINES_INVERT, after the emit pass: the first match of every context line
 cudaError_t launch_context_match(const DevPattern& P, const ContextArgs& a, int sm_count, cudaStream_t st);
 
+// ---- Boolean line queries (bool_lines.cu, ugx_count_lines_bool / ugx_find_lines_bool: `--and`, `--andnot`, `--bool`) ----
+// After every term's selection launch_bool_mark ORs its bit into the term mask of each record's line; then a count pass
+// (selected lines per line block, newlines per byte region), launch_tile_prefix over both, and for records an index
+// pass (every line's end) and an emit pass.
+constexpr uint32_t BOOL_LINES_PER_BLOCK = 8192; // lines per block of the count and emit passes
+constexpr uint32_t BOOL_REGION = 65536;         // bytes per block of the newline count and the index pass
+struct BoolQuery {                              // the clauses, passed by value in the kernel parameters
+  uint32_t pos[UGX_BOOL_MAX_CLAUSES];
+  uint32_t neg[UGX_BOOL_MAX_CLAUSES];
+  uint32_t nclauses;
+  uint32_t invert;                              // UGX_LINES_INVERT: the lines that do not satisfy the query
+};
+struct BoolArgs {
+  const uint8_t* buf;
+  uint64_t n;
+  uint64_t nlines;          // newlines + (last byte != '\n')
+  const uint32_t* mask;     // [nlines] term mask of every line
+  uint64_t* blk;            // [2 * nblocks] count pass: selected lines of line block b | newlines of region b;
+                            //   after the prefix: the same before b
+  uint64_t nblocks;         // grid of the count pass: line blocks, or with want_index the larger of them and the regions
+  uint32_t want_index;      // the count pass also counts newlines per region (records follow)
+  uint64_t* eol;            // [nlines] index pass: offset of every line's '\n' (the buffer end for an unterminated one)
+  ugx_line* out;            // emit pass: [selected lines] in input order
+  uint64_t base_offset, base_line;
+};
+uint64_t bool_line_blocks(uint64_t nlines);
+uint64_t bool_regions(uint64_t n);
+cudaError_t launch_bool_mark(const ugx_line* rec, uint64_t nrec, uint32_t* mask, uint32_t bit, int sm_count,
+                             cudaStream_t st);
+cudaError_t launch_bool_count(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
+cudaError_t launch_bool_index(const BoolArgs& a, cudaStream_t st);
+cudaError_t launch_bool_emit(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
+
 // reflex::isutf8 / NUL test (utf8_check.cu): flags bit 0 = not UTF-8 by the reference's rule, bit 1 = has a NUL
 cudaError_t launch_utf8_check(const uint8_t* buf, uint64_t n, unsigned int* flags, int sm_count, cudaStream_t st);
 
