@@ -42,12 +42,22 @@ int cuda_fail(cudaError_t e, const char* what)
       return cuda_fail(e_, #call);       \
   } while (0)
 
+// a status code other than UGX_OK ends the calling function with it
+#define TRY(call)                        \
+  do                                     \
+  {                                      \
+    const int rc_ = (call);              \
+    if (rc_ != UGX_OK)                   \
+      return rc_;                        \
+  } while (0)
+
 const int k_word_ranges[] = {
 #include "word_ranges.inc"
 };
 
+// a device copy of host[bytes] in `dev`, owned by the pattern's `allocs`
 template <typename T>
-int upload(T*& dev, const void* host, size_t bytes)
+int upload(std::vector<void*>& allocs, const T*& dev, const void* host, size_t bytes)
 {
   void* p = nullptr;
   cudaError_t e = cudaMalloc(&p, bytes ? bytes : 16);
@@ -62,7 +72,8 @@ int upload(T*& dev, const void* host, size_t bytes)
       return cuda_fail(e, "cudaMemcpy");
     }
   }
-  dev = static_cast<T*>(p);
+  allocs.push_back(p);
+  dev = static_cast<const T*>(p);
   return UGX_OK;
 }
 
@@ -71,6 +82,61 @@ void set256(uint32_t* set, const uint8_t* bytes32)
   for (int i = 0; i < 8; ++i)
     set[i] = static_cast<uint32_t>(bytes32[4 * i]) | (static_cast<uint32_t>(bytes32[4 * i + 1]) << 8) |
              (static_cast<uint32_t>(bytes32[4 * i + 2]) << 16) | (static_cast<uint32_t>(bytes32[4 * i + 3]) << 24);
+}
+
+// device scratch of a scanner: grown on demand (by an eighth and 64 elements over the need), freed with the scanner
+template <typename T>
+struct DevBuf {
+  T* p = nullptr;
+  uint64_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { cudaFree(p); }
+  int ensure(uint64_t need)
+  {
+    if (need <= cap)
+      return UGX_OK;
+    if (p != nullptr)
+      cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    uint64_t want = need + need / 8 + 64;
+    void* q = nullptr;
+    cudaError_t e = cudaMalloc(&q, want * sizeof(T));
+    if (e != cudaSuccess)
+    {
+      g_err = std::string("cudaMalloc scratch: ") + cudaGetErrorString(e);
+      return e == cudaErrorMemoryAllocation ? UGX_E_NOMEM : UGX_E_CUDA;
+    }
+    p = static_cast<T*>(q);
+    cap = want;
+    return UGX_OK;
+  }
+  void swap(DevBuf& o)
+  {
+    std::swap(p, o.p);
+    std::swap(cap, o.cap);
+  }
+};
+
+// no C++ exception may cross the C ABI: an allocation failure becomes UGX_E_NOMEM "out of host memory", and any other
+// exception becomes `code` with the exception's text after `who` (who == nullptr: "out of host memory")
+template <typename F>
+int guarded(int code, const char* who, F&& body)
+{
+  try
+  {
+    return body();
+  }
+  catch (const std::bad_alloc&)
+  {
+    return fail(UGX_E_NOMEM, "out of host memory");
+  }
+  catch (const std::exception& ex)
+  {
+    return fail(code, who ? std::string(who) + ": " + ex.what() : std::string("out of host memory"));
+  }
 }
 
 } // namespace
@@ -98,67 +164,51 @@ struct ugx_scanner {
   int sm_count = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   // scratch
-  uint64_t* tile_matches = nullptr;
-  uint64_t* tile_newlines = nullptr;
-  uint64_t tiles_cap = 0;
-  uint32_t* strip_counts = nullptr;
-  uint64_t strips_cap = 0;
-  unsigned long long* totals = nullptr; // device [4]
-  unsigned long long* h_totals = nullptr; // pinned [4]
-  ugx_match* records = nullptr;
-  uint64_t records_cap = 0;
+  DevBuf<uint64_t> tile_matches;
+  DevBuf<uint64_t> tile_newlines;
+  DevBuf<uint32_t> strip_counts;
+  unsigned long long* totals = nullptr; // device [ugx::SLOT_COUNT]
+  unsigned long long* h_totals = nullptr; // pinned [ugx::SLOT_COUNT]
+  DevBuf<ugx_match> records;
   uint64_t records_n = 0;
-  uint8_t* stage = nullptr; // device copy of a host buffer
+  DevBuf<uint8_t> stage; // device copy of a host buffer
   bool force_generic = false; // tests: always take the generic line-scan kernel
   bool legacy_any = false;    // tests / A-B timing: the tile-synchronous count_lines_any kernel instead of the streaming one
   bool count_newlines = false; // the streaming count also counts newlines
   bool match_lines = false;      // counting takes match_lines_kernel (position-parallel attempts) instead of scan_lines_kernel
   bool two_pass_records = false; // records by count pass + emit pass (A/B against the single-pass staging form)
-  uint64_t* tile_base = nullptr;  // staging base of every tile's records
-  uint64_t tile_base_cap = 0;
-  ugx_match* rec_stage = nullptr; // records in tile completion order
-  uint64_t rec_stage_cap = 0;
+  DevBuf<uint64_t> tile_base;    // staging base of every tile's records
+  DevBuf<ugx_match> rec_stage;   // records in tile completion order
   bool no_pipeline = false;    // host buffers: one copy, then the scan (A/B timing of the overlapped path)
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t ev_copy = nullptr;
   bool stream_dfa = false;     // DFA patterns take the streaming count too (default: the tile-synchronous kernel)
   // streaming count scratch
-  uint8_t* region_sum = nullptr;
-  uint64_t region_cap = 0;
+  DevBuf<uint8_t> region_sum;
   unsigned long long* partials = nullptr; // [2 * STREAM_MAX_GRID]
   unsigned long long* ticket = nullptr;   // {ticket (u64), done (u32)}
-  uint64_t stage_cap = 0;
   // span scan scratch
-  uint64_t* span_regions = nullptr; // [5 * regions]
-  uint64_t span_regions_cap = 0;
+  DevBuf<uint64_t> span_regions; // [5 * regions]
   // pageable host buffers: feeder threads copy chunks into pinned slots, each slot goes to the device on its thread's stream
   std::vector<uint8_t*> feed_slots;      // [2 * feed_threads] pinned, FEED_CHUNK bytes each
   std::vector<cudaStream_t> feed_streams; // [feed_threads]
   std::vector<cudaEvent_t> feed_events;   // [2 * feed_threads] slot free again
   bool no_feeder = false;         // pageable buffers take one plain cudaMemcpyAsync (A/B timing)
-  uint16_t* span_sel = nullptr;   // records: selected match starts per 16-byte chunk
-  uint64_t span_sel_cap = 0;
-  uint64_t* batch = nullptr;      // ugx_count_batch: file table, counters, tile table
-  uint64_t batch_cap = 0;
+  DevBuf<uint16_t> span_sel;      // records: selected match starts per 16-byte chunk
+  DevBuf<uint64_t> batch;         // ugx_count_batch: file table, counters, tile table
   bool no_span = false;           // counting matches / records take the line-at-a-time kernels (A/B timing, tests)
   bool no_cover = false;          // the streaming count evaluates the candidate predicate even where it is proven implied
   bool no_search = false;         // `-c` keeps count_lines_stream_kernel where the search automaton applies (A/B, tests)
   // line records (ugx_find_lines*): an arena of their own, so that they and the match records stay valid side by side
-  ugx_line* lines = nullptr;
-  uint64_t lines_cap = 0;
+  DevBuf<ugx_line> lines;
   uint64_t lines_n = 0;
-  uint64_t* lines_regions = nullptr; // [5 * regions + 8] span route: SpanLinesArgs region values and the last line
-  uint64_t lines_regions_cap = 0;
+  DevBuf<uint64_t> lines_regions; // [5 * regions + 8] span route: SpanLinesArgs region values and the last line
   // context lines (ugx_find_context*): the selected records, swapped out of the line arena, and the count pass scratch
-  ugx_line* ctx_sel = nullptr;
-  uint64_t ctx_sel_cap = 0;
-  uint64_t* ctx_pos = nullptr;   // [nsel] | [2 * blocks] | a batch: fsel, ftile, fout [nfiles + 1] each
-  uint64_t ctx_pos_cap = 0;
+  DevBuf<ugx_line> ctx_sel;
+  DevBuf<uint64_t> ctx_pos;      // [nsel] | [2 * blocks] | a batch: fsel, ftile, fout [nfiles + 1] each
   // Boolean line queries (ugx_*_lines_bool): the term mask of every line, and the count pass's block values + line ends
-  uint32_t* bool_mask = nullptr;
-  uint64_t bool_mask_cap = 0;
-  uint64_t* bool_pos = nullptr;  // [2 * blocks] | [lines]
-  uint64_t bool_pos_cap = 0;
+  DevBuf<uint32_t> bool_mask;
+  DevBuf<uint64_t> bool_pos;     // [2 * blocks] | [lines]
 };
 
 extern "C" {
@@ -180,22 +230,10 @@ static void plan_search(const ugx::HostDfa& dfa, const ugx_prefilter& pf, uint32
     sd.refusal = UGX_SEARCH_ROUTE;
 }
 
-// no C++ exception may cross the C ABI: allocation failures inside the export become status codes
 int ugx_pattern_create(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, int device,
                        ugx_pattern** out)
 {
-  try
-  {
-    return pattern_create_impl(opc, nop, pf, matcher_flags, device, out);
-  }
-  catch (const std::bad_alloc&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
-  catch (const std::exception& ex)
-  {
-    return fail(UGX_E_INVALID, std::string("ugx_pattern_create: ") + ex.what());
-  }
+  return guarded(UGX_E_INVALID, "ugx_pattern_create", [&] { return pattern_create_impl(opc, nop, pf, matcher_flags, device, out); });
 }
 
 static int pattern_create_impl(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, int device,
@@ -303,59 +341,26 @@ static int pattern_create_impl(const uint32_t* opc, uint32_t nop, const ugx_pref
   via.pair.resize((via.pair.size() + 15) / 16 * 16 + 16, 0);
   d.via_words = static_cast<uint32_t>(via.bits.size());
   d.via_pair_bytes = static_cast<uint32_t>(via.pair.size());
-  uint32_t* d_vids = nullptr;
-  uint32_t* d_vbits = nullptr;
-  uint8_t* d_vpair = nullptr;
-  uint8_t* d_cls = nullptr;
-  uint16_t* d_next = nullptr;
-  uint32_t* d_acc = nullptr;
-  uint32_t* d_opc = nullptr;
-  uint8_t* d_pred = nullptr;
-  uint8_t* d_tap = nullptr;
-  int* d_words = nullptr;
-  rc = upload(d_cls, p->dfa.cls, 256);
-  if (rc == UGX_OK) { p->allocs.push_back(d_cls); rc = upload(d_next, next.data(), next.size() * 2); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_next); rc = upload(d_acc, acc.data(), acc.size() * 4); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_acc); rc = upload(d_opc, opcp.data(), opcp.size() * 4); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_opc); rc = upload(d_pred, pf->min < 4 ? pf->pma : pf->pmh, UGX_HASH); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_pred); rc = upload(d_tap, pf->tap, UGX_BTAP); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_tap); rc = upload(d_words, k_word_ranges, sizeof(k_word_ranges)); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_words); rc = upload(d_vids, via_t.data(), via_t.size() * 4); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_vids); rc = upload(d_vbits, via.bits.data(), via.bits.size() * 4); }
-  if (rc == UGX_OK) { p->allocs.push_back(d_vbits); rc = upload(d_vpair, via.pair.data(), via.pair.size()); }
-  if (rc == UGX_OK) p->allocs.push_back(d_vpair);
-  uint8_t* d_scls = nullptr;
-  uint16_t* d_snext = nullptr;
-  if (rc == UGX_OK && sd.refusal == UGX_SEARCH_OK)
+  TRY(upload(p->allocs, d.cls, p->dfa.cls, 256));
+  TRY(upload(p->allocs, d.next, next.data(), next.size() * 2));
+  TRY(upload(p->allocs, d.accept, acc.data(), acc.size() * 4));
+  TRY(upload(p->allocs, d.opc, opcp.data(), opcp.size() * 4));
+  TRY(upload(p->allocs, d.pred, pf->min < 4 ? pf->pma : pf->pmh, UGX_HASH));
+  TRY(upload(p->allocs, d.tap, pf->tap, UGX_BTAP));
+  TRY(upload(p->allocs, d.word_ranges, k_word_ranges, sizeof(k_word_ranges)));
+  TRY(upload(p->allocs, d.via_ids, via_t.data(), via_t.size() * 4));
+  TRY(upload(p->allocs, d.via_bits, via.bits.data(), via.bits.size() * 4));
+  TRY(upload(p->allocs, d.via_pair, via.pair.data(), via.pair.size()));
+  if (sd.refusal == UGX_SEARCH_OK)
   {
     sd.next.resize((sd.next.size() + 7) / 8 * 8, 0); // whole 16-byte units for the bulk copy into shared memory
-    rc = upload(d_scls, sd.cls, 256);
-    if (rc == UGX_OK) { p->allocs.push_back(d_scls); rc = upload(d_snext, sd.next.data(), sd.next.size() * 2); }
-    if (rc == UGX_OK)
-    {
-      p->allocs.push_back(d_snext);
-      d.search_ok = 1;
-      d.search_depth = sd.depth;
-      d.search_ncls = sd.ncls;
-      d.search_bytes = static_cast<uint32_t>(sd.next.size() * 2);
-      d.search_cls = d_scls;
-      d.search_next = d_snext;
-    }
+    TRY(upload(p->allocs, d.search_cls, sd.cls, 256));
+    TRY(upload(p->allocs, d.search_next, sd.next.data(), sd.next.size() * 2));
+    d.search_ok = 1;
+    d.search_depth = sd.depth;
+    d.search_ncls = sd.ncls;
+    d.search_bytes = static_cast<uint32_t>(sd.next.size() * 2);
   }
-  if (rc != UGX_OK)
-  {
-    return rc;
-  }
-  d.cls = d_cls;
-  d.next = d_next;
-  d.accept = d_acc;
-  d.opc = d_opc;
-  d.pred = d_pred;
-  d.tap = d_tap;
-  d.word_ranges = d_words;
-  d.via_ids = d_vids;
-  d.via_bits = d_vbits;
-  d.via_pair = d_vpair;
   *out = holder.release();
   return UGX_OK;
 }
@@ -364,18 +369,7 @@ static int plan_describe_impl(const uint32_t* opc, uint32_t nop, const ugx_prefi
 
 int ugx_plan_describe(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, ugx_plan_info* out)
 {
-  try
-  {
-    return plan_describe_impl(opc, nop, pf, matcher_flags, out);
-  }
-  catch (const std::bad_alloc&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
-  catch (const std::exception& ex)
-  {
-    return fail(UGX_E_INVALID, std::string("ugx_plan_describe: ") + ex.what());
-  }
+  return guarded(UGX_E_INVALID, "ugx_plan_describe", [&] { return plan_describe_impl(opc, nop, pf, matcher_flags, out); });
 }
 
 static int plan_describe_impl(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags, ugx_plan_info* out)
@@ -428,8 +422,7 @@ int ugx_viability_describe(const uint32_t* opc, uint32_t nop, uint32_t* k, uint3
   if (opc == nullptr || nop == 0 || k == nullptr || stride == nullptr || t01 == nullptr || t23 == nullptr ||
       npair == nullptr || words == nullptr)
     return fail(UGX_E_INVALID, "ugx_viability_describe: null argument");
-  try
-  {
+  return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     ugx::HostDfa dfa;
     std::string err;
     const int rc = ugx::flatten_dfa(opc, nop, dfa, err);
@@ -450,11 +443,7 @@ int ugx_viability_describe(const uint32_t* opc, uint32_t nop, uint32_t* k, uint3
     if (!v.bits.empty() && bits != nullptr)
       memcpy(bits, v.bits.data(), v.bits.size() * 4);
     return UGX_OK;
-  }
-  catch (const std::exception&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
+  });
 }
 
 int ugx_search_describe(const uint32_t* opc, uint32_t nop, const ugx_prefilter* pf, uint32_t matcher_flags,
@@ -462,8 +451,7 @@ int ugx_search_describe(const uint32_t* opc, uint32_t nop, const ugx_prefilter* 
 {
   if (opc == nullptr || nop == 0 || pf == nullptr || out == nullptr)
     return fail(UGX_E_INVALID, "ugx_search_describe: null argument");
-  try
-  {
+  return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     ugx::HostDfa dfa;
     std::string err;
     int rc = ugx::flatten_dfa(opc, nop, dfa, err);
@@ -492,11 +480,7 @@ int ugx_search_describe(const uint32_t* opc, uint32_t nop, const ugx_prefilter* 
       memcpy(table, sd.next.data(), sd.next.size() * 2);
     }
     return UGX_OK;
-  }
-  catch (const std::exception&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
+  });
 }
 
 int ugx_pattern_load(const char* path, int device, ugx_pattern** out)
@@ -582,9 +566,9 @@ int ugx_scanner_create(int device, void* stream, ugx_scanner** out)
   if (e == cudaSuccess)
     e = cudaEventCreateWithFlags(&s->ev_copy, cudaEventDisableTiming);
   if (e == cudaSuccess)
-    e = cudaMalloc(reinterpret_cast<void**>(&s->totals), 8 * sizeof(unsigned long long));
+    e = cudaMalloc(reinterpret_cast<void**>(&s->totals), ugx::SLOT_COUNT * sizeof(unsigned long long));
   if (e == cudaSuccess)
-    e = cudaMallocHost(reinterpret_cast<void**>(&s->h_totals), 8 * sizeof(unsigned long long));
+    e = cudaMallocHost(reinterpret_cast<void**>(&s->h_totals), ugx::SLOT_COUNT * sizeof(unsigned long long));
   if (e == cudaSuccess)
     e = cudaMalloc(reinterpret_cast<void**>(&s->partials), 2 * ugx::STREAM_MAX_GRID * sizeof(unsigned long long));
   if (e == cudaSuccess)
@@ -605,34 +589,17 @@ void ugx_scanner_destroy(ugx_scanner* s)
 {
   if (s == nullptr)
     return;
-  cudaSetDevice(s->device);
-  cudaFree(s->tile_matches);
-  cudaFree(s->tile_newlines);
-  cudaFree(s->strip_counts);
+  cudaSetDevice(s->device); // the scratch buffers are freed by their destructors in `delete s`
   cudaFree(s->totals);
   cudaFreeHost(s->h_totals);
-  cudaFree(s->region_sum);
-  cudaFree(s->span_regions);
-  cudaFree(s->span_sel);
   for (uint8_t* p : s->feed_slots)
     cudaFreeHost(p);
   for (cudaEvent_t e : s->feed_events)
     cudaEventDestroy(e);
   for (cudaStream_t st : s->feed_streams)
     cudaStreamDestroy(st);
-  cudaFree(s->batch);
-  cudaFree(s->tile_base);
-  cudaFree(s->rec_stage);
   cudaFree(s->partials);
   cudaFree(s->ticket);
-  cudaFree(s->records);
-  cudaFree(s->lines);
-  cudaFree(s->lines_regions);
-  cudaFree(s->ctx_sel);
-  cudaFree(s->ctx_pos);
-  cudaFree(s->bool_mask);
-  cudaFree(s->bool_pos);
-  cudaFree(s->stage);
   if (s->ev0)
     cudaEventDestroy(s->ev0);
   if (s->ev1)
@@ -647,28 +614,6 @@ void ugx_scanner_destroy(ugx_scanner* s)
 } // extern "C"
 
 namespace {
-
-template <typename T>
-int ensure(T*& ptr, uint64_t& cap, uint64_t need)
-{
-  if (need <= cap)
-    return UGX_OK;
-  if (ptr != nullptr)
-    cudaFree(ptr);
-  ptr = nullptr;
-  cap = 0;
-  uint64_t want = need + need / 8 + 64;
-  void* p = nullptr;
-  cudaError_t e = cudaMalloc(&p, want * sizeof(T));
-  if (e != cudaSuccess)
-  {
-    g_err = std::string("cudaMalloc scratch: ") + cudaGetErrorString(e);
-    return e == cudaErrorMemoryAllocation ? UGX_E_NOMEM : UGX_E_CUDA;
-  }
-  ptr = static_cast<T*>(p);
-  cap = want;
-  return UGX_OK;
-}
 
 constexpr uint64_t FEED_CHUNK = 8ull << 20; // bytes per pinned slot of the pageable feeder
 constexpr uint64_t FEED_MIN = 32ull << 20;  // smaller pageable buffers take one plain copy
@@ -768,9 +713,8 @@ int feed_pageable(ugx_scanner* s, uint8_t* dst, const uint8_t* src, uint64_t n)
 }
 
 // make `buf` visible to the device: device pointers are used in place, host pointers are staged
-int resolve(ugx_scanner* s, const void* buf, uint64_t n, const uint8_t** dev, uint64_t* h2d)
+int resolve(ugx_scanner* s, const void* buf, uint64_t n, const uint8_t** dev)
 {
-  *h2d = 0;
   cudaPointerAttributes at;
   cudaError_t e = cudaPointerGetAttributes(&at, buf);
   if (e == cudaSuccess && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged))
@@ -781,59 +725,184 @@ int resolve(ugx_scanner* s, const void* buf, uint64_t n, const uint8_t** dev, ui
       return UGX_OK;
     }
     // the kernels use 16-byte vector loads: a misaligned device buffer is copied to aligned scratch
-    int rc = ensure(s->stage, s->stage_cap, n + 16);
-    if (rc != UGX_OK)
-      return rc;
-    CU(cudaMemcpyAsync(s->stage, buf, n, cudaMemcpyDeviceToDevice, s->stream));
-    *dev = s->stage;
+    TRY(s->stage.ensure(n + 16));
+    CU(cudaMemcpyAsync(s->stage.p, buf, n, cudaMemcpyDeviceToDevice, s->stream));
+    *dev = s->stage.p;
     return UGX_OK;
   }
   if (e != cudaSuccess)
     cudaGetLastError(); // plain host memory on older drivers reports an error: clear it
-  int rc = ensure(s->stage, s->stage_cap, n + 16);
-  if (rc != UGX_OK)
-    return rc;
+  TRY(s->stage.ensure(n + 16));
   const bool pageable = e != cudaSuccess || at.type == cudaMemoryTypeUnregistered;
   if (pageable && n >= FEED_MIN && !s->no_feeder)
   {
     // earlier work on the scan stream may still read the staging buffer
     CU(cudaStreamSynchronize(s->stream));
-    rc = feed_pageable(s, s->stage, static_cast<const uint8_t*>(buf), n);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(feed_pageable(s, s->stage.p, static_cast<const uint8_t*>(buf), n));
   }
   else
-    CU(cudaMemcpyAsync(s->stage, buf, n, cudaMemcpyHostToDevice, s->stream));
-  *dev = s->stage;
-  *h2d = n;
+    CU(cudaMemcpyAsync(s->stage.p, buf, n, cudaMemcpyHostToDevice, s->stream));
+  *dev = s->stage.p;
   return UGX_OK;
 }
 
 constexpr uint64_t PIPE_CHUNK = 32ull << 20; // bytes per host-to-device chunk of the pipelined path (region-aligned)
 
-bool is_host_pointer(const void* buf)
+// a host buffer the pipelined path takes: page-locked memory (cudaHostAlloc / cudaHostRegister: DMA reads it
+// directly), and with pageable_too any host memory
+bool pipeline_source(const void* buf, bool pageable_too)
 {
   cudaPointerAttributes at;
   const cudaError_t e = cudaPointerGetAttributes(&at, buf);
   if (e != cudaSuccess)
   {
     cudaGetLastError();
-    return true;
+    return pageable_too;
   }
-  return at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged;
+  return at.type == cudaMemoryTypeHost ||
+         (pageable_too && at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged);
 }
 
-// page-locked host memory (cudaHostAlloc / cudaHostRegister): DMA reads it directly
-bool is_pinned_host_pointer(const void* buf)
+// ---- the call frame of the scan entry points ----
+// An entry point checks its arguments (check_scan) and zeroes its outputs.  begin_scan answers an empty buffer with
+// *totals = tt and no device work (*dbuf stays nullptr); otherwise it sets the device, makes the buffer visible to the
+// device (resolve; with stage_only just the staging buffer, which the pipelined stream route fills itself), enqueues
+// `setup` (what is not kernel time: uploads, flags to zero, scratch) and records ev0 before the first launch.
+// end_scan records ev1 after the last launch and the copies of the results, waits for the stream, and fills
+// kernel_ms, the results `read` from h_totals and *totals.
+
+// the checks of a scan over one pattern, in the order the entry points report them; `who` names the entry point
+int check_scan(const char* who, const ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, uint32_t flags = 0)
 {
-  cudaPointerAttributes at;
-  const cudaError_t e = cudaPointerGetAttributes(&at, buf);
-  if (e != cudaSuccess)
+  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
+    return fail(UGX_E_INVALID, "null argument");
+  if ((flags & ~UGX_LINES_INVERT) != 0)
+    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
+  if (s->device != p->device)
+    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+  return UGX_OK;
+}
+
+int no_setup() { return UGX_OK; }
+
+template <typename Setup = int (&)()>
+int begin_scan(ugx_scanner* s, const void* buf, uint64_t n, const ugx_totals& tt, ugx_totals* totals, const uint8_t** dbuf,
+               Setup&& setup = no_setup, bool stage_only = false)
+{
+  *dbuf = nullptr;
+  if (n == 0)
   {
-    cudaGetLastError();
-    return false;
+    if (totals)
+      *totals = tt;
+    return UGX_OK;
   }
-  return at.type == cudaMemoryTypeHost;
+  CU(cudaSetDevice(s->device));
+  TRY(stage_only ? s->stage.ensure(n + 16) : resolve(s, buf, n, dbuf));
+  if (stage_only)
+    *dbuf = s->stage.p;
+  TRY(setup());
+  CU(cudaEventRecord(s->ev0, s->stream));
+  return UGX_OK;
+}
+
+enum : unsigned { READ_MATCHES = 1, READ_NEWLINES = 2 }; // results end_scan takes from h_totals
+
+// ev1_recorded: the caller stopped the clock itself, before copies that are not kernel time
+int end_scan(ugx_scanner* s, ugx_totals& tt, ugx_totals* totals, unsigned read = 0, bool ev1_recorded = false)
+{
+  if (!ev1_recorded)
+    CU(cudaEventRecord(s->ev1, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  CU(cudaEventElapsedTime(&tt.kernel_ms, s->ev0, s->ev1));
+  if (read & READ_MATCHES)
+    tt.matches = s->h_totals[ugx::SLOT_MATCHES];
+  if (read & READ_NEWLINES)
+    tt.newlines = s->h_totals[ugx::SLOT_NEWLINES];
+  if (totals)
+    *totals = tt;
+  return UGX_OK;
+}
+
+// the host's read of totals slots [0, k) after a count pass
+int read_totals(ugx_scanner* s, int k)
+{
+  CU(cudaMemcpyAsync(s->h_totals, s->totals, k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  return UGX_OK;
+}
+
+// ... and the arena grown for the *nrec = h_totals[SLOT_MATCHES] records of the emit pass
+template <typename T>
+int read_count(ugx_scanner* s, int k, DevBuf<T>& arena, uint64_t* nrec)
+{
+  TRY(read_totals(s, k));
+  *nrec = s->h_totals[ugx::SLOT_MATCHES];
+  return arena.ensure(*nrec);
+}
+
+// the records of the last call from the device to the caller's out[cap]; *n_out is set before an overflow is reported.
+// With keep_on_device (the batch calls), out == NULL with cap == 0 leaves the records on the device.
+int copy_out(ugx_scanner* s, const void* dev, size_t rec_bytes, uint64_t n, void* out, uint64_t cap, uint64_t* n_out,
+             bool keep_on_device, const char* overflow)
+{
+  if (n_out)
+    *n_out = n;
+  if (keep_on_device && out == nullptr && cap == 0)
+    return UGX_OK;
+  if (n > cap)
+    return fail(UGX_E_OVERFLOW, overflow);
+  if (n > 0)
+  {
+    if (out == nullptr)
+      return fail(UGX_E_INVALID, "null record buffer");
+    CU(cudaMemcpyAsync(out, dev, n * rec_bytes, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+  }
+  return UGX_OK;
+}
+
+// ugx_scanner_fetch / ugx_scanner_fetch_lines: records [first, first + count) of the n in `arena`
+template <typename R>
+int fetch(ugx_scanner* s, const DevBuf<R>& arena, uint64_t n, R* out, uint64_t first, uint64_t count, const char* range)
+{
+  if (first > n || count > n - first)
+    return fail(UGX_E_INVALID, range);
+  if (count == 0)
+    return UGX_OK;
+  CU(cudaSetDevice(s->device));
+  CU(cudaMemcpyAsync(out, arena.p + first, count * sizeof(R), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaStreamSynchronize(s->stream));
+  return UGX_OK;
+}
+
+// the record outputs of an entry point: zeroed on entry, the arena and its count once a result stands
+template <typename R>
+void set_records(const R** dev_out, uint64_t* n_out, const R* dev, uint64_t n)
+{
+  if (n_out)
+    *n_out = n;
+  if (dev_out)
+    *dev_out = dev;
+}
+
+// the per-tile sums of the line-at-a-time and batch kernels
+int ensure_tiles(ugx_scanner* s, uint64_t ntiles)
+{
+  TRY(s->tile_matches.ensure(ntiles));
+  return s->tile_newlines.ensure(ntiles);
+}
+
+// reflex::nlcount into the newlines slot, read back by end_scan (READ_NEWLINES): ugx_count_newlines, and every scan
+// with a pattern whose prefilter admits no candidate
+int newline_pass(ugx_scanner* s, const uint8_t* dbuf, uint64_t n, ugx_totals& tt)
+{
+  CU(ugx::launch_count_newlines(dbuf, n, s->totals + ugx::SLOT_NEWLINES, s->sm_count, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals + ugx::SLOT_NEWLINES, s->totals + ugx::SLOT_NEWLINES, sizeof(unsigned long long),
+                     cudaMemcpyDeviceToHost, s->stream));
+  tt.flags |= UGX_TOT_NEWLINES;
+  tt.launches = 1;
+  tt.kernel = UGX_K_NEWLINES;
+  return UGX_OK;
 }
 
 // the count pass of the span kernels (last line, span_scan_kernel, span_final_kernel) up to the host's read of
@@ -842,361 +911,374 @@ int span_count_pass(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, u
                     uint64_t base_line, ugx::SpanArgs& a, ugx_totals* tt)
 {
   const uint64_t nreg = ugx::stream_regions(n);
-  int rc = ensure(s->span_regions, s->span_regions_cap, 5 * nreg + 8);
-  if (rc == UGX_OK && want_sel)
-    rc = ensure(s->span_sel, s->span_sel_cap, (n + 15) / 16 + 64);
-  if (rc != UGX_OK)
-    return rc;
+  TRY(s->span_regions.ensure(5 * nreg + 8));
+  if (want_sel)
+    TRY(s->span_sel.ensure((n + 15) / 16 + 64));
   memset(&a, 0, sizeof(a));
-  a.reg_matches = s->span_regions;
-  a.reg_newlines = s->span_regions + nreg;
-  a.reg_emain = s->span_regions + 2 * nreg;
-  a.reg_elast = s->span_regions + 3 * nreg;
-  a.reg_v = s->span_regions + 4 * nreg;
-  a.sel_bits = want_sel ? s->span_sel : nullptr;
+  a.reg_matches = s->span_regions.p;
+  a.reg_newlines = s->span_regions.p + nreg;
+  a.reg_emain = s->span_regions.p + 2 * nreg;
+  a.reg_elast = s->span_regions.p + 3 * nreg;
+  a.reg_v = s->span_regions.p + 4 * nreg;
+  a.sel_bits = want_sel ? s->span_sel.p : nullptr;
   a.base_offset = base_offset;
   a.base_line = base_line;
   a.no_cover = s->no_cover ? 1u : 0u;
-  a.tail = reinterpret_cast<const uint64_t*>(s->totals + 5);
-  a.flags = reinterpret_cast<unsigned int*>(s->totals + 6);
-  CU(cudaMemsetAsync(s->totals + 6, 0, sizeof(unsigned long long), s->stream));
-  CU(ugx::launch_last_line(dbuf, n, reinterpret_cast<uint64_t*>(s->totals + 5), s->stream));
+  a.tail = reinterpret_cast<const uint64_t*>(s->totals + ugx::SLOT_LAST_LINE);
+  a.flags = reinterpret_cast<unsigned int*>(s->totals + ugx::SLOT_SPAN_FLAGS);
+  CU(cudaMemsetAsync(s->totals + ugx::SLOT_SPAN_FLAGS, 0, sizeof(unsigned long long), s->stream));
+  CU(ugx::launch_last_line(dbuf, n, reinterpret_cast<uint64_t*>(s->totals + ugx::SLOT_LAST_LINE), s->stream));
   CU(ugx::launch_span_scan(p->dev, dbuf, n, a, false, s->sm_count, s->stream));
   CU(ugx::launch_span_final(p->dev, dbuf, n, a, false, s->totals, s->stream));
-  CU(cudaMemcpyAsync(s->h_totals, s->totals, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
+  TRY(read_totals(s, 3));
   tt->launches += 3;
   return UGX_OK;
 }
 
-// `ugrep -c -o` / `ugrep -o -n -b` through the span kernels (span_scan.cu).  *valid = false: the spans could not vouch
-// for their result on this buffer (a match longer than a window across a region start in a line without newlines, an
-// attempt that failed at the very end of the buffer, a match of 64 KiB or more) — the caller then takes the
-// line-at-a-time kernels.
-int scan_spans(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, bool want_records, uint64_t base_offset,
-               uint64_t base_line, ugx_totals* tt, bool* valid)
+// ScanArgs of the line-at-a-time kernels over dbuf[0, n), with the scanner's tile sums and, for the count pass of
+// records, its strip counts
+int line_scan_args(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64_t n, bool strips, uint64_t base_offset,
+                   uint64_t base_line, ugx::ScanArgs& a)
 {
+  const uint64_t tile_bytes = ugx::scan_tile_bytes(p->dev);
+  const uint64_t ntiles = (n + tile_bytes - 1) / tile_bytes;
+  TRY(ensure_tiles(s, ntiles));
+  if (strips)
+    TRY(s->strip_counts.ensure((n + ugx::SCAN_STRIP - 1) / ugx::SCAN_STRIP));
+  a.buf = dbuf;
+  a.n = n;
+  a.ntiles = ntiles;
+  a.tile_matches = s->tile_matches.p;
+  a.tile_newlines = s->tile_newlines.p;
+  a.strip_counts = strips ? s->strip_counts.p : nullptr;
+  a.out = nullptr;
+  a.out_cap = 0;
+  a.base_offset = base_offset;
+  a.base_line = base_line;
+  return UGX_OK;
+}
+
+// ---- ugx_count_lines / ugx_count_matches / ugx_find_all*: scan_route picks a route, and each route reports its own
+// results: the totals, the results its last copy leaves in h_totals for end_scan (`read`), and the match records ----
+enum class Route {
+  NEVER,       // the prefilter admits no candidate: the result is empty, the pass over the text only counts newlines
+  SPAN,        // the span kernels; they may hand over to RECORDS or LINE_SCAN
+  STREAM,      // streaming `-c`: literal, DFA or search automaton
+  TILE_ANY,    // the tile-synchronous count_lines_any_kernel
+  MATCH_LINES, // counting with position-parallel attempts
+  RECORDS,     // single-pass match records: staging pass, prefix, reorder
+  TWO_PASS,    // match records by a count pass and an emit pass of the line scan
+  LINE_SCAN,   // counting with scan_lines_kernel
+};
+
+// the span kernels take line records, and match counts and records where scan_route allows, unless an option sends
+// the scan to the line-at-a-time kernels
+bool span_route(const ugx_scanner* s, const ugx_pattern* p)
+{
+  return !p->never && !s->force_generic && !s->no_span && ugx::span_scan_eligible(p->dev);
+}
+
+Route scan_route(const ugx_scanner* s, const ugx_pattern* p, int mode, bool want_records)
+{
+  const ugx::DevPattern& d = p->dev;
+  if (p->never)
+    return Route::NEVER;
+  if (mode == 1 && !s->match_lines && !s->two_pass_records && span_route(s, p))
+    return Route::SPAN;
+  if (mode == 0 && !want_records && !s->force_generic)
+  {
+    if (!s->legacy_any && ugx::count_lines_stream_eligible(d) &&
+        (s->stream_dfa || ugx::count_lines_literal_eligible(d) || d.plan.h4_terms >= 1 || d.plan.pm2 != 0 ||
+         (d.plan.kind == ugx::FK_LUT && d.plan.nterms >= 1 && d.one == 0)))
+      return Route::STREAM;
+    if (ugx::count_lines_any_eligible(d))
+      return Route::TILE_ANY;
+  }
+  if (!want_records && !s->force_generic && s->match_lines && ugx::match_lines_eligible(d))
+    return Route::MATCH_LINES;
+  if (want_records)
+    return s->two_pass_records ? Route::TWO_PASS : Route::RECORDS;
+  return Route::LINE_SCAN;
+}
+
+// one call: its arguments, the device view of its buffer, ScanArgs of the line-at-a-time routes, and the results
+struct Scan {
+  ugx_scanner* s;
+  const ugx_pattern* p;
+  const void* buf;
+  uint64_t n;
+  int mode;
+  bool want_records;
+  uint64_t base_offset, base_line;
+  const ugx_match** dev_out;
+  uint64_t* n_out;
+  const uint8_t* dbuf;
+  ugx::ScanArgs a;
+  ugx_totals tt;
+  unsigned read;
+};
+
+// the end of a counting route: the two result slots to the host for end_scan
+int copy_results(Scan& c, bool newlines)
+{
+  CU(cudaMemcpyAsync(c.s->h_totals, c.s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c.s->stream));
+  c.read = READ_MATCHES | READ_NEWLINES;
+  if (newlines)
+    c.tt.flags |= UGX_TOT_NEWLINES;
+  return UGX_OK;
+}
+
+// the end of a records route: the match arena holds nrec records, published to the caller
+void publish_records(Scan& c, uint64_t nrec)
+{
+  c.s->records_n = nrec;
+  set_records(c.dev_out, c.n_out, c.s->records.p, nrec);
+}
+
+// Route::SPAN (span_scan.cu).  *valid = false: the spans could not vouch for their result on this buffer (a match
+// longer than a window across a region start in a line without newlines, an attempt that failed at the very end of
+// the buffer, a match of 64 KiB or more) — the caller then takes the line-at-a-time kernels.
+int scan_spans(Scan& c, bool* valid)
+{
+  ugx_scanner* s = c.s;
   *valid = false;
   ugx::SpanArgs a;
-  int rc = span_count_pass(s, p, dbuf, n, want_records, base_offset, base_line, a, tt);
-  if (rc != UGX_OK)
-    return rc;
-  if (s->h_totals[2] != 0)
+  TRY(span_count_pass(s, c.p, c.dbuf, c.n, c.want_records, c.base_offset, c.base_line, a, &c.tt));
+  if (s->h_totals[ugx::SLOT_HANDOVER] != 0)
     return UGX_OK; // not valid: nothing of this attempt is used
-  const uint64_t nrec = s->h_totals[0];
-  if (want_records)
+  const uint64_t nrec = s->h_totals[ugx::SLOT_MATCHES];
+  if (c.want_records)
   {
-    rc = ensure(s->records, s->records_cap, nrec);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(s->records.ensure(nrec));
     if (nrec > 0)
     {
-      a.out = s->records;
+      a.out = s->records.p;
       a.out_cap = nrec;
-      CU(ugx::launch_span_scan(p->dev, dbuf, n, a, true, s->sm_count, s->stream));
-      CU(ugx::launch_span_final(p->dev, dbuf, n, a, true, s->totals, s->stream));
-      tt->launches += 2;
+      CU(ugx::launch_span_scan(c.p->dev, c.dbuf, c.n, a, true, s->sm_count, s->stream));
+      CU(ugx::launch_span_final(c.p->dev, c.dbuf, c.n, a, true, s->totals, s->stream));
+      c.tt.launches += 2;
     }
-    s->records_n = nrec;
+    publish_records(c, nrec);
   }
-  tt->matches = nrec;
-  tt->newlines = s->h_totals[1];
-  tt->flags |= UGX_TOT_NEWLINES;
-  tt->kernel = UGX_K_SPAN;
+  c.tt.matches = nrec;
+  c.tt.newlines = s->h_totals[ugx::SLOT_NEWLINES];
+  c.tt.flags |= UGX_TOT_NEWLINES;
+  c.tt.kernel = UGX_K_SPAN;
   *valid = true;
   return UGX_OK;
+}
+
+// Route::STREAM; a pipelined host buffer is copied into s->stage here
+int stream_count(Scan& c, bool pipelined)
+{
+  ugx_scanner* s = c.s;
+  const ugx_pattern* p = c.p;
+  const uint8_t* dbuf = c.dbuf;
+  const uint64_t n = c.n;
+  TRY(s->region_sum.ensure(ugx::stream_regions(n) + 64));
+  ugx::StreamArgs sa;
+  sa.region_sum = s->region_sum.p;
+  sa.partials = s->partials;
+  sa.ticket = s->ticket;
+  sa.done = reinterpret_cast<unsigned int*>(s->ticket + 1);
+  sa.totals = s->totals;
+  sa.stage_table = 0;
+  sa.use_h4 = 0;
+  sa.use_via = 0;
+  sa.no_cover = s->no_cover ? 1u : 0u;
+  const uint64_t nreg = ugx::stream_regions(n);
+  const bool search = p->dev.search_ok != 0 && !s->no_search;
+  if (pipelined)
+  {
+    // host buffer: copy in chunks on the copy stream and scan chunk i while chunk i + 1 is in flight.  A launch
+    // trails the copied bytes by one region, so that every read of a scanned position (literal verify, a DFA
+    // attempt of bounded length) finds its bytes; the region summaries chain the launches.
+    uint64_t copied = 0, scanned = 0;
+    c.tt.launches = 0;
+    while (scanned < nreg)
+    {
+      const uint64_t take = n - copied < PIPE_CHUNK ? n - copied : PIPE_CHUNK;
+      if (take > 0)
+      {
+        CU(cudaMemcpyAsync(s->stage.p + copied, static_cast<const uint8_t*>(c.buf) + copied, take, cudaMemcpyHostToDevice,
+                           s->copy_stream));
+        copied += take;
+        CU(cudaEventRecord(s->ev_copy, s->copy_stream));
+        CU(cudaStreamWaitEvent(s->stream, s->ev_copy, 0));
+      }
+      const uint64_t upto = copied == n ? nreg : copied / ugx::SC_REGION - 1;
+      if (upto <= scanned)
+        continue;
+      sa.region_begin = scanned;
+      sa.region_end = upto;
+      sa.finalize = upto == nreg ? 1u : 0u;
+      sa.accumulate = scanned == 0 ? 0u : 1u;
+      CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream)
+                : ugx::launch_count_lines_stream(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream));
+      scanned = upto;
+      ++c.tt.launches;
+    }
+  }
+  else
+  {
+    sa.region_begin = 0;
+    sa.region_end = nreg;
+    sa.finalize = 1;
+    sa.accumulate = 0;
+    CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream)
+              : ugx::launch_count_lines_stream(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream));
+    c.tt.launches = 1;
+  }
+  c.tt.kernel = ugx::count_lines_literal_eligible(p->dev) ? UGX_K_STREAM_LITERAL
+                : search                                   ? UGX_K_STREAM_SEARCH
+                                                           : UGX_K_STREAM_DFA;
+  return copy_results(c, s->count_newlines);
+}
+
+// Route::MATCH_LINES (match_lines.cu); its tiles are smaller than the line scan's
+int match_lines_count(Scan& c)
+{
+  ugx_scanner* s = c.s;
+  const uint64_t tb = ugx::match_lines_tile_bytes(c.p->dev);
+  const uint64_t nt = (c.n + tb - 1) / tb;
+  TRY(ensure_tiles(s, nt));
+  c.a.ntiles = nt;
+  c.a.tile_matches = s->tile_matches.p;
+  c.a.tile_newlines = s->tile_newlines.p;
+  CU(ugx::launch_match_lines(c.p->dev, c.a, c.mode, s->sm_count, s->stream));
+  CU(ugx::launch_tile_prefix(s->tile_matches.p, s->tile_newlines.p, nt, s->totals, s->stream));
+  c.tt.launches = 2;
+  c.tt.kernel = UGX_K_MATCH_LINES;
+  return copy_results(c, true);
+}
+
+// Route::RECORDS: staging pass (tiles in completion order) + prefix + reorder into input order.  The staging capacity
+// is a guess (the last result, or one record per 96 bytes); the cursor tells the exact need, so a second staging pass
+// always fits.
+int staged_records(Scan& c)
+{
+  ugx_scanner* s = c.s;
+  const ugx::ScanArgs& a = c.a;
+  TRY(s->tile_base.ensure(a.ntiles));
+  TRY(s->rec_stage.ensure(s->records_n + s->records_n / 4 + a.n / 96 + 1024));
+  unsigned long long* cursor = s->totals + ugx::SLOT_HANDOVER;
+  uint64_t nrec = 0;
+  for (int attempt = 0; attempt < 2; ++attempt)
+  {
+    CU(ugx::launch_scan_records(c.p->dev, a, s->tile_base.p, s->rec_stage.p, s->rec_stage.cap, cursor, s->sm_count, s->stream));
+    CU(ugx::launch_tile_prefix(a.tile_matches, a.tile_newlines, a.ntiles, s->totals, s->stream));
+    TRY(read_totals(s, 2));
+    c.tt.launches += 2;
+    nrec = s->h_totals[ugx::SLOT_MATCHES];
+    if (nrec <= s->rec_stage.cap)
+      break;
+    if (attempt == 1)
+      return fail(UGX_E_CUDA, "record staging overflowed twice");
+    TRY(s->rec_stage.ensure(nrec));
+  }
+  TRY(s->records.ensure(nrec));
+  if (nrec > 0)
+  {
+    CU(ugx::launch_reorder_records(s->rec_stage.p, s->records.p, a.tile_matches, a.tile_newlines, s->tile_base.p, a.ntiles,
+                                   s->totals, a.base_line, s->sm_count, s->stream));
+    c.tt.launches += 1;
+  }
+  c.tt.kernel = UGX_K_RECORDS;
+  c.tt.flags |= UGX_TOT_NEWLINES;
+  c.read = READ_MATCHES | READ_NEWLINES; // left in h_totals by the last staging pass
+  publish_records(c, nrec);
+  return UGX_OK;
+}
+
+// Route::TWO_PASS: the line scan's count pass into the strip counts, the tile prefix, and its emit pass
+int two_pass_records(Scan& c)
+{
+  ugx_scanner* s = c.s;
+  CU(ugx::launch_scan_lines(c.p->dev, c.a, c.mode, false, s->sm_count, s->stream));
+  CU(ugx::launch_tile_prefix(c.a.tile_matches, c.a.tile_newlines, c.a.ntiles, s->totals, s->stream));
+  c.tt.launches = 2;
+  c.tt.kernel = UGX_K_LINE_SCAN;
+  uint64_t nrec = 0;
+  TRY(read_count(s, 2, s->records, &nrec));
+  if (nrec > 0)
+  {
+    c.a.out = s->records.p;
+    c.a.out_cap = nrec;
+    CU(ugx::launch_scan_lines(c.p->dev, c.a, c.mode, true, s->sm_count, s->stream));
+    c.tt.launches += 1;
+  }
+  c.tt.flags |= UGX_TOT_NEWLINES;
+  c.read = READ_MATCHES | READ_NEWLINES; // left in h_totals by the count pass
+  publish_records(c, nrec);
+  return UGX_OK;
+}
+
+// every route but SPAN, once ScanArgs and ev0 are in place
+int run_route(Scan& c, Route r, bool pipelined)
+{
+  ugx_scanner* s = c.s;
+  switch (r)
+  {
+    case Route::NEVER:
+      TRY(newline_pass(s, c.dbuf, c.n, c.tt));
+      c.read = READ_NEWLINES;
+      s->records_n = 0;
+      return UGX_OK;
+    case Route::SPAN: return UGX_OK; // scan_spans has run
+    case Route::STREAM: return stream_count(c, pipelined);
+    case Route::TILE_ANY:
+      CU(ugx::launch_count_lines_any(c.p->dev, c.dbuf, c.n, s->totals, s->sm_count, s->stream));
+      c.tt.launches = 1;
+      c.tt.kernel = UGX_K_TILE_ANY;
+      return copy_results(c, true);
+    case Route::MATCH_LINES: return match_lines_count(c);
+    case Route::RECORDS: return staged_records(c);
+    case Route::TWO_PASS: return two_pass_records(c);
+    case Route::LINE_SCAN: break;
+  }
+  CU(ugx::launch_scan_lines(c.p->dev, c.a, c.mode, false, s->sm_count, s->stream));
+  CU(ugx::launch_tile_prefix(c.a.tile_matches, c.a.tile_newlines, c.a.ntiles, s->totals, s->stream));
+  c.tt.launches = 2;
+  c.tt.kernel = UGX_K_LINE_SCAN;
+  return copy_results(c, true);
 }
 
 int scan_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t n, int mode, bool want_records,
                 uint64_t base_offset, uint64_t base_line, const ugx_match** dev_out, uint64_t* n_out, ugx_totals* totals)
 {
-  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
-    return fail(UGX_E_INVALID, "null argument");
-  if (s->device != p->device)
-    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
-  if (n_out)
-    *n_out = 0;
-  if (dev_out)
-    *dev_out = nullptr;
-  if (n == 0)
-  {
-    if (totals)
-      *totals = tt;
-    return UGX_OK;
-  }
-  CU(cudaSetDevice(s->device));
-  const uint8_t* dbuf = nullptr;
-  uint64_t h2d = 0;
-  const bool stream_route = mode == 0 && !want_records && !s->force_generic && !s->legacy_any &&
-                            ugx::count_lines_stream_eligible(p->dev) &&
-                            (s->stream_dfa || ugx::count_lines_literal_eligible(p->dev) || p->dev.plan.h4_terms >= 1 || p->dev.plan.pm2 != 0 ||
-                             (p->dev.plan.kind == ugx::FK_LUT && p->dev.plan.nterms >= 1 && p->dev.one == 0));
+  TRY(check_scan("scan", s, p, buf, n));
+  Scan c{s, p, buf, n, mode, want_records, base_offset, base_line, dev_out, n_out};
+  set_records<ugx_match>(dev_out, n_out, nullptr, 0);
+  Route r = scan_route(s, p, mode, want_records);
   // a host buffer on the streaming route is copied chunk by chunk, overlapped with the scan, when every read of a
   // scanned position stays within one region of it: pure literals, and DFAs whose longest match is bounded
   const bool bounded = ugx::count_lines_literal_eligible(p->dev) || p->dfa.max_match_len < ugx::SC_REGION - 512;
   // (chunk-wise overlap of copy and scan for page-locked buffers; pageable ones go through the feeder threads of resolve())
-  const bool pipelined = stream_route && bounded && !p->never && !s->no_pipeline && n >= 2 * PIPE_CHUNK && is_host_pointer(buf) &&
-                         (is_pinned_host_pointer(buf) || s->no_feeder);
-  int rc;
-  if (pipelined)
-  {
-    rc = ensure(s->stage, s->stage_cap, n + 16);
-    dbuf = s->stage;
-    h2d = n;
-  }
-  else
-    rc = resolve(s, buf, n, &dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
-  if (p->never)
-  {
-    // no position can be a candidate: the result is empty; the pass over the text only counts newlines
-    CU(cudaEventRecord(s->ev0, s->stream));
-    CU(ugx::launch_count_newlines(dbuf, n, s->totals + 1, s->sm_count, s->stream));
-    CU(cudaMemcpyAsync(s->h_totals + 1, s->totals + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaEventRecord(s->ev1, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    float ms0 = 0;
-    CU(cudaEventElapsedTime(&ms0, s->ev0, s->ev1));
-    tt.newlines = s->h_totals[1];
-    tt.flags |= UGX_TOT_NEWLINES;
-    tt.kernel_ms = ms0;
-    tt.launches = 1;
-    tt.kernel = UGX_K_NEWLINES;
-    s->records_n = 0;
-    if (totals)
-      *totals = tt;
+  const bool pipelined = r == Route::STREAM && bounded && !s->no_pipeline && n >= 2 * PIPE_CHUNK &&
+                         pipeline_source(buf, s->no_feeder);
+  // the line-at-a-time routes size their tile sums before the clock starts
+  const bool tiles = r != Route::NEVER && r != Route::SPAN;
+  TRY(begin_scan(s, buf, n, c.tt, totals, &c.dbuf, [&]() -> int {
+    return tiles ? line_scan_args(s, p, c.dbuf, n, r == Route::TWO_PASS, base_offset, base_line, c.a) : UGX_OK;
+  }, pipelined));
+  if (c.dbuf == nullptr)
     return UGX_OK;
-  }
-  if (mode == 1 && !s->force_generic && !s->no_span && !s->match_lines && !s->two_pass_records &&
-      ugx::span_scan_eligible(p->dev))
+  if (r == Route::SPAN)
   {
     bool valid = false;
-    CU(cudaEventRecord(s->ev0, s->stream));
-    rc = scan_spans(s, p, dbuf, n, want_records, base_offset, base_line, &tt, &valid);
-    if (rc != UGX_OK)
-      return rc;
-    if (valid)
+    TRY(scan_spans(c, &valid));
+    if (!valid)
     {
-      CU(cudaEventRecord(s->ev1, s->stream));
-      CU(cudaStreamSynchronize(s->stream));
-      float sms = 0;
-      CU(cudaEventElapsedTime(&sms, s->ev0, s->ev1));
-      tt.kernel_ms = sms;
-      if (want_records)
-      {
-        if (n_out)
-          *n_out = s->records_n;
-        if (dev_out)
-          *dev_out = s->records;
-      }
-      if (totals)
-        *totals = tt;
-      return UGX_OK;
+      // the line-at-a-time kernels take over (the span route excludes match_lines and two_pass_records)
+      r = want_records ? Route::RECORDS : Route::LINE_SCAN;
+      c.tt.launches = 0;
+      c.tt.flags |= UGX_TOT_SPAN_HANDOVER;
+      TRY(line_scan_args(s, p, c.dbuf, n, false, base_offset, base_line, c.a));
+      CU(cudaEventRecord(s->ev0, s->stream));
     }
-    tt.launches = 0; // the line-at-a-time kernels take over
-    tt.flags |= UGX_TOT_SPAN_HANDOVER;
   }
-  const uint64_t tile_bytes = ugx::scan_tile_bytes(p->dev);
-  const uint64_t ntiles = (n + tile_bytes - 1) / tile_bytes;
-  const uint64_t nstrips = (n + ugx::SCAN_STRIP - 1) / ugx::SCAN_STRIP;
-  uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
-  rc = ensure(s->tile_matches, cap1, ntiles);
-  if (rc == UGX_OK)
-    rc = ensure(s->tile_newlines, cap2, ntiles);
-  s->tiles_cap = cap1 < cap2 ? cap1 : cap2;
-  if (rc == UGX_OK && want_records && s->two_pass_records)
-    rc = ensure(s->strip_counts, s->strips_cap, nstrips);
-  if (rc != UGX_OK)
-    return rc;
-  ugx::ScanArgs a;
-  a.buf = dbuf;
-  a.n = n;
-  a.ntiles = ntiles;
-  a.tile_matches = s->tile_matches;
-  a.tile_newlines = s->tile_newlines;
-  a.strip_counts = want_records && s->two_pass_records ? s->strip_counts : nullptr;
-  a.out = nullptr;
-  a.out_cap = 0;
-  a.base_offset = base_offset;
-  a.base_line = base_line;
-  CU(cudaEventRecord(s->ev0, s->stream));
-  if (stream_route)
-  {
-    rc = ensure(s->region_sum, s->region_cap, ugx::stream_regions(n) + 64);
-    if (rc != UGX_OK)
-      return rc;
-    ugx::StreamArgs sa;
-    sa.region_sum = s->region_sum;
-    sa.partials = s->partials;
-    sa.ticket = s->ticket;
-    sa.done = reinterpret_cast<unsigned int*>(s->ticket + 1);
-    sa.totals = s->totals;
-    sa.stage_table = 0;
-    sa.use_h4 = 0;
-    sa.use_via = 0;
-    sa.no_cover = s->no_cover ? 1u : 0u;
-    const uint64_t nreg = ugx::stream_regions(n);
-    const bool search = p->dev.search_ok != 0 && !s->no_search;
-    if (pipelined)
-    {
-      // host buffer: copy in chunks on the copy stream and scan chunk i while chunk i + 1 is in flight.  A launch
-      // trails the copied bytes by one region, so that every read of a scanned position (literal verify, a DFA
-      // attempt of bounded length) finds its bytes; the region summaries chain the launches.
-      uint64_t copied = 0, scanned = 0;
-      tt.launches = 0;
-      while (scanned < nreg)
-      {
-        const uint64_t take = n - copied < PIPE_CHUNK ? n - copied : PIPE_CHUNK;
-        if (take > 0)
-        {
-          CU(cudaMemcpyAsync(s->stage + copied, static_cast<const uint8_t*>(buf) + copied, take, cudaMemcpyHostToDevice,
-                             s->copy_stream));
-          copied += take;
-          CU(cudaEventRecord(s->ev_copy, s->copy_stream));
-          CU(cudaStreamWaitEvent(s->stream, s->ev_copy, 0));
-        }
-        const uint64_t upto = copied == n ? nreg : copied / ugx::SC_REGION - 1;
-        if (upto <= scanned)
-          continue;
-        sa.region_begin = scanned;
-        sa.region_end = upto;
-        sa.finalize = upto == nreg ? 1u : 0u;
-        sa.accumulate = scanned == 0 ? 0u : 1u;
-        CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream)
-                  : ugx::launch_count_lines_stream(p->dev, dbuf, copied, sa, s->count_newlines, s->sm_count, s->stream));
-        scanned = upto;
-        ++tt.launches;
-      }
-    }
-    else
-    {
-      sa.region_begin = 0;
-      sa.region_end = nreg;
-      sa.finalize = 1;
-      sa.accumulate = 0;
-      CU(search ? ugx::launch_count_lines_search(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream)
-                : ugx::launch_count_lines_stream(p->dev, dbuf, n, sa, s->count_newlines, s->sm_count, s->stream));
-      tt.launches = 1;
-    }
-    tt.kernel = ugx::count_lines_literal_eligible(p->dev) ? UGX_K_STREAM_LITERAL
-                : search                                   ? UGX_K_STREAM_SEARCH
-                                                           : UGX_K_STREAM_DFA;
-  }
-  else if (mode == 0 && !want_records && !s->force_generic && ugx::count_lines_any_eligible(p->dev))
-  {
-    CU(ugx::launch_count_lines_any(p->dev, dbuf, n, s->totals, s->sm_count, s->stream));
-    tt.launches = 1;
-    tt.kernel = UGX_K_TILE_ANY;
-  }
-  else if (!want_records && !s->force_generic && s->match_lines && ugx::match_lines_eligible(p->dev))
-  {
-    // counting with position-parallel attempts (match_lines.cu); its tiles are smaller than the line scan's
-    const uint64_t tb = ugx::match_lines_tile_bytes(p->dev);
-    const uint64_t nt = (n + tb - 1) / tb;
-    uint64_t c1 = s->tiles_cap, c2 = s->tiles_cap;
-    rc = ensure(s->tile_matches, c1, nt);
-    if (rc == UGX_OK)
-      rc = ensure(s->tile_newlines, c2, nt);
-    s->tiles_cap = c1 < c2 ? c1 : c2;
-    if (rc != UGX_OK)
-      return rc;
-    a.ntiles = nt;
-    a.tile_matches = s->tile_matches;
-    a.tile_newlines = s->tile_newlines;
-    CU(ugx::launch_match_lines(p->dev, a, mode, s->sm_count, s->stream));
-    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, nt, s->totals, s->stream));
-    tt.launches = 2;
-    tt.kernel = UGX_K_MATCH_LINES;
-  }
-  else if (want_records && !s->two_pass_records)
-  {
-    // single-pass records: staging pass (tiles in completion order) + prefix + reorder into input order.  The staging
-    // capacity is a guess (the last result, or one record per 96 bytes); the cursor tells the exact need, so a
-    // second staging pass always fits.
-    rc = ensure(s->tile_base, s->tile_base_cap, ntiles);
-    uint64_t guess = s->records_n + s->records_n / 4 + n / 96 + 1024;
-    if (rc == UGX_OK && s->rec_stage_cap < guess)
-      rc = ensure(s->rec_stage, s->rec_stage_cap, guess);
-    if (rc != UGX_OK)
-      return rc;
-    unsigned long long* cursor = s->totals + 2;
-    uint64_t nrec = 0;
-    for (int attempt = 0; attempt < 2; ++attempt)
-    {
-      CU(ugx::launch_scan_records(p->dev, a, s->tile_base, s->rec_stage, s->rec_stage_cap, cursor, s->sm_count, s->stream));
-      CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
-      CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-      CU(cudaStreamSynchronize(s->stream));
-      tt.launches += 2;
-      nrec = s->h_totals[0];
-      if (nrec <= s->rec_stage_cap)
-        break;
-      if (attempt == 1)
-        return fail(UGX_E_CUDA, "record staging overflowed twice");
-      rc = ensure(s->rec_stage, s->rec_stage_cap, nrec);
-      if (rc != UGX_OK)
-        return rc;
-    }
-    rc = ensure(s->records, s->records_cap, nrec);
-    if (rc != UGX_OK)
-      return rc;
-    if (nrec > 0)
-    {
-      CU(ugx::launch_reorder_records(s->rec_stage, s->records, s->tile_matches, s->tile_newlines, s->tile_base, ntiles,
-                                     s->totals, base_line, s->sm_count, s->stream));
-      tt.launches += 1;
-    }
-    tt.kernel = UGX_K_RECORDS;
-    s->records_n = nrec;
-    if (n_out)
-      *n_out = nrec;
-    if (dev_out)
-      *dev_out = s->records;
-  }
-  else
-  {
-    CU(ugx::launch_scan_lines(p->dev, a, mode, false, s->sm_count, s->stream));
-    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
-    tt.launches = 2;
-    tt.kernel = UGX_K_LINE_SCAN;
-  }
-  if (!(want_records && !s->two_pass_records))
-    CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  if (want_records && s->two_pass_records)
-  {
-    CU(cudaStreamSynchronize(s->stream));
-    const uint64_t nrec = s->h_totals[0];
-    rc = ensure(s->records, s->records_cap, nrec);
-    if (rc != UGX_OK)
-      return rc;
-    if (nrec > 0)
-    {
-      a.out = s->records;
-      a.out_cap = nrec;
-      CU(ugx::launch_scan_lines(p->dev, a, mode, true, s->sm_count, s->stream));
-      tt.launches += 1;
-    }
-    s->records_n = nrec;
-    if (n_out)
-      *n_out = nrec;
-    if (dev_out)
-      *dev_out = s->records;
-  }
-  CU(cudaEventRecord(s->ev1, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  float ms = 0;
-  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-  tt.matches = s->h_totals[0];
-  tt.newlines = s->h_totals[1];
-  if (!stream_route || s->count_newlines)
-    tt.flags |= UGX_TOT_NEWLINES;
-  tt.kernel_ms = ms;
-  if (totals)
-    *totals = tt;
-  return UGX_OK;
+  TRY(run_route(c, r, pipelined));
+  return end_scan(s, c.tt, totals, c.read);
 }
 
 // line records through the span kernels: the selected match starts of span_scan_kernel, then span_lines_kernel's count
@@ -1206,47 +1288,38 @@ int span_lines(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint64
 {
   *valid = false;
   ugx::SpanArgs sa;
-  int rc = span_count_pass(s, p, dbuf, n, true, base_offset, base_line, sa, tt);
-  if (rc != UGX_OK)
-    return rc;
-  if (s->h_totals[2] != 0)
+  TRY(span_count_pass(s, p, dbuf, n, true, base_offset, base_line, sa, tt));
+  if (s->h_totals[ugx::SLOT_HANDOVER] != 0)
     return UGX_OK;
   const uint64_t nreg = ugx::stream_regions(n);
-  rc = ensure(s->lines_regions, s->lines_regions_cap, 5 * nreg + 8);
-  if (rc != UGX_OK)
-    return rc;
-  ugx::SpanLinesArgs a;
-  memset(&a, 0, sizeof(a));
-  a.reg_nl = s->lines_regions;
-  a.reg_m = s->lines_regions + nreg;
-  a.reg_bol = s->lines_regions + 2 * nreg;
-  a.reg_fb = s->lines_regions + 3 * nreg;
-  a.reg_fa = s->lines_regions + 4 * nreg;
-  a.tail = s->lines_regions + 5 * nreg;
-  a.sel_bits = s->span_sel;
+  TRY(s->lines_regions.ensure(5 * nreg + 8));
+  ugx::SpanLinesArgs a{};
+  a.reg_nl = s->lines_regions.p;
+  a.reg_m = s->lines_regions.p + nreg;
+  a.reg_bol = s->lines_regions.p + 2 * nreg;
+  a.reg_fb = s->lines_regions.p + 3 * nreg;
+  a.reg_fa = s->lines_regions.p + 4 * nreg;
+  a.tail = s->lines_regions.p + 5 * nreg;
+  a.sel_bits = s->span_sel.p;
   a.limit = sa.tail;
   a.base_offset = base_offset;
   a.base_line = base_line;
   a.invert = flags & UGX_LINES_INVERT;
   CU(ugx::launch_span_lines(p->dev, dbuf, n, a, false, s->sm_count, s->stream));
   CU(ugx::launch_span_lines_final(p->dev, dbuf, n, a, s->totals, s->stream));
-  CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
+  uint64_t nrec = 0;
+  TRY(read_count(s, 2, s->lines, &nrec));
   tt->launches += 2;
-  const uint64_t nrec = s->h_totals[0];
-  rc = ensure(s->lines, s->lines_cap, nrec);
-  if (rc != UGX_OK)
-    return rc;
   if (nrec > 0)
   {
-    a.out = s->lines;
+    a.out = s->lines.p;
     a.out_cap = nrec;
     CU(ugx::launch_span_lines(p->dev, dbuf, n, a, true, s->sm_count, s->stream));
     tt->launches += 1;
   }
   s->lines_n = nrec;
   tt->matches = nrec;
-  tt->newlines = s->h_totals[1];
+  tt->newlines = s->h_totals[ugx::SLOT_NEWLINES];
   tt->flags |= UGX_TOT_NEWLINES;
   tt->kernel = UGX_K_SPAN_LINES;
   *valid = true;
@@ -1262,12 +1335,14 @@ struct Context {
   uint32_t before, after;
 };
 
-int context_stage(ugx_scanner* s, const ugx_pattern* p, ugx::ContextArgs& a, const uint64_t* fsel_host,
-                  const std::vector<uint64_t>& ftile_host, uint64_t* first_out, ugx_totals* tt)
+int context_stage(ugx_scanner* s, const ugx_pattern* p, const Context& ctx, uint32_t flags, ugx::ContextArgs& a,
+                  const uint64_t* fsel_host, const std::vector<uint64_t>& ftile_host, uint64_t* first_out, ugx_totals* tt)
 {
+  a.before = ctx.before;
+  a.after = ctx.after;
+  a.invert = flags & UGX_LINES_INVERT;
   const uint64_t nsel = s->lines_n;
-  std::swap(s->lines, s->ctx_sel);
-  std::swap(s->lines_cap, s->ctx_sel_cap);
+  s->lines.swap(s->ctx_sel);
   s->lines_n = 0;
   const bool batch = fsel_host != nullptr;
   const uint64_t nf = batch ? a.nfiles + 1 : 0;
@@ -1278,13 +1353,11 @@ int context_stage(ugx_scanner* s, const ugx_pattern* p, ugx::ContextArgs& a, con
     return UGX_OK;
   }
   const uint64_t nblk = ugx::context_blocks(nsel);
-  int rc = ensure(s->ctx_pos, s->ctx_pos_cap, nsel + 2 * nblk + 3 * nf);
-  if (rc != UGX_OK)
-    return rc;
-  a.sel = s->ctx_sel;
+  TRY(s->ctx_pos.ensure(nsel + 2 * nblk + 3 * nf));
+  a.sel = s->ctx_sel.p;
   a.nsel = nsel;
-  a.pos = s->ctx_pos;
-  a.blk = s->ctx_pos + nsel;
+  a.pos = s->ctx_pos.p;
+  a.blk = s->ctx_pos.p + nsel;
   if (batch)
   {
     uint64_t* d_fsel = a.blk + 2 * nblk;
@@ -1296,14 +1369,10 @@ int context_stage(ugx_scanner* s, const ugx_pattern* p, ugx::ContextArgs& a, con
   }
   CU(ugx::launch_context_count(a, s->stream));
   CU(ugx::launch_tile_prefix(a.blk, a.blk + nblk, nblk, s->totals, s->stream));
-  CU(cudaMemcpyAsync(s->h_totals, s->totals, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
+  uint64_t nout = 0;
+  TRY(read_count(s, 1, s->lines, &nout));
   tt->launches += 2;
-  const uint64_t nout = s->h_totals[0];
-  rc = ensure(s->lines, s->lines_cap, nout);
-  if (rc != UGX_OK)
-    return rc;
-  a.out = s->lines;
+  a.out = s->lines.p;
   a.nout = nout;
   CU(ugx::launch_context_emit(a, s->sm_count, s->stream));
   tt->launches += 1;
@@ -1325,66 +1394,35 @@ int select_lines(ugx_scanner* s, const ugx_pattern* p, const uint8_t* dbuf, uint
                  uint64_t base_line, ugx_totals* tt)
 {
   int rc;
-  bool done = false;
-  if (!p->never && !s->force_generic && !s->no_span && ugx::span_scan_eligible(p->dev))
+  if (span_route(s, p))
   {
+    bool done = false;
     rc = span_lines(s, p, dbuf, n, flags, base_offset, base_line, tt, &done);
-    if (rc != UGX_OK)
+    if (rc != UGX_OK || done)
       return rc;
-    if (!done)
-    {
-      tt->launches = 0; // the line-at-a-time kernels take over
-      tt->flags |= UGX_TOT_SPAN_HANDOVER;
-    }
+    tt->launches = 0; // the line-at-a-time kernels take over
+    tt->flags |= UGX_TOT_SPAN_HANDOVER;
   }
-  if (!done)
+  // the line-at-a-time kernels: a count pass into strip_counts, the tile prefix, an emit pass.  A pattern whose
+  // prefilter admits no candidate searches no line (all lines are records of the inverted form).
+  ugx::ScanArgs a;
+  TRY(line_scan_args(s, p, dbuf, n, true, base_offset, base_line, a));
+  const uint32_t lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
+  CU(ugx::launch_scan_line_records(p->dev, a, nullptr, lflags, false, s->sm_count, s->stream));
+  CU(ugx::launch_tile_prefix(a.tile_matches, a.tile_newlines, a.ntiles, s->totals, s->stream));
+  uint64_t nrec = 0;
+  TRY(read_count(s, 2, s->lines, &nrec));
+  tt->launches += 2;
+  if (nrec > 0)
   {
-    // the line-at-a-time kernels: a count pass into strip_counts, the tile prefix, an emit pass.  A pattern whose
-    // prefilter admits no candidate searches no line (all lines are records of the inverted form).
-    const uint64_t tile_bytes = ugx::scan_tile_bytes(p->dev);
-    const uint64_t ntiles = (n + tile_bytes - 1) / tile_bytes;
-    const uint64_t nstrips = (n + ugx::SCAN_STRIP - 1) / ugx::SCAN_STRIP;
-    uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
-    rc = ensure(s->tile_matches, cap1, ntiles);
-    if (rc == UGX_OK)
-      rc = ensure(s->tile_newlines, cap2, ntiles);
-    s->tiles_cap = cap1 < cap2 ? cap1 : cap2;
-    if (rc == UGX_OK)
-      rc = ensure(s->strip_counts, s->strips_cap, nstrips);
-    if (rc != UGX_OK)
-      return rc;
-    ugx::ScanArgs a;
-    a.buf = dbuf;
-    a.n = n;
-    a.ntiles = ntiles;
-    a.tile_matches = s->tile_matches;
-    a.tile_newlines = s->tile_newlines;
-    a.strip_counts = s->strip_counts;
-    a.out = nullptr;
-    a.out_cap = 0;
-    a.base_offset = base_offset;
-    a.base_line = base_line;
-    const uint32_t lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
-    CU(ugx::launch_scan_line_records(p->dev, a, nullptr, lflags, false, s->sm_count, s->stream));
-    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
-    CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    tt->launches += 2;
-    const uint64_t nrec = s->h_totals[0];
-    rc = ensure(s->lines, s->lines_cap, nrec);
-    if (rc != UGX_OK)
-      return rc;
-    if (nrec > 0)
-    {
-      a.out_cap = nrec;
-      CU(ugx::launch_scan_line_records(p->dev, a, s->lines, lflags, true, s->sm_count, s->stream));
-      tt->launches += 1;
-    }
-    s->lines_n = nrec;
-    tt->matches = nrec;
-    tt->newlines = s->h_totals[1];
-    tt->kernel = UGX_K_LINE_SCAN;
+    a.out_cap = nrec;
+    CU(ugx::launch_scan_line_records(p->dev, a, s->lines.p, lflags, true, s->sm_count, s->stream));
+    tt->launches += 1;
   }
+  s->lines_n = nrec;
+  tt->matches = nrec;
+  tt->newlines = s->h_totals[ugx::SLOT_NEWLINES];
+  tt->kernel = UGX_K_LINE_SCAN;
   return UGX_OK;
 }
 
@@ -1392,65 +1430,30 @@ int find_lines_common(ugx_scanner* s, const ugx_pattern* p, const void* buf, uin
                       uint64_t base_line, uint32_t flags, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals,
                       const Context* ctx = nullptr)
 {
-  const char* who = ctx ? "ugx_find_context" : "ugx_find_lines";
-  if (s == nullptr || p == nullptr || (buf == nullptr && n != 0))
-    return fail(UGX_E_INVALID, "null argument");
-  if ((flags & ~UGX_LINES_INVERT) != 0)
-    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
-  if (s->device != p->device)
-    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
+  TRY(check_scan(ctx ? "ugx_find_context" : "ugx_find_lines", s, p, buf, n, flags));
+  ugx_totals tt{};
   tt.flags = UGX_TOT_NEWLINES;
-  if (n_out)
-    *n_out = 0;
-  if (dev_out)
-    *dev_out = nullptr;
+  set_records<ugx_line>(dev_out, n_out, nullptr, 0);
   if (n == 0)
-  {
     s->lines_n = 0;
-    if (totals)
-      *totals = tt;
+  const uint8_t* dbuf;
+  TRY(begin_scan(s, buf, n, tt, totals, &dbuf));
+  if (dbuf == nullptr)
     return UGX_OK;
-  }
-  CU(cudaSetDevice(s->device));
-  const uint8_t* dbuf = nullptr;
-  uint64_t h2d = 0;
-  int rc = resolve(s, buf, n, &dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
-  CU(cudaEventRecord(s->ev0, s->stream));
-  rc = select_lines(s, p, dbuf, n, flags, base_offset, base_line, &tt);
-  if (rc != UGX_OK)
-    return rc;
+  TRY(select_lines(s, p, dbuf, n, flags, base_offset, base_line, &tt));
   if (ctx != nullptr)
   {
-    ugx::ContextArgs a;
-    memset(&a, 0, sizeof(a));
+    ugx::ContextArgs a{};
     a.buf = dbuf;
     a.n = n;
     a.nl_total = tt.newlines;
     a.base_offset = base_offset;
     a.base_line = base_line;
     a.nfiles = 1;
-    a.before = ctx->before;
-    a.after = ctx->after;
-    a.invert = flags & UGX_LINES_INVERT;
-    rc = context_stage(s, p, a, nullptr, {}, nullptr, &tt);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(context_stage(s, p, *ctx, flags, a, nullptr, {}, nullptr, &tt));
   }
-  CU(cudaEventRecord(s->ev1, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  float ms = 0;
-  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-  tt.kernel_ms = ms;
-  if (n_out)
-    *n_out = s->lines_n;
-  if (dev_out)
-    *dev_out = s->lines;
-  if (totals)
-    *totals = tt;
+  TRY(end_scan(s, tt, totals));
+  set_records(dev_out, n_out, s->lines.p, s->lines_n);
   return UGX_OK;
 }
 
@@ -1461,21 +1464,8 @@ int find_lines_to_host(ugx_scanner* s, const ugx_pattern* p, const void* buf, ui
 {
   const ugx_line* dev = nullptr;
   uint64_t n = 0;
-  int rc = find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, &dev, &n, totals, ctx);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  if (n > cap)
-    return fail(UGX_E_OVERFLOW, "line record buffer too small");
-  if (n > 0)
-  {
-    if (out == nullptr)
-      return fail(UGX_E_INVALID, "null record buffer");
-    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-  }
-  return UGX_OK;
+  TRY(find_lines_common(s, p, buf, nbytes, base_offset, base_line, flags, &dev, &n, totals, ctx));
+  return copy_out(s, dev, sizeof(ugx_line), n, out, cap, n_out, false, "line record buffer too small");
 }
 
 // ugx_*_lines_bool: every check before any device work
@@ -1490,10 +1480,7 @@ int bool_check(const ugx_scanner* s, const ugx_pattern* const* patterns, uint32_
     return fail(UGX_E_UNSUPPORTED, "ugx_lines_bool: more than 32 patterns or 64 clauses");
   for (uint32_t j = 0; j < npatterns; ++j)
   {
-    if (patterns[j] == nullptr)
-      return fail(UGX_E_INVALID, "null argument");
-    if (patterns[j]->device != s->device)
-      return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
+    TRY(check_scan("ugx_lines_bool", s, patterns[j], buf, n));
   }
   const uint32_t terms = npatterns == 32 ? ~0u : (1u << npatterns) - 1u;
   for (uint32_t c = 0; c < nclauses; ++c)
@@ -1514,39 +1501,21 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
                 uint32_t nclauses, const void* buf, uint64_t n, uint64_t base_offset, uint64_t base_line, uint32_t flags,
                 bool want_records, const ugx_line** dev_out, uint64_t* n_out, ugx_totals* totals)
 {
-  int rc = bool_check(s, patterns, npatterns, clauses, nclauses, buf, n, flags);
-  if (rc != UGX_OK)
-    return rc;
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
+  TRY(bool_check(s, patterns, npatterns, clauses, nclauses, buf, n, flags));
+  ugx_totals tt{};
   tt.flags = UGX_TOT_NEWLINES;
   tt.kernel = UGX_K_BOOL_LINES;
-  if (n_out)
-    *n_out = 0;
-  if (dev_out)
-    *dev_out = nullptr;
+  set_records<ugx_line>(dev_out, n_out, nullptr, 0);
   s->lines_n = 0;
-  if (n == 0)
-  {
-    if (totals)
-      *totals = tt;
+  const uint8_t* dbuf;
+  TRY(begin_scan(s, buf, n, tt, totals, &dbuf));
+  if (dbuf == nullptr)
     return UGX_OK;
-  }
-  CU(cudaSetDevice(s->device));
-  const uint8_t* dbuf = nullptr;
-  uint64_t h2d = 0;
-  rc = resolve(s, buf, n, &dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
-  CU(cudaEventRecord(s->ev0, s->stream));
   uint64_t nlines = 0;
   for (uint32_t j = 0; j < npatterns; ++j)
   {
-    ugx_totals t;
-    memset(&t, 0, sizeof(t));
-    rc = select_lines(s, patterns[j], dbuf, n, 0, 0, 0, &t);
-    if (rc != UGX_OK)
-      return rc;
+    ugx_totals t{};
+    TRY(select_lines(s, patterns[j], dbuf, n, 0, 0, 0, &t));
     tt.launches += t.launches;
     tt.flags |= t.flags & UGX_TOT_SPAN_HANDOVER;
     if (j == 0)
@@ -1556,20 +1525,17 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
       CU(cudaStreamSynchronize(s->stream));
       tt.newlines = t.newlines;
       nlines = t.newlines + (last != '\n' ? 1u : 0u);
-      rc = ensure(s->bool_mask, s->bool_mask_cap, nlines);
-      if (rc != UGX_OK)
-        return rc;
-      CU(cudaMemsetAsync(s->bool_mask, 0, nlines * sizeof(uint32_t), s->stream));
+      TRY(s->bool_mask.ensure(nlines));
+      CU(cudaMemsetAsync(s->bool_mask.p, 0, nlines * sizeof(uint32_t), s->stream));
     }
     if (s->lines_n > 0)
     {
-      CU(ugx::launch_bool_mark(s->lines, s->lines_n, s->bool_mask, 1u << j, s->sm_count, s->stream));
+      CU(ugx::launch_bool_mark(s->lines.p, s->lines_n, s->bool_mask.p, 1u << j, s->sm_count, s->stream));
       tt.launches += 1;
     }
   }
   s->lines_n = 0;
-  ugx::BoolQuery q;
-  memset(&q, 0, sizeof(q));
+  ugx::BoolQuery q{};
   for (uint32_t c = 0; c < nclauses; ++c)
   {
     q.pos[c] = clauses[c].pos;
@@ -1579,50 +1545,35 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
   q.invert = flags & UGX_LINES_INVERT;
   const uint64_t nlb = ugx::bool_line_blocks(nlines), nreg = want_records ? ugx::bool_regions(n) : 0;
   const uint64_t nblk = nlb > nreg ? nlb : nreg;
-  rc = ensure(s->bool_pos, s->bool_pos_cap, 2 * nblk + (want_records ? nlines : 0));
-  if (rc != UGX_OK)
-    return rc;
-  ugx::BoolArgs a;
-  memset(&a, 0, sizeof(a));
+  TRY(s->bool_pos.ensure(2 * nblk + (want_records ? nlines : 0)));
+  ugx::BoolArgs a{};
   a.buf = dbuf;
   a.n = n;
   a.nlines = nlines;
-  a.mask = s->bool_mask;
-  a.blk = s->bool_pos;
+  a.mask = s->bool_mask.p;
+  a.blk = s->bool_pos.p;
   a.nblocks = nblk;
   a.want_index = want_records ? 1u : 0u;
-  a.eol = s->bool_pos + 2 * nblk;
+  a.eol = s->bool_pos.p + 2 * nblk;
   a.base_offset = base_offset;
   a.base_line = base_line;
   CU(ugx::launch_bool_count(a, q, s->stream));
   CU(ugx::launch_tile_prefix(a.blk, a.blk + nblk, nblk, s->totals, s->stream));
-  CU(cudaMemcpyAsync(s->h_totals, s->totals, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
+  TRY(read_totals(s, 1));
   tt.launches += 2;
-  const uint64_t nsel = s->h_totals[0];
+  const uint64_t nsel = s->h_totals[ugx::SLOT_MATCHES];
   tt.matches = nsel;
   if (want_records && nsel > 0)
   {
-    rc = ensure(s->lines, s->lines_cap, nsel);
-    if (rc != UGX_OK)
-      return rc;
-    a.out = s->lines;
+    TRY(s->lines.ensure(nsel));
+    a.out = s->lines.p;
     CU(ugx::launch_bool_index(a, s->stream));
     CU(ugx::launch_bool_emit(a, q, s->stream));
     tt.launches += 2;
     s->lines_n = nsel;
   }
-  CU(cudaEventRecord(s->ev1, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  float ms = 0;
-  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-  tt.kernel_ms = ms;
-  if (n_out)
-    *n_out = s->lines_n;
-  if (dev_out)
-    *dev_out = s->lines;
-  if (totals)
-    *totals = tt;
+  TRY(end_scan(s, tt, totals));
+  set_records(dev_out, n_out, s->lines.p, s->lines_n);
   return UGX_OK;
 }
 
@@ -1681,36 +1632,16 @@ int ugx_find_lines_bool(ugx_scanner* s, const ugx_pattern* const* patterns, uint
 {
   const ugx_line* dev = nullptr;
   uint64_t n = 0;
-  int rc = bool_common(s, patterns, npatterns, clauses, nclauses, buf, nbytes, base_offset, base_line, flags, true, &dev,
-                       &n, totals);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  if (n > cap)
-    return fail(UGX_E_OVERFLOW, "line record buffer too small");
-  if (n > 0)
-  {
-    if (out == nullptr)
-      return fail(UGX_E_INVALID, "null record buffer");
-    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-  }
-  return UGX_OK;
+  TRY(bool_common(s, patterns, npatterns, clauses, nclauses, buf, nbytes, base_offset, base_line, flags, true, &dev,
+                       &n, totals));
+  return copy_out(s, dev, sizeof(ugx_line), n, out, cap, n_out, false, "line record buffer too small");
 }
 
 int ugx_scanner_fetch_lines(ugx_scanner* s, ugx_line* out, uint64_t first, uint64_t count)
 {
   if (s == nullptr || (out == nullptr && count != 0))
     return fail(UGX_E_INVALID, "null argument");
-  if (first > s->lines_n || count > s->lines_n - first)
-    return fail(UGX_E_INVALID, "record range outside the last line-record result");
-  if (count == 0)
-    return UGX_OK;
-  CU(cudaSetDevice(s->device));
-  CU(cudaMemcpyAsync(out, s->lines + first, count * sizeof(ugx_line), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  return UGX_OK;
+  return fetch(s, s->lines, s->lines_n, out, first, count, "record range outside the last line-record result");
 }
 
 int ugx_count_lines(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, ugx_totals* totals)
@@ -1734,21 +1665,8 @@ int ugx_find_all(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t
 {
   const ugx_match* dev = nullptr;
   uint64_t n = 0;
-  int rc = scan_common(s, p, buf, nbytes, 1, true, base_offset, base_line, &dev, &n, totals);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  if (n > cap)
-    return fail(UGX_E_OVERFLOW, "record buffer too small");
-  if (n > 0)
-  {
-    if (out == nullptr)
-      return fail(UGX_E_INVALID, "null record buffer");
-    CU(cudaMemcpyAsync(out, dev, n * sizeof(ugx_match), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-  }
-  return UGX_OK;
+  TRY(scan_common(s, p, buf, nbytes, 1, true, base_offset, base_line, &dev, &n, totals));
+  return copy_out(s, dev, sizeof(ugx_match), n, out, cap, n_out, false, "record buffer too small");
 }
 
 const char* ugx_kernel_name(uint32_t id)
@@ -1775,61 +1693,24 @@ int ugx_scanner_set_option(ugx_scanner* s, const char* name, int value)
 {
   if (s == nullptr || name == nullptr)
     return fail(UGX_E_INVALID, "null argument");
-  if (strcmp(name, "force_generic") == 0)
-  {
-    s->force_generic = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "legacy_any") == 0)
-  {
-    s->legacy_any = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "match_lines") == 0)
-  {
-    s->match_lines = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "two_pass_records") == 0)
-  {
-    s->two_pass_records = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "no_pipeline") == 0)
-  {
-    s->no_pipeline = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "stream_dfa") == 0)
-  {
-    s->stream_dfa = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "no_feeder") == 0)
-  {
-    s->no_feeder = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "no_span") == 0)
-  {
-    s->no_span = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "no_cover") == 0)
-  {
-    s->no_cover = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "no_search") == 0)
-  {
-    s->no_search = value != 0;
-    return UGX_OK;
-  }
-  if (strcmp(name, "count_newlines") == 0)
-  {
-    s->count_newlines = value != 0;
-    return UGX_OK;
-  }
+  using Flag = bool ugx_scanner::*;
+  static const struct {
+    const char* name;
+    Flag flag;
+  } options[] = {
+      {"force_generic", &ugx_scanner::force_generic}, {"legacy_any", &ugx_scanner::legacy_any},
+      {"match_lines", &ugx_scanner::match_lines},     {"two_pass_records", &ugx_scanner::two_pass_records},
+      {"no_pipeline", &ugx_scanner::no_pipeline},     {"stream_dfa", &ugx_scanner::stream_dfa},
+      {"no_feeder", &ugx_scanner::no_feeder},         {"no_span", &ugx_scanner::no_span},
+      {"no_cover", &ugx_scanner::no_cover},           {"no_search", &ugx_scanner::no_search},
+      {"count_newlines", &ugx_scanner::count_newlines},
+  };
+  for (const auto& o : options)
+    if (strcmp(name, o.name) == 0)
+    {
+      s->*o.flag = value != 0;
+      return UGX_OK;
+    }
   return fail(UGX_E_INVALID, std::string("unknown scanner option ") + name);
 }
 
@@ -1837,14 +1718,7 @@ int ugx_scanner_fetch(ugx_scanner* s, ugx_match* out, uint64_t first, uint64_t c
 {
   if (s == nullptr || (out == nullptr && count != 0))
     return fail(UGX_E_INVALID, "null argument");
-  if (first > s->records_n || count > s->records_n - first)
-    return fail(UGX_E_INVALID, "record range outside the last result");
-  if (count == 0)
-    return UGX_OK;
-  CU(cudaSetDevice(s->device));
-  CU(cudaMemcpyAsync(out, s->records + first, count * sizeof(ugx_match), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  return UGX_OK;
+  return fetch(s, s->records, s->records_n, out, first, count, "record range outside the last result");
 }
 
 } // extern "C"
@@ -1879,22 +1753,14 @@ int batch_tiles(const char* who, uint64_t nbytes, const uint64_t* begins, const 
   return UGX_OK;
 }
 
-// the buffer made visible to the device, the file and tile tables uploaded and the per-file counters zeroed, all on the
+// begin_scan's setup for a batch: the file and tile tables uploaded and the per-file counters zeroed, all on the
 // scanner's stream: b.a is ready for a launch
-int batch_upload(ugx_scanner* s, const void* buf, uint64_t nbytes, const uint64_t* begins, const uint64_t* lens,
-                 uint64_t nfiles, Batch& b)
+int batch_upload(ugx_scanner* s, const uint64_t* begins, const uint64_t* lens, uint64_t nfiles, Batch& b)
 {
-  CU(cudaSetDevice(s->device));
-  uint64_t h2d = 0;
-  int rc = resolve(s, buf, nbytes, &b.dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
   // one scratch block: begins | lens | counts | tile_file | tile_index
   const uint64_t words = 3 * nfiles + (b.tf.size() + 1) / 2 * 2;
-  rc = ensure(s->batch, s->batch_cap, words + 4);
-  if (rc != UGX_OK)
-    return rc;
-  uint64_t* d_begins = s->batch;
+  TRY(s->batch.ensure(words + 4));
+  uint64_t* d_begins = s->batch.p;
   uint64_t* d_lens = d_begins + nfiles;
   unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(d_lens + nfiles);
   uint32_t* d_tf = reinterpret_cast<uint32_t*>(d_counts + nfiles);
@@ -1916,46 +1782,45 @@ int batch_upload(ugx_scanner* s, const void* buf, uint64_t nbytes, const uint64_
 
 // match records (lines == false) or line records of a batch: the count pass, the tile prefix, then the per-file counts
 // and the totals to the host in the one synchronise that sizes the arena, and the emit pass into the scanner's match or
-// line arena.  first[nfiles + 1] receives every file's record range, *n_out the number of records.
+// line arena.  first[nfiles + 1] receives every file's record range, *n_out the number of records, out[cap] the
+// records (out == NULL with cap == 0: they stay on the device).
 int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
-                  const uint64_t* lens, uint64_t nfiles, bool lines, uint32_t flags, uint64_t* first, uint64_t* n_out,
-                  ugx_totals* totals, const Context* ctx = nullptr)
+                  const uint64_t* lens, uint64_t nfiles, bool lines, uint32_t flags, uint64_t* first, void* out, uint64_t cap,
+                  uint64_t* n_out, ugx_totals* totals, const Context* ctx = nullptr)
 {
+  if (n_out)
+    *n_out = 0;
   const char* who = ctx ? "ugx_find_context_batch" : lines ? "ugx_find_lines_batch" : "ugx_find_all_batch";
   if (s == nullptr || p == nullptr || (buf == nullptr && nbytes != 0) ||
       (nfiles != 0 && (begins == nullptr || lens == nullptr || first == nullptr)))
     return fail(UGX_E_INVALID, std::string(who) + ": bad argument");
-  if ((flags & ~UGX_LINES_INVERT) != 0)
-    return fail(UGX_E_INVALID, std::string(who) + ": unknown flags");
-  if (s->device != p->device)
-    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
+  TRY(check_scan(who, s, p, buf, nbytes, flags));
+  ugx_totals tt{};
   tt.flags = UGX_TOT_NEWLINES;
   if (totals)
     *totals = tt;
-  *n_out = 0;
   if (first != nullptr)
     first[0] = 0;
+  uint64_t& arena_n = lines ? s->lines_n : s->records_n;
   if (nfiles == 0)
   {
-    (lines ? s->lines_n : s->records_n) = 0;
+    arena_n = 0;
     return UGX_OK;
   }
-  try
-  {
+  return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     Batch b;
-    int rc = batch_tiles(who, nbytes, begins, lens, nfiles, b);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(batch_tiles(who, nbytes, begins, lens, nfiles, b));
     // the arena is rewritten below: its last result is gone from here on
-    (lines ? s->lines_n : s->records_n) = 0;
+    arena_n = 0;
     memset(first, 0, (nfiles + 1) * sizeof(uint64_t));
     if (b.tf.empty())
       return UGX_OK; // only empty files: no lines, no records
-    rc = batch_upload(s, buf, nbytes, begins, lens, nfiles, b);
-    if (rc != UGX_OK)
-      return rc;
+    const uint64_t ntiles = b.tf.size();
+    TRY(begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&]() -> int {
+      TRY(batch_upload(s, begins, lens, nfiles, b));
+      TRY(ensure_tiles(s, ntiles));
+      return s->strip_counts.ensure(ntiles * ugx::SCAN_THREADS);
+    }));
     // with context, first[] receives the printed lines' ranges and the selected records' ranges go to sfirst
     std::vector<uint64_t> ctx_first;
     uint64_t* sfirst = first;
@@ -1964,110 +1829,61 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
       ctx_first.assign(nfiles + 1, 0);
       sfirst = ctx_first.data();
     }
-    const uint64_t ntiles = b.tf.size();
-    uint64_t cap1 = s->tiles_cap, cap2 = s->tiles_cap;
-    rc = ensure(s->tile_matches, cap1, ntiles);
-    if (rc == UGX_OK)
-      rc = ensure(s->tile_newlines, cap2, ntiles);
-    s->tiles_cap = cap1 < cap2 ? cap1 : cap2;
-    if (rc == UGX_OK)
-      rc = ensure(s->strip_counts, s->strips_cap, ntiles * ugx::SCAN_THREADS);
-    if (rc != UGX_OK)
-      return rc;
     ugx::BatchRecordArgs r;
-    r.tile_matches = s->tile_matches;
-    r.tile_newlines = s->tile_newlines;
-    r.strip_counts = s->strip_counts;
+    r.tile_matches = s->tile_matches.p;
+    r.tile_newlines = s->tile_newlines.p;
+    r.strip_counts = s->strip_counts.p;
     r.out = nullptr;
     r.lout = nullptr;
     r.out_cap = 0;
     // a prefilter that admits no candidate (config 3) searches no line: no match records, and the inverted line
     // records are every line
     r.lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
-    CU(cudaEventRecord(s->ev0, s->stream));
     CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, false, s->sm_count, s->stream));
-    CU(ugx::launch_tile_prefix(s->tile_matches, s->tile_newlines, ntiles, s->totals, s->stream));
+    CU(ugx::launch_tile_prefix(s->tile_matches.p, s->tile_newlines.p, ntiles, s->totals, s->stream));
     CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
     CU(cudaMemcpyAsync(sfirst + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
     CU(cudaStreamSynchronize(s->stream));
     tt.launches = 2;
-    const uint64_t nrec = s->h_totals[0];
-    const uint64_t nl_total = s->h_totals[1];
+    const uint64_t nrec = s->h_totals[ugx::SLOT_MATCHES];
+    const uint64_t nl_total = s->h_totals[ugx::SLOT_NEWLINES];
     for (uint64_t f = 0; f < nfiles; ++f)
       sfirst[f + 1] += sfirst[f];
     if (sfirst[nfiles] != nrec)
       return fail(UGX_E_CUDA, std::string(who) + ": per-file record counts disagree with the total");
-    if (lines)
-      rc = ensure(s->lines, s->lines_cap, nrec);
-    else
-      rc = ensure(s->records, s->records_cap, nrec);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(lines ? s->lines.ensure(nrec) : s->records.ensure(nrec));
     if (nrec > 0)
     {
-      r.out = lines ? nullptr : s->records;
-      r.lout = lines ? s->lines : nullptr;
+      r.out = lines ? nullptr : s->records.p;
+      r.lout = lines ? s->lines.p : nullptr;
       r.out_cap = nrec;
       CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, true, s->sm_count, s->stream));
       tt.launches += 1;
     }
-    (lines ? s->lines_n : s->records_n) = nrec;
+    arena_n = nrec;
     if (ctx != nullptr)
     {
       // every file's first batch tile: the tiles are ordered by file
       std::vector<uint64_t> ftile(nfiles + 1, 0);
       for (uint64_t f = 0; f < nfiles; ++f)
         ftile[f + 1] = ftile[f] + (lens[f] + ugx::SCAN_TILE - 1) / ugx::SCAN_TILE;
-      ugx::ContextArgs c;
-      memset(&c, 0, sizeof(c));
+      ugx::ContextArgs c{};
       c.buf = b.dbuf;
       c.nl_total = nl_total;
       c.nfiles = nfiles;
       c.begins = b.a.begins;
       c.lens = b.a.lens;
-      c.tile_nl = s->tile_newlines;
+      c.tile_nl = s->tile_newlines.p;
       c.ntiles = ntiles;
-      c.before = ctx->before;
-      c.after = ctx->after;
-      c.invert = flags & UGX_LINES_INVERT;
-      rc = context_stage(s, p, c, sfirst, ftile, first, &tt);
-      if (rc != UGX_OK)
-        return rc;
+      TRY(context_stage(s, p, *ctx, flags, c, sfirst, ftile, first, &tt));
     }
-    CU(cudaEventRecord(s->ev1, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    *n_out = lines ? s->lines_n : s->records_n;
     tt.matches = nrec;
     tt.newlines = nl_total;
-    tt.kernel_ms = ms;
     tt.kernel = UGX_K_BATCH;
-    if (totals)
-      *totals = tt;
-    return UGX_OK;
-  }
-  catch (const std::bad_alloc&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
-}
-
-// the host side of ugx_find_{all,lines}_batch: out == NULL with cap == 0 leaves the records on the device
-int batch_copy_out(ugx_scanner* s, const void* dev, size_t rec_bytes, void* out, uint64_t cap, uint64_t n)
-{
-  if (out == nullptr && cap == 0)
-    return UGX_OK;
-  if (n > cap)
-    return fail(UGX_E_OVERFLOW, "record buffer too small");
-  if (n > 0)
-  {
-    if (out == nullptr)
-      return fail(UGX_E_INVALID, "null record buffer");
-    CU(cudaMemcpyAsync(out, dev, n * rec_bytes, cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-  }
-  return UGX_OK;
+    TRY(end_scan(s, tt, totals));
+    return lines ? copy_out(s, s->lines.p, sizeof(ugx_line), arena_n, out, cap, n_out, true, "record buffer too small")
+                 : copy_out(s, s->records.p, sizeof(ugx_match), arena_n, out, cap, n_out, true, "record buffer too small");
+  });
 }
 
 } // namespace
@@ -2080,92 +1896,53 @@ int ugx_count_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint6
   if (s == nullptr || p == nullptr || (buf == nullptr && nbytes != 0) || (nfiles != 0 && (begins == nullptr || lens == nullptr || counts == nullptr)) ||
       (mode != UGX_MODE_LINES && mode != UGX_MODE_MATCHES))
     return fail(UGX_E_INVALID, "ugx_count_batch: bad argument");
-  if (s->device != p->device)
-    return fail(UGX_E_INVALID, "pattern and scanner live on different devices");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
+  TRY(check_scan("ugx_count_batch", s, p, buf, nbytes));
+  ugx_totals tt{};
   if (totals)
     *totals = tt;
   if (nfiles == 0)
     return UGX_OK;
-  try
-  {
+  return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     Batch b;
-    int rc = batch_tiles("ugx_count_batch", nbytes, begins, lens, nfiles, b);
-    if (rc != UGX_OK)
-      return rc;
+    TRY(batch_tiles("ugx_count_batch", nbytes, begins, lens, nfiles, b));
     memset(counts, 0, nfiles * sizeof(uint64_t));
     if (b.tf.empty() || p->never)
       return UGX_OK; // only empty files, or a prefilter that admits no candidate (config 3): nothing matches
-    rc = batch_upload(s, buf, nbytes, begins, lens, nfiles, b);
-    if (rc != UGX_OK)
-      return rc;
-    CU(cudaEventRecord(s->ev0, s->stream));
+    TRY(begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&] { return batch_upload(s, begins, lens, nfiles, b); }));
     CU(ugx::launch_scan_batch(p->dev, b.dbuf, b.a, mode, s->sm_count, s->stream));
-    CU(cudaEventRecord(s->ev1, s->stream));
+    CU(cudaEventRecord(s->ev1, s->stream)); // the counts' copy is not kernel time
     CU(cudaMemcpyAsync(counts, b.a.counts, nfiles * 8, cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    TRY(end_scan(s, tt, nullptr, 0, true));
     for (uint64_t f = 0; f < nfiles; ++f)
       tt.matches += counts[f];
-    tt.kernel_ms = ms;
     tt.launches = 1;
     tt.kernel = UGX_K_BATCH;
     if (totals)
       *totals = tt;
     return UGX_OK;
-  }
-  catch (const std::bad_alloc&)
-  {
-    return fail(UGX_E_NOMEM, "out of host memory");
-  }
+  });
 }
 
 int ugx_find_all_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                        const uint64_t* lens, uint64_t nfiles, uint64_t* first, ugx_match* out, uint64_t cap,
                        uint64_t* n_out, ugx_totals* totals)
 {
-  uint64_t n = 0;
-  if (n_out)
-    *n_out = 0;
-  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, false, 0, first, &n, totals);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  return batch_copy_out(s, s->records, sizeof(ugx_match), out, cap, n);
+  return batch_records(s, p, buf, nbytes, begins, lens, nfiles, false, 0, first, out, cap, n_out, totals);
 }
 
 int ugx_find_lines_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                          const uint64_t* lens, uint64_t nfiles, uint32_t flags, uint64_t* first, ugx_line* out,
                          uint64_t cap, uint64_t* n_out, ugx_totals* totals)
 {
-  uint64_t n = 0;
-  if (n_out)
-    *n_out = 0;
-  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, &n, totals);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  return batch_copy_out(s, s->lines, sizeof(ugx_line), out, cap, n);
+  return batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, out, cap, n_out, totals);
 }
 
 int ugx_find_context_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                            const uint64_t* lens, uint64_t nfiles, uint32_t flags, uint32_t before, uint32_t after,
                            uint64_t* first, ugx_line* out, uint64_t cap, uint64_t* n_out, ugx_totals* totals)
 {
-  uint64_t n = 0;
-  if (n_out)
-    *n_out = 0;
   const Context ctx{before, after};
-  const int rc = batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, &n, totals, &ctx);
-  if (rc != UGX_OK)
-    return rc;
-  if (n_out)
-    *n_out = n;
-  return batch_copy_out(s, s->lines, sizeof(ugx_line), out, cap, n);
+  return batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, out, cap, n_out, totals, &ctx);
 }
 
 int ugx_check_text(ugx_scanner* s, const void* buf, uint64_t nbytes, ugx_text_info* out)
@@ -2174,27 +1951,22 @@ int ugx_check_text(ugx_scanner* s, const void* buf, uint64_t nbytes, ugx_text_in
     return fail(UGX_E_INVALID, "null argument");
   memset(out, 0, sizeof(*out));
   out->is_utf8 = 1;
-  if (nbytes == 0)
+  ugx_totals tt{};
+  const uint8_t* dbuf;
+  unsigned long long* dflags = s->totals + ugx::SLOT_UTF8;
+  TRY(begin_scan(s, buf, nbytes, tt, nullptr, &dbuf, [&]() -> int {
+    CU(cudaMemsetAsync(dflags, 0, sizeof(unsigned long long), s->stream));
     return UGX_OK;
-  CU(cudaSetDevice(s->device));
-  const uint8_t* dbuf = nullptr;
-  uint64_t h2d = 0;
-  const int rc = resolve(s, buf, nbytes, &dbuf, &h2d);
-  if (rc != UGX_OK)
-    return rc;
-  unsigned int* dflags = reinterpret_cast<unsigned int*>(s->totals + 7);
-  CU(cudaMemsetAsync(dflags, 0, sizeof(unsigned long long), s->stream));
-  CU(cudaEventRecord(s->ev0, s->stream));
-  CU(ugx::launch_utf8_check(dbuf, nbytes, dflags, s->sm_count, s->stream));
-  CU(cudaMemcpyAsync(s->h_totals + 7, s->totals + 7, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-  CU(cudaEventRecord(s->ev1, s->stream));
-  CU(cudaStreamSynchronize(s->stream));
-  float ms = 0;
-  CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-  const unsigned int f = static_cast<unsigned int>(s->h_totals[7]);
+  }));
+  if (dbuf == nullptr)
+    return UGX_OK;
+  CU(ugx::launch_utf8_check(dbuf, nbytes, reinterpret_cast<unsigned int*>(dflags), s->sm_count, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals + ugx::SLOT_UTF8, dflags, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  TRY(end_scan(s, tt, nullptr));
+  const unsigned int f = static_cast<unsigned int>(s->h_totals[ugx::SLOT_UTF8]);
   out->is_utf8 = (f & 1u) == 0;
   out->has_nul = (f & 2u) != 0;
-  out->kernel_ms = ms;
+  out->kernel_ms = tt.kernel_ms;
   out->launches = 1;
   return UGX_OK;
 }
@@ -2203,32 +1975,14 @@ int ugx_count_newlines(ugx_scanner* s, const void* buf, uint64_t nbytes, ugx_tot
 {
   if (s == nullptr || (buf == nullptr && nbytes != 0))
     return fail(UGX_E_INVALID, "null argument");
-  ugx_totals tt;
-  memset(&tt, 0, sizeof(tt));
-  if (nbytes != 0)
-  {
-    CU(cudaSetDevice(s->device));
-    const uint8_t* dbuf = nullptr;
-    uint64_t h2d = 0;
-    const int rc = resolve(s, buf, nbytes, &dbuf, &h2d);
-    if (rc != UGX_OK)
-      return rc;
-    CU(cudaEventRecord(s->ev0, s->stream));
-    CU(ugx::launch_count_newlines(dbuf, nbytes, s->totals + 1, s->sm_count, s->stream));
-    CU(cudaMemcpyAsync(s->h_totals + 1, s->totals + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaEventRecord(s->ev1, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    tt.newlines = s->h_totals[1];
-    tt.kernel_ms = ms;
-    tt.launches = 1;
-    tt.kernel = UGX_K_NEWLINES;
-  }
-  tt.flags |= UGX_TOT_NEWLINES;
-  if (totals)
-    *totals = tt;
-  return UGX_OK;
+  ugx_totals tt{};
+  tt.flags = UGX_TOT_NEWLINES;
+  const uint8_t* dbuf;
+  TRY(begin_scan(s, buf, nbytes, tt, totals, &dbuf));
+  if (dbuf == nullptr)
+    return UGX_OK;
+  TRY(newline_pass(s, dbuf, nbytes, tt));
+  return end_scan(s, tt, totals, READ_NEWLINES);
 }
 
 } // extern "C"

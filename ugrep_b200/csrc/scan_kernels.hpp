@@ -21,6 +21,20 @@ constexpr uint32_t SCAN_LINE_CAP = 1024;                // line starts per tile 
 constexpr uint32_t SCAN_MAX_SMEM_TABLE = 198 * 1024;   // largest transition table staged in shared memory
 constexpr uint32_t ANY_TILE = 32768;                   // bytes per CTA iteration of count_lines_any_kernel
 
+// The slots of a scanner's device array `totals` (and of its pinned host copy).  The kernels that take `totals` write
+// the result slots at [0] and [1]; the span kernels and the UTF-8 check use the others at these fixed offsets.
+enum TotalsSlot : int {
+  SLOT_MATCHES = 0,     // result: matches, matching lines, records or selected lines
+  SLOT_NEWLINES = 1,    // result: newlines
+  SLOT_HANDOVER = 2,    // span count pass: 1 = the spans' result is not valid; single-pass records: the staging cursor
+  SLOT_TAIL_MATCHES = 3, // span_final_kernel: matches before the last line
+  SLOT_TAIL_NEWLINES = 4, // span_final_kernel: newlines before the last line
+  SLOT_LAST_LINE = 5,   // launch_last_line: start of the buffer's last line
+  SLOT_SPAN_FLAGS = 6,  // SpanArgs::flags
+  SLOT_UTF8 = 7,        // launch_utf8_check's flags
+  SLOT_COUNT = 8
+};
+
 struct ScanArgs {
   const uint8_t* buf;
   uint64_t n;
