@@ -413,6 +413,39 @@ int  ugx_find_context_batch(ugx_scanner *s, const ugx_pattern *p, const void *bu
                             const uint64_t *begins, const uint64_t *lens, uint64_t nfiles, uint32_t flags,
                             uint32_t before, uint32_t after, uint64_t *first,
                             ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
+/*
+ * Boolean line queries over many files (`ugrep -rn -e A --and -e B tree/`, `ugrep -rc A --andnot B`, `ugrep -rl --bool
+ * 'A|B -C'`, `-v` with UGX_LINES_INVERT).  The query, its clauses, flags and errors are those of ugx_find_lines_bool;
+ * the file layout is that of ugx_count_batch (host or device buffer, every begins[i] a multiple of 16; the bytes
+ * between files are never text).  File i's records are byte for byte what ugx_find_lines_bool returns for that file
+ * ALONE with the same patterns, clauses and flags and base_offset = base_line = 0: line numbers start at 1 in every
+ * file, offsets count from the file's start, offset = bol, len = 0, cap = M(L) over all K patterns.  counts[i] is what
+ * ugx_count_lines_bool gives for file i alone (`ugrep -rc --and ...`; `-l` is counts[i] != 0, `-L` counts[i] == 0).  An
+ * empty file has no lines and selects nothing, UGX_LINES_INVERT included.
+ *
+ * Records are grouped by file in file order; first[nfiles + 1] (host) receives the ranges, file i owning
+ * [first[i], first[i + 1]).  They live in the line arena (ugx_scanner_fetch_lines pages through them) and the last
+ * ugx_find_all_device result stays valid.  out == NULL with cap == 0: the records stay on the device, UGX_OK.
+ * Otherwise n > cap returns UGX_E_OVERFLOW with *n_out and first[] filled, and the records remain fetchable.
+ * ugx_count_lines_bool_batch leaves the line arena with zero records.
+ *
+ * Errors, all checked before any device work: those of ugx_find_lines_bool, a file that is not a 16-byte aligned range
+ * of the buffer (UGX_E_INVALID), and a null begins, lens, counts or first with nfiles > 0 (UGX_E_INVALID).
+ * nfiles == 0: UGX_OK with first[0] = 0.  A batch of only empty files: zeros, no launch.
+ *
+ * Totals: matches = selected lines over all files; newlines = the files' '\n' bytes (padding is not counted);
+ * UGX_TOT_NEWLINES; launches = every kernel of the call; kernel_ms = the whole call on the device; kernel =
+ * UGX_K_BOOL_LINES.
+ */
+int  ugx_count_lines_bool_batch(ugx_scanner *s, const ugx_pattern *const *patterns, uint32_t npatterns,
+                                const ugx_bool_clause *clauses, uint32_t nclauses,
+                                const void *buf, uint64_t nbytes, const uint64_t *begins, const uint64_t *lens,
+                                uint64_t nfiles, uint32_t flags, uint64_t *counts, ugx_totals *totals);
+int  ugx_find_lines_bool_batch(ugx_scanner *s, const ugx_pattern *const *patterns, uint32_t npatterns,
+                               const ugx_bool_clause *clauses, uint32_t nclauses,
+                               const void *buf, uint64_t nbytes, const uint64_t *begins, const uint64_t *lens,
+                               uint64_t nfiles, uint32_t flags, uint64_t *first,
+                               ugx_line *out, uint64_t cap, uint64_t *n_out, ugx_totals *totals);
 
 /* what ugrep asks about a file before it prints from it (Grep::init_is_binary, src/ugrep.cpp:3998-4017):
  * is_utf8 = reflex::isutf8 (lib/simd.cpp:169-421: valid UTF-8 structure, no NUL), has_nul = memchr(buf, 0, n) != NULL;

@@ -33,7 +33,8 @@ EXPORTS = ["ugx_last_error", "ugx_kernel_name", "ugx_plan_describe", "ugx_abi_ve
            "ugx_viability_describe", "ugx_search_describe", "ugx_check_text", "ugx_compile_literal", "ugx_compile_words", "ugx_compile_words_ex", "ugx_compile_plain_regex", "ugx_count_batch", "ugx_sharded_create", "ugx_sharded_destroy", "ugx_sharded_set_option", "ugx_sharded_scan", "ugx_sharded_last_error", "ugx_find_all", "ugx_find_all_device", "ugx_scanner_fetch", "ugx_scanner_set_option", "ugx_count_newlines",
            "ugx_find_lines", "ugx_find_lines_device", "ugx_scanner_fetch_lines", "ugx_sharded_find_lines",
            "ugx_find_all_batch", "ugx_find_lines_batch", "ugx_find_context", "ugx_find_context_device",
-           "ugx_find_context_batch", "ugx_count_lines_bool", "ugx_find_lines_bool", "ugx_find_lines_bool_device"]
+           "ugx_find_context_batch", "ugx_count_lines_bool", "ugx_find_lines_bool", "ugx_find_lines_bool_device",
+           "ugx_count_lines_bool_batch", "ugx_find_lines_bool_batch"]
 
 
 class UgxError(RuntimeError):
@@ -155,6 +156,10 @@ def lib():
                                                              C.POINTER(C.c_uint64), C.POINTER(_Totals)]
         L.ugx_find_lines_bool.argtypes = bool_args + [C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64,
                                                       C.POINTER(C.c_uint64), C.POINTER(_Totals)]
+        bool_batch = bool_args + [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]
+        L.ugx_count_lines_bool_batch.argtypes = bool_batch + [C.c_void_p, C.POINTER(_Totals)]
+        L.ugx_find_lines_bool_batch.argtypes = bool_batch + [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64),
+                                                             C.POINTER(_Totals)]
         _lib = L
     return _lib
 
@@ -503,6 +508,36 @@ class Scanner:
         offset = bol, len = 0, and cap is the line's term mask: bit j set iff patterns[j] matches on the line."""
         t = self.find_lines_bool_device(patterns, cnf, data, invert, base_offset, base_line)
         return self.fetch_lines(0, self.last_lines[1]), t
+
+    def count_lines_bool_batch(self, patterns, cnf, files, invert: bool = False):
+        """`ugrep -rc -e A --and -e B` of many files in one launch sequence: (per-file counts, totals).  counts[i] is
+        count_lines_bool(file i).matches; `-l` is counts != 0.  `files` as for batch_records_device."""
+        ptr, n, keep, begins, lens = _batch_input(files)
+        counts = np.zeros(max(1, len(lens)), dtype=np.uint64)
+        t = _Totals()
+        _check(lib().ugx_count_lines_bool_batch(self._h, *self._bool_query(patterns, cnf), ptr, n, begins.ctypes.data,
+                                                lens.ctypes.data, len(lens), LINES_INVERT if invert else 0,
+                                                counts.ctypes.data, C.byref(t)))
+        return counts[:len(lens)], self._totals(t)
+
+    def find_lines_bool_batch_device(self, patterns, cnf, files, invert: bool = False):
+        """ugx_find_lines_bool_batch with the records left on the device: (first, totals); fetch_lines() pages through
+        them.  `files` as for batch_records_device."""
+        ptr, n, keep, begins, lens = _batch_input(files)
+        first = np.zeros(len(lens) + 1, dtype=np.uint64)
+        cnt = C.c_uint64()
+        t = _Totals()
+        _check(lib().ugx_find_lines_bool_batch(self._h, *self._bool_query(patterns, cnf), ptr, n, begins.ctypes.data,
+                                               lens.ctypes.data, len(lens), LINES_INVERT if invert else 0,
+                                               first.ctypes.data, None, 0, C.byref(cnt), C.byref(t)))
+        return first, self._totals(t)
+
+    def find_lines_bool_batch(self, patterns, cnf, files, invert: bool = False):
+        """`ugrep -rn -e A --and -e B` of many files in one launch sequence: (line records, first, totals).  File i's
+        records are rec[first[i]:first[i + 1]], exactly find_lines_bool(file i, invert).  `files` as for
+        batch_records_device."""
+        first, t = self.find_lines_bool_batch_device(patterns, cnf, files, invert)
+        return self.fetch_lines(0, t.matches), first, t
 
     def close(self):
         if self._h:

@@ -209,6 +209,7 @@ struct ugx_scanner {
   // Boolean line queries (ugx_*_lines_bool): the term mask of every line, and the count pass's block values + line ends
   DevBuf<uint32_t> bool_mask;
   DevBuf<uint64_t> bool_pos;     // [2 * blocks] | [lines]
+  DevBuf<uint64_t> bool_files;   // a batch: every file's lines | newlines [nfiles + 1] each, selected lines [nfiles]
 };
 
 extern "C" {
@@ -1495,6 +1496,20 @@ int bool_check(const ugx_scanner* s, const ugx_pattern* const* patterns, uint32_
   return UGX_OK;
 }
 
+// the clauses as the Boolean kernels take them, by value
+ugx::BoolQuery bool_query(const ugx_bool_clause* clauses, uint32_t nclauses, uint32_t flags)
+{
+  ugx::BoolQuery q{};
+  for (uint32_t c = 0; c < nclauses; ++c)
+  {
+    q.pos[c] = clauses[c].pos;
+    q.neg[c] = clauses[c].neg;
+  }
+  q.nclauses = nclauses;
+  q.invert = flags & UGX_LINES_INVERT;
+  return q;
+}
+
 // Boolean line queries: every term's matching lines (select_lines, bases 0) marked into one term mask per line, then
 // the clauses (bool_lines.cu).  want_records = false stops after the count (ugx_count_lines_bool).
 int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns, const ugx_bool_clause* clauses,
@@ -1535,14 +1550,7 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
     }
   }
   s->lines_n = 0;
-  ugx::BoolQuery q{};
-  for (uint32_t c = 0; c < nclauses; ++c)
-  {
-    q.pos[c] = clauses[c].pos;
-    q.neg[c] = clauses[c].neg;
-  }
-  q.nclauses = nclauses;
-  q.invert = flags & UGX_LINES_INVERT;
+  const ugx::BoolQuery q = bool_query(clauses, nclauses, flags);
   const uint64_t nlb = ugx::bool_line_blocks(nlines), nreg = want_records ? ugx::bool_regions(n) : 0;
   const uint64_t nblk = nlb > nreg ? nlb : nreg;
   TRY(s->bool_pos.ensure(2 * nblk + (want_records ? nlines : 0)));
@@ -1729,6 +1737,7 @@ namespace {
 // The files lie in one buffer, file f at buf[begins[f], begins[f] + lens[f]); tile g of a launch is tile ti[g] of file
 // tf[g], so the tiles are ordered by file and then by offset.
 struct Batch {
+  uint64_t nfiles = 0;
   std::vector<uint32_t> tf, ti;
   const uint8_t* dbuf = nullptr;
   ugx::BatchArgs a;
@@ -1737,6 +1746,7 @@ struct Batch {
 // the checks of the file table every batch entry point makes, and the tile table; `who` names the entry point
 int batch_tiles(const char* who, uint64_t nbytes, const uint64_t* begins, const uint64_t* lens, uint64_t nfiles, Batch& b)
 {
+  b.nfiles = nfiles;
   for (uint64_t f = 0; f < nfiles; ++f)
   {
     if ((begins[f] & 15) != 0 || begins[f] > nbytes || lens[f] > nbytes - begins[f])
@@ -1780,10 +1790,58 @@ int batch_upload(ugx_scanner* s, const uint64_t* begins, const uint64_t* lens, u
   return UGX_OK;
 }
 
-// match records (lines == false) or line records of a batch: the count pass, the tile prefix, then the per-file counts
-// and the totals to the host in the one synchronise that sizes the arena, and the emit pass into the scanner's match or
-// line arena.  first[nfiles + 1] receives every file's record range, *n_out the number of records, out[cap] the
-// records (out == NULL with cap == 0: they stay on the device).
+// the selection of a batch, match records (lines == false) or line records: the count pass, the tile prefix, then the
+// per-file counts and the totals to the host in the one synchronise that sizes the arena (`before_sync` enqueues
+// whatever else the caller reads there), and the emit pass into the scanner's match or line arena.  The batch is
+// uploaded (batch_upload, b.a.counts zero) and the tile scratch sized.  sfirst[nfiles + 1] receives every file's record
+// range; *tt the records, the newlines and the launches.  Afterwards tile_matches / tile_newlines hold the exclusive
+// record and newline prefix of the batch tiles.
+template <typename BeforeSync = int (&)()>
+int select_lines_batch(ugx_scanner* s, const ugx_pattern* p, const Batch& b, bool lines, uint32_t flags, const char* who,
+                       uint64_t* sfirst, ugx_totals* tt, BeforeSync&& before_sync = no_setup)
+{
+  const uint64_t nfiles = b.nfiles, ntiles = b.tf.size();
+  ugx::BatchRecordArgs r;
+  r.tile_matches = s->tile_matches.p;
+  r.tile_newlines = s->tile_newlines.p;
+  r.strip_counts = s->strip_counts.p;
+  r.out = nullptr;
+  r.lout = nullptr;
+  r.out_cap = 0;
+  // a prefilter that admits no candidate (config 3) searches no line: no match records, and the inverted line
+  // records are every line
+  r.lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
+  CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, false, s->sm_count, s->stream));
+  CU(ugx::launch_tile_prefix(s->tile_matches.p, s->tile_newlines.p, ntiles, s->totals, s->stream));
+  CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+  CU(cudaMemcpyAsync(sfirst + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+  TRY(before_sync());
+  CU(cudaStreamSynchronize(s->stream));
+  tt->launches += 2;
+  const uint64_t nrec = s->h_totals[ugx::SLOT_MATCHES];
+  sfirst[0] = 0;
+  for (uint64_t f = 0; f < nfiles; ++f)
+    sfirst[f + 1] += sfirst[f];
+  if (sfirst[nfiles] != nrec)
+    return fail(UGX_E_CUDA, std::string(who) + ": per-file record counts disagree with the total");
+  TRY(lines ? s->lines.ensure(nrec) : s->records.ensure(nrec));
+  if (nrec > 0)
+  {
+    r.out = lines ? nullptr : s->records.p;
+    r.lout = lines ? s->lines.p : nullptr;
+    r.out_cap = nrec;
+    CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, true, s->sm_count, s->stream));
+    tt->launches += 1;
+  }
+  (lines ? s->lines_n : s->records_n) = nrec;
+  tt->matches = nrec;
+  tt->newlines = s->h_totals[ugx::SLOT_NEWLINES];
+  return UGX_OK;
+}
+
+// match records (lines == false) or line records of a batch: select_lines_batch, and with ctx the context stage.
+// first[nfiles + 1] receives every file's record range, *n_out the number of records, out[cap] the records (out ==
+// NULL with cap == 0: they stay on the device).
 int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_t nbytes, const uint64_t* begins,
                   const uint64_t* lens, uint64_t nfiles, bool lines, uint32_t flags, uint64_t* first, void* out, uint64_t cap,
                   uint64_t* n_out, ugx_totals* totals, const Context* ctx = nullptr)
@@ -1829,38 +1887,8 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
       ctx_first.assign(nfiles + 1, 0);
       sfirst = ctx_first.data();
     }
-    ugx::BatchRecordArgs r;
-    r.tile_matches = s->tile_matches.p;
-    r.tile_newlines = s->tile_newlines.p;
-    r.strip_counts = s->strip_counts.p;
-    r.out = nullptr;
-    r.lout = nullptr;
-    r.out_cap = 0;
-    // a prefilter that admits no candidate (config 3) searches no line: no match records, and the inverted line
-    // records are every line
-    r.lflags = flags | (p->never ? ugx::SCAN_LINES_NEVER : 0u);
-    CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, false, s->sm_count, s->stream));
-    CU(ugx::launch_tile_prefix(s->tile_matches.p, s->tile_newlines.p, ntiles, s->totals, s->stream));
-    CU(cudaMemcpyAsync(s->h_totals, s->totals, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaMemcpyAsync(sfirst + 1, b.a.counts, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    tt.launches = 2;
-    const uint64_t nrec = s->h_totals[ugx::SLOT_MATCHES];
-    const uint64_t nl_total = s->h_totals[ugx::SLOT_NEWLINES];
-    for (uint64_t f = 0; f < nfiles; ++f)
-      sfirst[f + 1] += sfirst[f];
-    if (sfirst[nfiles] != nrec)
-      return fail(UGX_E_CUDA, std::string(who) + ": per-file record counts disagree with the total");
-    TRY(lines ? s->lines.ensure(nrec) : s->records.ensure(nrec));
-    if (nrec > 0)
-    {
-      r.out = lines ? nullptr : s->records.p;
-      r.lout = lines ? s->lines.p : nullptr;
-      r.out_cap = nrec;
-      CU(ugx::launch_scan_batch_records(p->dev, b.dbuf, b.a, r, lines, true, s->sm_count, s->stream));
-      tt.launches += 1;
-    }
-    arena_n = nrec;
+    TRY(select_lines_batch(s, p, b, lines, flags, who, sfirst, &tt));
+    const uint64_t nrec = tt.matches, nl_total = tt.newlines;
     if (ctx != nullptr)
     {
       // every file's first batch tile: the tiles are ordered by file
@@ -1883,6 +1911,138 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
     TRY(end_scan(s, tt, totals));
     return lines ? copy_out(s, s->lines.p, sizeof(ugx_line), arena_n, out, cap, n_out, true, "record buffer too small")
                  : copy_out(s, s->records.p, sizeof(ugx_match), arena_n, out, cap, n_out, true, "record buffer too small");
+  });
+}
+
+// Boolean line queries over a batch: every term's batch selection (select_lines_batch, flags 0) marked into one term
+// mask per line of the batch, the lines numbered across the files from the first term's newline prefix, then the
+// clauses (bool_lines.cu).  want_records = false stops after the count: counts[nfiles] (ugx_count_lines_bool_batch);
+// otherwise first[nfiles + 1] and the records as in ugx_find_lines_batch.
+int bool_batch(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns, const ugx_bool_clause* clauses,
+               uint32_t nclauses, const void* buf, uint64_t nbytes, const uint64_t* begins, const uint64_t* lens,
+               uint64_t nfiles, uint32_t flags, bool want_records, uint64_t* counts, uint64_t* first, ugx_line* out,
+               uint64_t cap, uint64_t* n_out, ugx_totals* totals)
+{
+  const char* who = want_records ? "ugx_find_lines_bool_batch" : "ugx_count_lines_bool_batch";
+  if (n_out)
+    *n_out = 0;
+  TRY(bool_check(s, patterns, npatterns, clauses, nclauses, buf, nbytes, flags));
+  // the per-file result: counts[nfiles], or first[nfiles + 1] with the records
+  uint64_t* per_file = want_records ? first : counts;
+  const uint64_t at = want_records ? 1 : 0;
+  if (nfiles != 0 && (begins == nullptr || lens == nullptr || per_file == nullptr))
+    return fail(UGX_E_INVALID, std::string(who) + ": bad argument");
+  ugx_totals tt{};
+  tt.flags = UGX_TOT_NEWLINES;
+  tt.kernel = UGX_K_BOOL_LINES;
+  if (totals)
+    *totals = tt;
+  if (want_records && first != nullptr)
+    first[0] = 0;
+  if (nfiles == 0)
+  {
+    s->lines_n = 0;
+    return UGX_OK;
+  }
+  return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
+    Batch b;
+    TRY(batch_tiles(who, nbytes, begins, lens, nfiles, b));
+    // the line arena is rewritten below: its last result is gone from here on
+    s->lines_n = 0;
+    memset(per_file, 0, (nfiles + at) * sizeof(uint64_t));
+    if (b.tf.empty())
+      return UGX_OK; // only empty files: no lines
+    const uint64_t ntiles = b.tf.size(), nf1 = nfiles + 1;
+    TRY(begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&]() -> int {
+      TRY(batch_upload(s, begins, lens, nfiles, b));
+      TRY(ensure_tiles(s, ntiles));
+      TRY(s->strip_counts.ensure(ntiles * ugx::SCAN_THREADS));
+      return s->bool_files.ensure(3 * nf1);
+    }));
+    // every file's lines, then lb[] (its first global line, lb[nfiles] = the batch's lines); its newlines; its
+    // selected lines
+    uint64_t* lb = s->bool_files.p;
+    uint64_t* fnl = lb + nf1;
+    unsigned long long* fsel = reinterpret_cast<unsigned long long*>(fnl + nf1);
+    std::vector<uint64_t> term_first(nf1);
+    uint64_t nlines = 0;
+    for (uint32_t j = 0; j < npatterns; ++j)
+    {
+      if (j > 0)
+        CU(cudaMemsetAsync(b.a.counts, 0, nfiles * sizeof(uint64_t), s->stream));
+      ugx_totals t{};
+      TRY(select_lines_batch(s, patterns[j], b, true, 0, who, term_first.data(), &t, [&]() -> int {
+        if (j > 0)
+          return UGX_OK;
+        // the line table from this term's newline prefix, read in the synchronise that sizes its arena
+        CU(cudaMemsetAsync(lb, 0, 2 * nf1 * sizeof(uint64_t), s->stream));
+        CU(ugx::launch_bool_batch_lines(b.dbuf, b.a, s->tile_newlines.p, s->totals + ugx::SLOT_NEWLINES, lb, fnl,
+                                        s->stream));
+        CU(ugx::launch_tile_prefix(lb, fnl, nf1, s->totals + ugx::SLOT_BATCH_LINES, s->stream));
+        CU(cudaMemcpyAsync(s->h_totals + ugx::SLOT_BATCH_LINES, s->totals + ugx::SLOT_BATCH_LINES,
+                           2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+        return UGX_OK;
+      }));
+      tt.launches += t.launches;
+      if (j == 0)
+      {
+        tt.launches += 2;
+        tt.newlines = t.newlines;
+        nlines = s->h_totals[ugx::SLOT_BATCH_LINES];
+        TRY(s->bool_mask.ensure(nlines));
+        CU(cudaMemsetAsync(s->bool_mask.p, 0, nlines * sizeof(uint32_t), s->stream));
+      }
+      if (s->lines_n > 0)
+      {
+        CU(ugx::launch_bool_batch_mark(s->lines.p, s->lines_n, s->tile_matches.p, b.a, lb, s->bool_mask.p, 1u << j,
+                                       s->sm_count, s->stream));
+        tt.launches += 1;
+      }
+    }
+    s->lines_n = 0;
+    const ugx::BoolQuery q = bool_query(clauses, nclauses, flags);
+    const uint64_t nlb = ugx::bool_line_blocks(nlines);
+    TRY(s->bool_pos.ensure(2 * nlb + (want_records ? nlines : 0)));
+    CU(cudaMemsetAsync(fsel, 0, nfiles * sizeof(unsigned long long), s->stream));
+    ugx::BoolBatchArgs a{};
+    a.buf = b.dbuf;
+    a.files = b.a;
+    a.nfiles = nfiles;
+    a.lb = lb;
+    a.nlines = nlines;
+    a.mask = s->bool_mask.p;
+    a.fsel = fsel;
+    a.blk = s->bool_pos.p;
+    a.nblocks = nlb;
+    a.tile_nl = s->tile_newlines.p;
+    a.eol = s->bool_pos.p + 2 * nlb;
+    CU(ugx::launch_bool_batch_count(a, q, s->stream));
+    CU(ugx::launch_tile_prefix(a.blk, a.blk + nlb, nlb, s->totals, s->stream));
+    CU(cudaMemcpyAsync(per_file + at, fsel, nfiles * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+    TRY(read_totals(s, 1));
+    tt.launches += 2;
+    const uint64_t nsel = s->h_totals[ugx::SLOT_MATCHES];
+    tt.matches = nsel;
+    if (want_records)
+    {
+      for (uint64_t f = 0; f < nfiles; ++f)
+        first[f + 1] += first[f];
+      if (first[nfiles] != nsel)
+        return fail(UGX_E_CUDA, std::string(who) + ": per-file line counts disagree with the total");
+      if (nsel > 0)
+      {
+        TRY(s->lines.ensure(nsel));
+        a.out = s->lines.p;
+        CU(ugx::launch_bool_batch_index(a, s->stream));
+        CU(ugx::launch_bool_batch_emit(a, q, s->stream));
+        tt.launches += 2;
+        s->lines_n = nsel;
+      }
+    }
+    TRY(end_scan(s, tt, totals));
+    return want_records ? copy_out(s, s->lines.p, sizeof(ugx_line), s->lines_n, out, cap, n_out, true,
+                                   "record buffer too small")
+                        : UGX_OK;
   });
 }
 
@@ -1943,6 +2103,24 @@ int ugx_find_context_batch(ugx_scanner* s, const ugx_pattern* p, const void* buf
 {
   const Context ctx{before, after};
   return batch_records(s, p, buf, nbytes, begins, lens, nfiles, true, flags, first, out, cap, n_out, totals, &ctx);
+}
+
+int ugx_count_lines_bool_batch(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns,
+                               const ugx_bool_clause* clauses, uint32_t nclauses, const void* buf, uint64_t nbytes,
+                               const uint64_t* begins, const uint64_t* lens, uint64_t nfiles, uint32_t flags,
+                               uint64_t* counts, ugx_totals* totals)
+{
+  return bool_batch(s, patterns, npatterns, clauses, nclauses, buf, nbytes, begins, lens, nfiles, flags, false, counts,
+                    nullptr, nullptr, 0, nullptr, totals);
+}
+
+int ugx_find_lines_bool_batch(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npatterns,
+                              const ugx_bool_clause* clauses, uint32_t nclauses, const void* buf, uint64_t nbytes,
+                              const uint64_t* begins, const uint64_t* lens, uint64_t nfiles, uint32_t flags,
+                              uint64_t* first, ugx_line* out, uint64_t cap, uint64_t* n_out, ugx_totals* totals)
+{
+  return bool_batch(s, patterns, npatterns, clauses, nclauses, buf, nbytes, begins, lens, nfiles, flags, true, nullptr,
+                    first, out, cap, n_out, totals);
 }
 
 int ugx_check_text(ugx_scanner* s, const void* buf, uint64_t nbytes, ugx_text_info* out)

@@ -32,7 +32,9 @@ enum TotalsSlot : int {
   SLOT_LAST_LINE = 5,   // launch_last_line: start of the buffer's last line
   SLOT_SPAN_FLAGS = 6,  // SpanArgs::flags
   SLOT_UTF8 = 7,        // launch_utf8_check's flags
-  SLOT_COUNT = 8
+  SLOT_BATCH_LINES = 8, // ugx_*_lines_bool_batch: the prefix over the file line table: lines of the batch
+  SLOT_BATCH_NEWLINES = 9, //   ... and its newlines
+  SLOT_COUNT = 10
 };
 
 struct ScanArgs {
@@ -260,6 +262,35 @@ cudaError_t launch_bool_mark(const ugx_line* rec, uint64_t nrec, uint32_t* mask,
 cudaError_t launch_bool_count(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
 cudaError_t launch_bool_index(const BoolArgs& a, cudaStream_t st);
 cudaError_t launch_bool_emit(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
+
+// ---- Boolean line queries over many files (bool_lines.cu, ugx_*_lines_bool_batch) ----
+// The batch's lines are numbered across the files, file f owning [lb[f], lb[f + 1]).  After the first term's count pass
+// (launch_scan_batch_records) and its tile prefix, launch_bool_batch_lines writes every file's lines and newlines, and
+// launch_tile_prefix over those columns ([nfiles + 1] each, zeroed by the caller) gives lb[] with lb[nfiles] = the lines.
+// After every term's selection launch_bool_batch_mark ORs its bit into the mask of each record's line (the batch tiles'
+// record prefix locates the records of a file).  Then the count pass, launch_tile_prefix over its block values, and
+// for records the index and emit passes.
+struct BoolBatchArgs {
+  const uint8_t* buf;            // the batch buffer
+  BatchArgs files;               // its file and tile tables
+  uint64_t nfiles;
+  const uint64_t* lb;            // [nfiles + 1] every file's first global line; lb[nfiles] = nlines
+  uint64_t nlines;
+  const uint32_t* mask;          // [nlines] term mask of every line
+  unsigned long long* fsel;      // [nfiles] count pass: selected lines of every file (zeroed by the caller)
+  uint64_t* blk;                 // [2 * nblocks] count pass: selected lines of line block b | 0; after the prefix: before b
+  uint64_t nblocks;              // line blocks (BOOL_LINES_PER_BLOCK lines each)
+  const uint64_t* tile_nl;       // [ntiles] index pass: the exclusive newline prefix of the batch tiles
+  uint64_t* eol;                 // [nlines] index pass: offset within its file of every line's '\n' (or the file's end)
+  ugx_line* out;                 // emit pass: [selected lines] grouped by file, in input order
+};
+cudaError_t launch_bool_batch_lines(const uint8_t* buf, const BatchArgs& b, const uint64_t* tile_nl,
+                                    const unsigned long long* nl_total, uint64_t* flines, uint64_t* fnl, cudaStream_t st);
+cudaError_t launch_bool_batch_mark(const ugx_line* rec, uint64_t nrec, const uint64_t* tile_rec, const BatchArgs& b,
+                                   const uint64_t* lb, uint32_t* mask, uint32_t bit, int sm_count, cudaStream_t st);
+cudaError_t launch_bool_batch_count(const BoolBatchArgs& a, const BoolQuery& q, cudaStream_t st);
+cudaError_t launch_bool_batch_index(const BoolBatchArgs& a, cudaStream_t st);
+cudaError_t launch_bool_batch_emit(const BoolBatchArgs& a, const BoolQuery& q, cudaStream_t st);
 
 // reflex::isutf8 / NUL test (utf8_check.cu): flags bit 0 = not UTF-8 by the reference's rule, bit 1 = has a NUL
 cudaError_t launch_utf8_check(const uint8_t* buf, uint64_t n, unsigned int* flags, int sm_count, cudaStream_t st);
