@@ -1553,10 +1553,13 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
   const ugx::BoolQuery q = bool_query(clauses, nclauses, flags);
   const uint64_t nlb = ugx::bool_line_blocks(nlines), nreg = want_records ? ugx::bool_regions(n) : 0;
   const uint64_t nblk = nlb > nreg ? nlb : nreg;
-  TRY(s->bool_pos.ensure(2 * nblk + (want_records ? nlines : 0)));
+  // block values | line ends | the emit pass's one-file line table
+  TRY(s->bool_pos.ensure(2 * nblk + (want_records ? nlines + 2 : 0)));
   ugx::BoolArgs a{};
   a.buf = dbuf;
   a.n = n;
+  a.nfiles = 1;
+  a.lb = s->bool_pos.p + 2 * nblk + nlines;
   a.nlines = nlines;
   a.mask = s->bool_mask.p;
   a.blk = s->bool_pos.p;
@@ -1576,7 +1579,7 @@ int bool_common(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npa
     TRY(s->lines.ensure(nsel));
     a.out = s->lines.p;
     CU(ugx::launch_bool_index(a, s->stream));
-    CU(ugx::launch_bool_emit(a, q, s->stream));
+    CU(ugx::launch_bool_batch_emit(a, q, s->stream));
     tt.launches += 2;
     s->lines_n = nsel;
   }
@@ -1790,6 +1793,29 @@ int batch_upload(ugx_scanner* s, const uint64_t* begins, const uint64_t* lens, u
   return UGX_OK;
 }
 
+// the start of a batch's records (batch_records, bool_batch), inside `guarded`: the tile table (b), the arena's last
+// result dropped, per_file[nper] zeroed, and begin_scan with the file and tile tables uploaded and the tile scratch
+// sized; `extra` sizes the caller's own scratch.  b.dbuf stays nullptr when every file is empty: nothing to scan.
+template <typename Extra = int (&)()>
+int begin_batch(ugx_scanner* s, const char* who, const void* buf, uint64_t nbytes, const uint64_t* begins,
+                const uint64_t* lens, uint64_t nfiles, uint64_t& arena_n, uint64_t* per_file, uint64_t nper,
+                const ugx_totals& tt, Batch& b, Extra&& extra = no_setup)
+{
+  TRY(batch_tiles(who, nbytes, begins, lens, nfiles, b));
+  // the arena is rewritten by the caller: its last result is gone from here on
+  arena_n = 0;
+  memset(per_file, 0, nper * sizeof(uint64_t));
+  if (b.tf.empty())
+    return UGX_OK;
+  const uint64_t ntiles = b.tf.size();
+  return begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&]() -> int {
+    TRY(batch_upload(s, begins, lens, nfiles, b));
+    TRY(ensure_tiles(s, ntiles));
+    TRY(s->strip_counts.ensure(ntiles * ugx::SCAN_THREADS));
+    return extra();
+  });
+}
+
 // the selection of a batch, match records (lines == false) or line records: the count pass, the tile prefix, then the
 // per-file counts and the totals to the host in the one synchronise that sizes the arena (`before_sync` enqueues
 // whatever else the caller reads there), and the emit pass into the scanner's match or line arena.  The batch is
@@ -1867,18 +1893,9 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
   }
   return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     Batch b;
-    TRY(batch_tiles(who, nbytes, begins, lens, nfiles, b));
-    // the arena is rewritten below: its last result is gone from here on
-    arena_n = 0;
-    memset(first, 0, (nfiles + 1) * sizeof(uint64_t));
-    if (b.tf.empty())
+    TRY(begin_batch(s, who, buf, nbytes, begins, lens, nfiles, arena_n, first, nfiles + 1, tt, b));
+    if (b.dbuf == nullptr)
       return UGX_OK; // only empty files: no lines, no records
-    const uint64_t ntiles = b.tf.size();
-    TRY(begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&]() -> int {
-      TRY(batch_upload(s, begins, lens, nfiles, b));
-      TRY(ensure_tiles(s, ntiles));
-      return s->strip_counts.ensure(ntiles * ugx::SCAN_THREADS);
-    }));
     // with context, first[] receives the printed lines' ranges and the selected records' ranges go to sfirst
     std::vector<uint64_t> ctx_first;
     uint64_t* sfirst = first;
@@ -1902,7 +1919,7 @@ int batch_records(ugx_scanner* s, const ugx_pattern* p, const void* buf, uint64_
       c.begins = b.a.begins;
       c.lens = b.a.lens;
       c.tile_nl = s->tile_newlines.p;
-      c.ntiles = ntiles;
+      c.ntiles = b.tf.size();
       TRY(context_stage(s, p, *ctx, flags, c, sfirst, ftile, first, &tt));
     }
     tt.matches = nrec;
@@ -1946,19 +1963,11 @@ int bool_batch(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npat
   }
   return guarded(UGX_E_NOMEM, nullptr, [&]() -> int {
     Batch b;
-    TRY(batch_tiles(who, nbytes, begins, lens, nfiles, b));
-    // the line arena is rewritten below: its last result is gone from here on
-    s->lines_n = 0;
-    memset(per_file, 0, (nfiles + at) * sizeof(uint64_t));
-    if (b.tf.empty())
+    const uint64_t nf1 = nfiles + 1;
+    TRY(begin_batch(s, who, buf, nbytes, begins, lens, nfiles, s->lines_n, per_file, nfiles + at, tt, b,
+                    [&] { return s->bool_files.ensure(3 * nf1); }));
+    if (b.dbuf == nullptr)
       return UGX_OK; // only empty files: no lines
-    const uint64_t ntiles = b.tf.size(), nf1 = nfiles + 1;
-    TRY(begin_scan(s, buf, nbytes, tt, nullptr, &b.dbuf, [&]() -> int {
-      TRY(batch_upload(s, begins, lens, nfiles, b));
-      TRY(ensure_tiles(s, ntiles));
-      TRY(s->strip_counts.ensure(ntiles * ugx::SCAN_THREADS));
-      return s->bool_files.ensure(3 * nf1);
-    }));
     // every file's lines, then lb[] (its first global line, lb[nfiles] = the batch's lines); its newlines; its
     // selected lines
     uint64_t* lb = s->bool_files.p;
@@ -2004,7 +2013,7 @@ int bool_batch(ugx_scanner* s, const ugx_pattern* const* patterns, uint32_t npat
     const uint64_t nlb = ugx::bool_line_blocks(nlines);
     TRY(s->bool_pos.ensure(2 * nlb + (want_records ? nlines : 0)));
     CU(cudaMemsetAsync(fsel, 0, nfiles * sizeof(unsigned long long), s->stream));
-    ugx::BoolBatchArgs a{};
+    ugx::BoolArgs a{};
     a.buf = b.dbuf;
     a.files = b.a;
     a.nfiles = nfiles;

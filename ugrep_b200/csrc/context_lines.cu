@@ -16,8 +16,10 @@
 //   context_match_kernel  under UGX_LINES_INVERT only: a context line is then a matching line, and a thread per
 //                         printed line runs find_in_line on it, as scan_lines_kernel does.  A kernel of its own keeps
 //                         the DFA code out of the walk.
+#include "block_scan.cuh"
 #include "device_pattern.cuh"
 #include "line_match.cuh"
+#include "line_stage.cuh"
 #include "scan_kernels.hpp"
 
 namespace ugx {
@@ -47,15 +49,7 @@ __device__ __forceinline__ CtxFile ctx_file(const ContextArgs& a, uint64_t i)
     return F;
   }
   // the last file whose first record is <= i (empty files share their first record with the next file)
-  uint64_t lo = 0, hi = a.nfiles; // fsel[lo] <= i < fsel[hi]
-  while (hi - lo > 1)
-  {
-    const uint64_t mid = (lo + hi) / 2;
-    if (a.fsel[mid] <= i)
-      lo = mid;
-    else
-      hi = mid;
-  }
+  const uint64_t lo = last_le(a.fsel, 0, a.nfiles, i);
   F.f = static_cast<uint32_t>(lo);
   F.lo = a.fsel[lo];
   F.hi = a.fsel[lo + 1];
@@ -92,77 +86,6 @@ __device__ __forceinline__ void ctx_window(const ContextArgs& a, const CtxFile& 
   ca = a.after < hi - L ? a.after : hi - L;
 }
 
-__device__ __forceinline__ uint64_t block_excl_scan64(uint64_t v, uint64_t* warp_sums, uint64_t* total)
-{
-  const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  uint64_t x = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1)
-  {
-    const uint64_t y = __shfl_up_sync(FULL, x, d);
-    if (lane >= static_cast<uint32_t>(d))
-      x += y;
-  }
-  if (lane == 31)
-    warp_sums[wid] = x;
-  __syncthreads();
-  if (wid == 0)
-  {
-    const uint64_t s = lane < nw ? warp_sums[lane] : 0;
-    uint64_t e = s;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1)
-    {
-      const uint64_t y = __shfl_up_sync(FULL, e, d);
-      if (lane >= static_cast<uint32_t>(d))
-        e += y;
-    }
-    if (lane < nw)
-      warp_sums[lane] = e - s;
-    if (lane == 31)
-      warp_sums[32] = e;
-  }
-  __syncthreads();
-  const uint64_t r = x - v + warp_sums[wid];
-  *total = warp_sums[32];
-  __syncthreads();
-  return r;
-}
-
-// bit b = byte b of the 16 bytes at t.b + c is '\n' (bytes at or past t.end read as none)
-__device__ __forceinline__ uint32_t newline_mask16(const Text& t, uint64_t c)
-{
-  uint32_t w[4];
-  if (c + 16 <= t.end)
-  {
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(t.b + c));
-    w[0] = v.x;
-    w[1] = v.y;
-    w[2] = v.z;
-    w[3] = v.w;
-  }
-  else
-  {
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-    {
-      w[k] = 0;
-#pragma unroll
-      for (int b = 0; b < 4; ++b)
-        if (c + 4 * k + b < t.end)
-          w[k] |= static_cast<uint32_t>(__ldg(t.b + c + 4 * k + b)) << (8 * b);
-    }
-  }
-  uint32_t m = 0;
-#pragma unroll
-  for (int k = 0; k < 4; ++k)
-  {
-    const uint32_t e = __vcmpeq4(w[k], 0x0a0a0a0au) & 0x80808080u;
-    m |= ((e >> 7) | (e >> 14) | (e >> 21) | (e >> 28)) << (4 * k) & (0xfu << (4 * k));
-  }
-  return m;
-}
-
 // one context line t[b, e) (e = its '\n', or the end of the file) without a match; under invert it is a matching line
 // and context_match_kernel fills in its first match (len = ~0 marks it)
 __device__ __forceinline__ void put_context(const ContextArgs& a, uint64_t line, uint64_t b, uint64_t e, uint64_t off,
@@ -190,7 +113,7 @@ __device__ __forceinline__ void walk_after(const ContextArgs& a, const Text& t, 
     uint32_t m = 0;
     if (c < t.end)
     {
-      m = newline_mask16(t, c);
+      m = newlines16(t.b, t.end, c);
       if (c < bol)
         m &= 0xffffu << (bol - c);
     }
@@ -242,7 +165,7 @@ __device__ __forceinline__ void walk_before(const ContextArgs& a, const Text& t,
     uint32_t m = 0;
     if (p >= 16ull * (lane + 1))
     {
-      m = newline_mask16(t, c);
+      m = newlines16(t.b, t.end, c);
       if (c + 16 > s)
         m &= (1u << (s - c)) - 1u; // below s only (s - c < 16)
     }
@@ -301,7 +224,7 @@ context_count_kernel(ContextArgs a)
       c = 1 + cb + ca;
     }
     uint64_t tot;
-    const uint64_t ex = block_excl_scan64(c, warp_sums, &tot);
+    const uint64_t ex = block_excl_scan(c, warp_sums, &tot);
     if (i < a.nsel)
       a.pos[i] = run + ex;
     run += tot;
@@ -380,15 +303,7 @@ context_match_kernel(const __grid_constant__ DevPattern P, ContextArgs a)
     uint64_t begin = 0, len = a.n;
     if (a.fout != nullptr)
     {
-      uint64_t lo = 0, hi = a.nfiles; // fout[lo] <= j < fout[hi]
-      while (hi - lo > 1)
-      {
-        const uint64_t mid = (lo + hi) / 2;
-        if (a.fout[mid] <= j)
-          lo = mid;
-        else
-          hi = mid;
-      }
+      const uint64_t lo = last_le(a.fout, 0, a.nfiles, j);
       begin = a.begins[lo];
       len = a.lens[lo];
     }
@@ -415,28 +330,18 @@ cudaError_t launch_context_count(const ContextArgs& a, cudaStream_t st)
 
 cudaError_t launch_context_emit(const ContextArgs& a, int sm_count, cudaStream_t st)
 {
-  uint64_t g = (a.nsel + CTX_THREADS - 1) / CTX_THREADS; // a warp per 32 records
-  const uint64_t gmax = static_cast<uint64_t>(sm_count) * 8;
-  if (g > gmax)
-    g = gmax;
-  if (g == 0)
-    g = 1;
-  context_emit_kernel<<<static_cast<unsigned>(g), CTX_THREADS, 0, st>>>(a);
+  const unsigned g = capped_grid(a.nsel, CTX_THREADS, sm_count, 8); // a warp per 32 records
+  context_emit_kernel<<<g, CTX_THREADS, 0, st>>>(a);
   return cudaGetLastError();
 }
 
 cudaError_t launch_context_match(const DevPattern& P, const ContextArgs& a, int sm_count, cudaStream_t st)
 {
-  uint64_t g = (a.nout + CTX_THREADS - 1) / CTX_THREADS;
-  const uint64_t gmax = static_cast<uint64_t>(sm_count) * 8;
-  if (g > gmax)
-    g = gmax;
-  if (g == 0)
-    g = 1;
+  const unsigned g = capped_grid(a.nout, CTX_THREADS, sm_count, 8);
   if (P.has_meta)
-    context_match_kernel<true><<<static_cast<unsigned>(g), CTX_THREADS, 0, st>>>(P, a);
+    context_match_kernel<true><<<g, CTX_THREADS, 0, st>>>(P, a);
   else
-    context_match_kernel<false><<<static_cast<unsigned>(g), CTX_THREADS, 0, st>>>(P, a);
+    context_match_kernel<false><<<g, CTX_THREADS, 0, st>>>(P, a);
   return cudaGetLastError();
 }
 

@@ -230,12 +230,19 @@ cudaError_t launch_context_emit(const ContextArgs& a, int sm_count, cudaStream_t
 // under UGX_LINES_INVERT, after the emit pass: the first match of every context line
 cudaError_t launch_context_match(const DevPattern& P, const ContextArgs& a, int sm_count, cudaStream_t st);
 
-// ---- Boolean line queries (bool_lines.cu, ugx_count_lines_bool / ugx_find_lines_bool: `--and`, `--andnot`, `--bool`) ----
-// After every term's selection launch_bool_mark ORs its bit into the term mask of each record's line; then a count pass
-// (selected lines per line block, newlines per byte region), launch_tile_prefix over both, and for records an index
-// pass (every line's end) and an emit pass.
+// ---- Boolean line queries (bool_lines.cu, ugx_*_lines_bool and ugx_*_lines_bool_batch: `--and`, `--andnot`, `--bool`) ----
+// One buffer: after every term's selection launch_bool_mark ORs its bit into the term mask of each record's line; then
+// a count pass (selected lines per line block, newlines per byte region), launch_tile_prefix over both, and for records
+// an index pass (every line's end) and the emit pass.
+// Many files: the batch's lines are numbered across the files, file f owning [lb[f], lb[f + 1]).  After the first term's
+// count pass (launch_scan_batch_records) and its tile prefix, launch_bool_batch_lines writes every file's lines and
+// newlines, and launch_tile_prefix over those columns ([nfiles + 1] each, zeroed by the caller) gives lb[] with
+// lb[nfiles] = the lines.  After every term's selection launch_bool_batch_mark ORs its bit into the mask of each
+// record's line (the batch tiles' record prefix locates the records of a file).  Then the batch count pass,
+// launch_tile_prefix over its block values, and for records the batch index pass and the emit pass.
+// The emit pass serves both: one buffer is one file, lines [0, nlines), with the call's bases.
 constexpr uint32_t BOOL_LINES_PER_BLOCK = 8192; // lines per block of the count and emit passes
-constexpr uint32_t BOOL_REGION = 65536;         // bytes per block of the newline count and the index pass
+constexpr uint32_t BOOL_REGION = 65536;         // bytes per block of the newline count and the index pass (one buffer)
 struct BoolQuery {                              // the clauses, passed by value in the kernel parameters
   uint32_t pos[UGX_BOOL_MAX_CLAUSES];
   uint32_t neg[UGX_BOOL_MAX_CLAUSES];
@@ -243,17 +250,24 @@ struct BoolQuery {                              // the clauses, passed by value 
   uint32_t invert;                              // UGX_LINES_INVERT: the lines that do not satisfy the query
 };
 struct BoolArgs {
-  const uint8_t* buf;
-  uint64_t n;
-  uint64_t nlines;          // newlines + (last byte != '\n')
-  const uint32_t* mask;     // [nlines] term mask of every line
-  uint64_t* blk;            // [2 * nblocks] count pass: selected lines of line block b | newlines of region b;
-                            //   after the prefix: the same before b
-  uint64_t nblocks;         // grid of the count pass: line blocks, or with want_index the larger of them and the regions
-  uint32_t want_index;      // the count pass also counts newlines per region (records follow)
-  uint64_t* eol;            // [nlines] index pass: offset of every line's '\n' (the buffer end for an unterminated one)
-  ugx_line* out;            // emit pass: [selected lines] in input order
-  uint64_t base_offset, base_line;
+  const uint8_t* buf;            // the buffer, or the batch buffer
+  uint64_t n;                    // one buffer: its size
+  BatchArgs files;               // a batch: its file and tile tables
+  uint64_t nfiles;               // 1 for one buffer
+  uint64_t* lb;                  // [nfiles + 1] every file's first line; lb[nfiles] = nlines.  One buffer: {0, nlines},
+                                 //   written by the count pass with want_index
+  uint64_t nlines;               // one buffer: newlines + (last byte != '\n')
+  const uint32_t* mask;          // [nlines] term mask of every line
+  unsigned long long* fsel;      // a batch, count pass: selected lines of every file (zeroed by the caller)
+  uint64_t* blk;                 // [2 * nblocks] count pass: selected lines of line block b | newlines of region b (a
+                                 //   batch: 0); after the prefix: the same before b
+  uint64_t nblocks;              // grid of the count pass: line blocks, or for one buffer with want_index the larger of
+                                 //   them and the regions
+  uint32_t want_index;           // one buffer: the count pass also counts newlines per region (records follow)
+  const uint64_t* tile_nl;       // a batch, index pass: the exclusive newline prefix of the batch tiles
+  uint64_t* eol;                 // [nlines] index pass: offset within its buffer or file of every line's '\n' (or its end)
+  ugx_line* out;                 // emit pass: [selected lines] grouped by file, in input order
+  uint64_t base_offset, base_line; // one buffer; 0 for a batch
 };
 uint64_t bool_line_blocks(uint64_t nlines);
 uint64_t bool_regions(uint64_t n);
@@ -261,36 +275,13 @@ cudaError_t launch_bool_mark(const ugx_line* rec, uint64_t nrec, uint32_t* mask,
                              cudaStream_t st);
 cudaError_t launch_bool_count(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
 cudaError_t launch_bool_index(const BoolArgs& a, cudaStream_t st);
-cudaError_t launch_bool_emit(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
-
-// ---- Boolean line queries over many files (bool_lines.cu, ugx_*_lines_bool_batch) ----
-// The batch's lines are numbered across the files, file f owning [lb[f], lb[f + 1]).  After the first term's count pass
-// (launch_scan_batch_records) and its tile prefix, launch_bool_batch_lines writes every file's lines and newlines, and
-// launch_tile_prefix over those columns ([nfiles + 1] each, zeroed by the caller) gives lb[] with lb[nfiles] = the lines.
-// After every term's selection launch_bool_batch_mark ORs its bit into the mask of each record's line (the batch tiles'
-// record prefix locates the records of a file).  Then the count pass, launch_tile_prefix over its block values, and
-// for records the index and emit passes.
-struct BoolBatchArgs {
-  const uint8_t* buf;            // the batch buffer
-  BatchArgs files;               // its file and tile tables
-  uint64_t nfiles;
-  const uint64_t* lb;            // [nfiles + 1] every file's first global line; lb[nfiles] = nlines
-  uint64_t nlines;
-  const uint32_t* mask;          // [nlines] term mask of every line
-  unsigned long long* fsel;      // [nfiles] count pass: selected lines of every file (zeroed by the caller)
-  uint64_t* blk;                 // [2 * nblocks] count pass: selected lines of line block b | 0; after the prefix: before b
-  uint64_t nblocks;              // line blocks (BOOL_LINES_PER_BLOCK lines each)
-  const uint64_t* tile_nl;       // [ntiles] index pass: the exclusive newline prefix of the batch tiles
-  uint64_t* eol;                 // [nlines] index pass: offset within its file of every line's '\n' (or the file's end)
-  ugx_line* out;                 // emit pass: [selected lines] grouped by file, in input order
-};
 cudaError_t launch_bool_batch_lines(const uint8_t* buf, const BatchArgs& b, const uint64_t* tile_nl,
                                     const unsigned long long* nl_total, uint64_t* flines, uint64_t* fnl, cudaStream_t st);
 cudaError_t launch_bool_batch_mark(const ugx_line* rec, uint64_t nrec, const uint64_t* tile_rec, const BatchArgs& b,
                                    const uint64_t* lb, uint32_t* mask, uint32_t bit, int sm_count, cudaStream_t st);
-cudaError_t launch_bool_batch_count(const BoolBatchArgs& a, const BoolQuery& q, cudaStream_t st);
-cudaError_t launch_bool_batch_index(const BoolBatchArgs& a, cudaStream_t st);
-cudaError_t launch_bool_batch_emit(const BoolBatchArgs& a, const BoolQuery& q, cudaStream_t st);
+cudaError_t launch_bool_batch_count(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
+cudaError_t launch_bool_batch_index(const BoolArgs& a, cudaStream_t st);
+cudaError_t launch_bool_batch_emit(const BoolArgs& a, const BoolQuery& q, cudaStream_t st);
 
 // reflex::isutf8 / NUL test (utf8_check.cu): flags bit 0 = not UTF-8 by the reference's rule, bit 1 = has a NUL
 cudaError_t launch_utf8_check(const uint8_t* buf, uint64_t n, unsigned int* flags, int sm_count, cudaStream_t st);
