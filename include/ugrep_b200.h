@@ -261,7 +261,10 @@ void ugx_scanner_destroy(ugx_scanner *s);
  *   "no_feeder"       pageable host buffers take one plain cudaMemcpyAsync instead of the feeder threads
  *   "no_span"         counting matches / records take the line-at-a-time kernels instead of the span kernels
  *   "no_search"       `-c` keeps count_lines_stream_kernel where the search automaton (count_lines_search_kernel,
- *                     ugx_search_describe) applies */
+ *                     ugx_search_describe) applies
+ *   "grid_sms"        k > 0: every launch sizes its grid as if the device had min(k, SMs) SMs, so that each warp takes
+ *                     many regions of a small buffer, as it does of a multi-GiB one (tests); 0 restores the device's
+ *                     count, k < 0 is UGX_E_INVALID.  Results do not depend on it. */
 int  ugx_scanner_set_option(ugx_scanner *s, const char *name, int value);
 
 /*

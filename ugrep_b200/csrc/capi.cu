@@ -161,7 +161,8 @@ struct ugx_pattern {
 struct ugx_scanner {
   int device = 0;
   cudaStream_t stream = nullptr;
-  int sm_count = 0;
+  int sm_count = 0;    // the SM count every launch sizes its grid by: device_sms, or fewer under the "grid_sms" option
+  int device_sms = 0;  // the device's own SM count
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   // scratch
   DevBuf<uint64_t> tile_matches;
@@ -581,7 +582,7 @@ int ugx_scanner_create(int device, void* stream, ugx_scanner** out)
     ugx_scanner_destroy(s);
     return cuda_fail(e, "ugx_scanner_create");
   }
-  s->sm_count = prop.multiProcessorCount;
+  s->device_sms = s->sm_count = prop.multiProcessorCount;
   *out = s;
   return UGX_OK;
 }
@@ -1704,6 +1705,16 @@ int ugx_scanner_set_option(ugx_scanner* s, const char* name, int value)
 {
   if (s == nullptr || name == nullptr)
     return fail(UGX_E_INVALID, "null argument");
+  // grids sized as if the device had min(value, SMs) SMs (0: all of them), so that a small buffer gives every warp the
+  // many regions a multi-GiB buffer gives it on the whole device.  No scratch depends on it: the stream partials hold
+  // STREAM_MAX_GRID CTAs whatever the grid, and the rest is sized by the buffer, its tiles, lines or records.
+  if (strcmp(name, "grid_sms") == 0)
+  {
+    if (value < 0)
+      return fail(UGX_E_INVALID, "scanner option grid_sms must be >= 0");
+    s->sm_count = value == 0 || value > s->device_sms ? s->device_sms : value;
+    return UGX_OK;
+  }
   using Flag = bool ugx_scanner::*;
   static const struct {
     const char* name;
